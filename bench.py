@@ -157,6 +157,17 @@ class ClockSampler:
                 "samples": len(self.sm), "source": "nvml" if self.nvml is not None else "nvidia-smi"}
 
 
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: what the timed path hands its caller at the end (the fitted mu / omega / alpha), one
+    DIR/<name>.npy each.  The inputs are a function of the arguments alone (seeded generator, device Philox noise
+    from --seed), so two builds run with the same arguments can be compared array for array."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def generate(cfg, device):
     """Synthetic sample (polee-synth-v1) as torch tensors on `device` + host tree arrays."""
     import torch
@@ -361,6 +372,8 @@ def run_ours(args):
         h.sync()
         barrier()
     ms = e0.elapsed_time(e1)
+    # before the per-kernel timings below, which launch ADAM updates of their own
+    outputs = dict(zip(("mu", "omega", "alpha"), h.get_params())) if args.dump_outputs else None
     if world > 1:
         t = torch.tensor([ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -538,6 +551,8 @@ def run_ours(args):
             line["parity"] = parity
         if cpu:
             line["cpu_baseline"] = cpu
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -661,6 +676,8 @@ def run_c4(args):
                              "kernels_ms": {"likelihood_pass_class+k1": round(t_k1, 4), "k_ec_lik": round(t_ec, 4),
                                             "k2_csc_grad": round(t_k2, 4), "k3_tree_reparam_adam": round(t_k3, 4)},
                              "note": "rank 0's launches; bytes = SURVEY 8(d) formula on the rows of the general layout"}}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dict(zip(("mu", "omega", "alpha"), out)))
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -728,6 +745,8 @@ def run_c5(args):
                 "e2e": {"value": round(v, 1), "unit": "evals/s", "h2d_bytes_per_step": int(agg[1].item() / agg[3].item()),
                         "d2h_bytes_per_step": int(3 * 4 * (n - 1)),
                         "step": "here a step = one whole sample (the e2e path IS the measured path of this config)"}}
+        if args.dump_outputs and fits:   # the fit of rank 0's last sample
+            dump_outputs(args.dump_outputs, {k: out[k] for k in ("mu", "omega", "alpha")})
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -809,13 +828,16 @@ def run_reference(args):
     for _ in range(args.steps):
         st.step()
         steps += 1
-        if time.perf_counter() - t0 > budget:
+        if args.budget_steps and time.perf_counter() - t0 > budget:
             break
     el = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("mu", "omega", "alpha"), st.params())))
     st.close()
     v = round(K * steps / el * scale, 3)
-    sample = "%d of the %d requested ADAM steps (x %d draws) on the full matrix within a %.0f s budget; %d warm-up%s" % (
-        steps, args.steps, K, budget, done_w, scale_note)
+    within = "within a %.0f s budget" % budget if args.budget_steps else "(--steps: no time budget)"
+    sample = "%d of the %d requested ADAM steps (x %d draws) on the full matrix %s; %d warm-up%s" % (
+        steps, args.steps, K, within, done_w, scale_note)
     print(json.dumps({
         "impl": "reference", "metric": "elbo_grad_evals_per_sec", "value": v, "unit": "evals/s", "n_gpus": args.gpus,
         "steps": steps, "warmup": done_w, "ms_per_step": round(el / steps * 1e3, 2), "higher_is_better": True,
@@ -831,7 +853,7 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 50)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="c3", choices=sorted(CONFIGS))
@@ -844,7 +866,16 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-budget", type=float, default=25.0)
     ap.add_argument("--samples", type=int, default=64, help="c5: number of samples")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the fitted mu / omega / alpha as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.steps is not None and args.config.startswith("c5"):
+        ap.error("--steps does not apply to %s: every sample is one whole %d-step fit" % (args.config, FIT_STEPS))
+    # the reference arm stops at its time budget only when the number of steps was left to it
+    args.budget_steps = args.steps is None
+    args.steps = 50 if args.steps is None else args.steps
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.oneshot_child:
         run_oneshot_child(args)

@@ -17,13 +17,13 @@ c_i64, c_u64, c_int, c_dbl = C.c_int64, C.c_uint64, C.c_int, C.c_double
 P = C.c_void_p
 
 
-def build(force=False):
-    """(Re)build the oracle; oracle/_ref only when /root/reference is present."""
+def build(force=False, reference=None):
+    """(Re)build the oracle; oracle/_ref only when `reference` names a checkout of the original Polee."""
     if force or not os.path.exists(_LIB) or \
             os.path.getmtime(_LIB) < os.path.getmtime(os.path.join(_HERE, "polee_oracle.c")):
         subprocess.check_call(["make", "-s", "-C", _HERE, "liboracle"])
-    if os.path.exists("/root/reference/src/tensorflow_ext/hsb_ops.cpp") and (force or not os.path.exists(_REF)):
-        subprocess.check_call(["make", "-s", "-C", _HERE, "ref"])
+    if reference and (force or not os.path.exists(_REF)):
+        subprocess.check_call(["make", "-s", "-C", _HERE, "ref", "REFERENCE=" + os.path.abspath(reference)])
 
 
 class OrcFitOpts(C.Structure):

@@ -1,10 +1,10 @@
 #!/usr/bin/env python3
 """Convert the reference's two HDF5 test fixtures into flat little-endian binaries.
 
-Run ONCE in the build container (where /root/reference exists); the outputs are
-committed under tests/golden/ because /root/reference does not exist on the GPU box.
+Run once on a checkout of the original Polee; the outputs are committed under tests/golden/
+so that the tests need none.
 
-    python tests/golden/make_fixtures.py
+    python tests/golden/make_fixtures.py <polee checkout>
 
 Inputs (reference test data, SURVEY.md section 4 / 8c):
   test/dataset/mBr_M_6w_1.likelihood-matrix.h5   written by rnaseq_sample.jl:505-519
@@ -23,7 +23,6 @@ import zlib
 
 import numpy as np
 
-REF = "/root/reference/test/dataset"
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -35,7 +34,8 @@ def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
-def main():
+def main(reference):
+    ref = os.path.join(reference, "test", "dataset")
     manifest = {}
 
     def dump(name, arr):
@@ -44,7 +44,7 @@ def main():
         arr.tofile(path)
         manifest[name] = {"dtype": str(arr.dtype), "count": int(arr.size), "sha256": sha(arr)}
 
-    lm = open(os.path.join(REF, "mBr_M_6w_1.likelihood-matrix.h5"), "rb").read()
+    lm = open(os.path.join(ref, "mBr_M_6w_1.likelihood-matrix.h5"), "rb").read()
     links = root_links(lm)
     m = int(read_dataset(lm, links["m"])[0])
     n = int(read_dataset(lm, links["n"])[0])
@@ -61,7 +61,7 @@ def main():
     dump("fixture_nzval.f32", nzval)
     dump("fixture_efflens.f32", efflens)
 
-    pp = open(os.path.join(REF, "mBr_M_6w_1.prep.h5"), "rb").read()
+    pp = open(os.path.join(ref, "mBr_M_6w_1.prep.h5"), "rb").read()
     links = root_links(pp)
     assert int(read_dataset(pp, links["m"])[0]) == m
     assert int(read_dataset(pp, links["n"])[0]) == n
@@ -84,4 +84,6 @@ def main():
 
 
 if __name__ == "__main__":
-    sys.exit(main())
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/make_fixtures.py <polee checkout>")
+    sys.exit(main(sys.argv[1]))

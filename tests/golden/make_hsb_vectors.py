@@ -2,10 +2,10 @@
 """Golden vectors for the three HSB ops, produced by the REFERENCE's own code.
 
 Runs the reference's src/tensorflow_ext/hsb_ops.cpp -- compiled unmodified into oracle/_ref/ over the stub
-TF API (oracle/Makefile target `ref`) -- on seeded inputs and stores inputs + outputs.  Only runnable where
-/root/reference exists (this build container); the .npz is committed because the GPU box has no reference.
+TF API (oracle/Makefile target `ref`) -- on seeded inputs and stores inputs + outputs.  It needs a checkout of
+the original Polee; the .npz is committed so that the tests need none.
 
-    python tests/golden/make_hsb_vectors.py
+    python tests/golden/make_hsb_vectors.py <polee checkout>
 """
 import os
 import sys
@@ -20,9 +20,9 @@ from polee_b200 import synth  # noqa: E402
 G = os.path.join(ROOT, "tests", "golden")
 
 
-def main():
-    O.build()
-    assert O.ref_lib() is not None, "oracle/_ref/libref_hsb_ops.so missing (needs /root/reference)"
+def main(reference):
+    O.build(force=True, reference=reference)   # never a stale oracle/_ref built from another checkout
+    assert O.ref_lib() is not None, "oracle/_ref/libref_hsb_ops.so missing (no hsb_ops.cpp under %s)" % reference
     rng = np.random.default_rng(20260417)
     out = {}
     pi = np.fromfile(os.path.join(G, "fixture_prep_node_parent_idxs.i32"), np.int32)
@@ -54,4 +54,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/make_hsb_vectors.py <polee checkout>")
+    main(sys.argv[1])

@@ -150,11 +150,106 @@ def test_opts_struct_layout_matches_header_in_python_and_julia():
     assert [(n, jmap[t]) for t, n in fields] == jfields
 
 
+class _H5Image:
+    """An HDF5 file laid out the way libhdf5 (through HDF5.jl) lays out the reference's test/dataset/*.h5, built byte by
+    byte from the format specification: superblock v0, v1 object headers (optionally split by a continuation block),
+    new-style groups (link messages in the object header, or dense storage in a fractal heap), contiguous scalars,
+    chunked + deflate arrays indexed by a v1 B-tree of two levels.  write_prep emits none of these group and array
+    encodings, so only this image exercises the reader paths those files take.  Checksums are left zero and the name
+    index of a dense group is left undefined: the reader uses neither."""
+
+    def __init__(self):
+        from polee_b200 import h5min
+        self.h5, self.f = h5min, h5min._File()
+
+    def header(self, msgs, split=None):
+        """v1 object header of (type, body) messages; from index `split` on they go to a continuation block"""
+        import struct
+        enc = [self.h5._msg(t, b) for t, b in msgs]
+        if split is None:
+            return self.f.append(self.h5._object_header(enc))
+        rest = b"".join(enc[split:])
+        head = b"".join(enc[:split]) + self.h5._msg(0x10, struct.pack("<QQ", self.f.append(rest), len(rest)))
+        return self.f.append(struct.pack("<BBHII4x", 1, 0, len(enc) + 1, 1, len(head)) + head)
+
+    def scalar(self, v):
+        return self.f.dataset(np.int64(v))
+
+    def chunked(self, arr, chunk, fanout=4, split=None):
+        """1-D dataset in deflate-compressed chunks of `chunk` elements (the last one stored whole, zero padded)"""
+        import struct
+        import zlib
+        arr = np.ascontiguousarray(arr)
+        leaves = []
+        for off in range(0, len(arr), chunk):
+            part = np.zeros(chunk, arr.dtype)
+            part[:len(arr) - off] = arr[off:off + chunk]
+            z = zlib.compress(part.tobytes(), 6)
+            leaves.append((len(z), off, self.f.append(z)))
+
+        def node(level, entries):   # entries: (bytes of the first chunk below, its element offset, child address)
+            b = b"TREE" + struct.pack("<BBHQQ", 1, level, len(entries), self.h5.UNDEF, self.h5.UNDEF)
+            for nbytes, off, child in entries:
+                b += struct.pack("<IIQQQ", nbytes, 0, off, 0, child)
+            return self.f.append(b + struct.pack("<IIQQ", 0, 0, len(arr), 0))
+
+        level0 = [leaves[i][:2] + (node(0, leaves[i:i + fanout]),) for i in range(0, len(leaves), fanout)]
+        root = node(1, level0) if len(level0) > 1 else level0[0][2]
+        deflate = struct.pack("<BB6x", 1, 1) + struct.pack("<HHHHI4x", 1, 0, 0, 1, 6)   # filter 1, level 6
+        msgs = [(0x01, self.h5._dataspace_msg(arr.shape)), (0x03, self.h5._dtype_msg(arr.dtype)),
+                (0x05, struct.pack("<BBBB", 2, 2, 2, 0)), (0x0B, deflate),
+                (0x08, struct.pack("<BBBQII", 3, 2, 2, root, chunk, arr.dtype.itemsize))]
+        return self.header(msgs, split)
+
+    @staticmethod
+    def link(name, addr, flags=0x10):
+        """link message v1 to a hard link; flags 0x10: UTF-8 character set field (what HDF5.jl asks for), 0x04:
+        creation order field"""
+        import struct
+        b = struct.pack("<BB", 1, flags) + (b"\0" * 8 if flags & 0x04 else b"") + (b"\x01" if flags & 0x10 else b"")
+        return b + struct.pack("<B", len(name)) + name.encode() + struct.pack("<Q", addr)
+
+    def compact_group(self, links, split=None):
+        import struct
+        u = self.h5.UNDEF
+        msgs = [(0x02, struct.pack("<BBQQ", 0, 0, u, u)), (0x0A, b"\0\0")]
+        msgs += [(0x06, self.link(k, a, 0x14 if i % 2 else 0x10)) for i, (k, a) in enumerate(links.items())]
+        return self.header(msgs, split)
+
+    def dense_group(self, links):
+        """links as managed objects of a fractal heap whose root is one direct block"""
+        import struct
+        u = self.h5.UNDEF
+        objs = b"".join(self.link(k, a) for k, a in links.items())
+        size = 512
+        while size < len(objs) + 21:
+            size *= 2
+        dblock = self.f.append(b"FHDB" + struct.pack("<BQI", 0, 0, 0) + objs.ljust(size - 21, b"\0") + b"\0" * 4)
+        frhp = self.f.append(b"FRHP" + struct.pack("<BHHBIQQQQQQQQQQQQ", 0, 7, 0, 0x02, 4096, 0, u, size - 21 - len(objs),
+                                                   u, size, size, size, len(links), 0, 0, 0, 0)
+                             + struct.pack("<HQQHHQH", 4, size, 65536, 32, 1, dblock, 0) + b"\0" * 4)
+        self.f.buf[dblock + 5:dblock + 13] = struct.pack("<Q", frhp)                  # the block's heap header
+        return self.header([(0x02, struct.pack("<BBQQ", 0, 0, frhp, u)), (0x0A, b"\0\0")])
+
+    def write(self, path, root):
+        """superblock v0 whose root symbol table entry caches nothing (a new-style root group)"""
+        import struct
+        f = self.f
+        f.buf += b"\0" * (-len(f.buf) % 8)
+        sb = self.h5.SIGNATURE + struct.pack("<BBBBBBBBHHI", 0, 0, 0, 0, 0, 8, 8, 0, 4, 16, 0)
+        sb += struct.pack("<QQQQ", 0, self.h5.UNDEF, len(f.buf), self.h5.UNDEF) + struct.pack("<QQII16x", 0, root, 0, 0)
+        f.buf[:96] = sb
+        with open(path, "wb") as fh:
+            fh.write(bytes(f.buf))
+        return bytes(f.buf)
+
+
 def test_h5min_prep_roundtrip_and_reference_files(tmp_path):
     """SURVEY 8f-3: the harness-side reader/writer of Polee's two HDF5 formats.  write_prep -> read_prep round trip
     (the file write_approximation produces, likelihood-approximation.jl:61-87), structural checks on the bytes, and
-    -- where the reference checkout is present (the build container) -- the reference's own files decode to the
-    committed golden arrays."""
+    the reference fixture (tests/golden) in files laid out as the reference's own test/dataset/*.h5 (_H5Image) decodes
+    to the committed golden arrays: the likelihood matrix with link messages in the root group, chunked + deflate
+    arrays and a continuation block, the prep file with its root group in a fractal heap."""
     import struct
     from polee_b200 import h5min
     rng = np.random.default_rng(1)
@@ -178,15 +273,29 @@ def test_h5min_prep_roundtrip_and_reference_files(tmp_path):
     md = back["metadata"]
     assert md["version"] == 2 and md["approximation"] == "Polee.LogitSkewNormalPTTApprox"
     assert md["gfffilename"] == "genes.gff3" and md["gffhash"] == "q83vEjRWeJA=" and md["args"] == "prep-sample a b"
-    ref = "/root/reference/test/dataset"
-    if not os.path.exists(ref):
-        pytest.skip("reference checkout not present (GPU box): the decode of its files is pinned by tests/golden")
     fx = Fixture()
-    lm = h5min.read_likelihood_matrix(os.path.join(ref, "mBr_M_6w_1.likelihood-matrix.h5"))
+    img = _H5Image()
+    links = {"m": img.scalar(fx.m), "n": img.scalar(fx.n), "colptr": img.chunked(fx.colptr, 64),
+             "rowval": img.chunked(fx.rowval, 4096, split=3), "nzval": img.chunked(fx.nzval, 4096),
+             "effective_lengths": img.chunked(fx.efflens, 313)}
+    raw = img.write(str(tmp_path / "lm.h5"), img.compact_group(links, split=4))
+    assert raw.count(b"TREE\x01\x01") == 3 and raw.count(b"TREE\x01\x00") == 9         # two-level chunk indexes
+    lm = h5min.read_likelihood_matrix(str(tmp_path / "lm.h5"))
     assert (lm["m"], lm["n"]) == (fx.m, fx.n) and np.array_equal(lm["colptr"], fx.colptr)
     assert np.array_equal(lm["rowval"], fx.rowval) and np.array_equal(lm["nzval"], fx.nzval)
-    pp = h5min.read_prep(os.path.join(ref, "mBr_M_6w_1.prep.h5"))
+    assert np.array_equal(lm["effective_lengths"], fx.efflens)
+    img = _H5Image()
+    links = {"n": img.scalar(fx.n), "m": img.scalar(fx.m), "effective_lengths": img.chunked(fx.efflens, 100),
+             "mu": img.chunked(fx.mu, 128, split=2), "omega": img.chunked(fx.omega, 128),
+             "alpha": img.chunked(fx.alpha, 128), "node_parent_idxs": img.chunked(fx.parent_idxs, 256),
+             "node_js": img.chunked(fx.js, 256), "metadata": img.compact_group({})}
+    raw = img.write(str(tmp_path / "pp.h5"), img.dense_group(links))
+    assert b"FHDB" in raw and b"FRHP" in raw
+    pp = h5min.read_prep(str(tmp_path / "pp.h5"))
     assert np.array_equal(pp["mu"], fx.mu) and np.array_equal(pp["node_js"], fx.js) and pp["n"] == fx.n
+    assert np.array_equal(pp["omega"], fx.omega) and np.array_equal(pp["alpha"], fx.alpha)
+    assert np.array_equal(pp["node_parent_idxs"], fx.parent_idxs) and pp["m"] == fx.m
+    assert np.array_equal(pp["effective_lengths"], fx.efflens) and pp["metadata"] == {}
 
 
 def test_hclust_host_restatement(oracle):
