@@ -156,9 +156,7 @@ int polee_step_stats(polee_handle *h, double *bytes_k1, double *bytes_k2, double
 /* which device layouts hold the matrix (a1-a2: replaces Xt = SparseMatrixCSC(transpose(X)),
  * likelihood-approximation.jl:407): info[0..5] = rows, entries, classes, tasks, blob bytes, partials of the
  * equivalence-class layout; info[6..7] = rows, entries of the general layouts; info[8] = their kind (0 none,
- * 1 split, 2 fused); info[9] = padded row slots of the class layout; info[10] = 1 when the tree set last has the
- * schedule of the experimental DFS-range backward kernel (POLEE_TREE_BWD=dfs), info[11] = its spans.  count <= 12
- * values are written. */
+ * 1 split, 2 fused); info[9] = padded row slots of the class layout.  count <= 10 values are written. */
 int polee_layout_info(polee_handle *h, int64_t *info, int32_t count);
 /* time (ms, CUDA events on the handle's stream) of `reps` launches of one named kernel group:
  * which = 1 (the likelihood pass; K1 alone on the pure split layout), 2 (K2 of the pure split layout),

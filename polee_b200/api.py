@@ -214,10 +214,10 @@ class Handle:
         return {"bytes_k1": b[0].value, "bytes_k2": b[1].value, "bytes_k3": b[2].value, "launches": nl.value}
 
     def layout_info(self):
-        v = (C.c_int64 * 12)()
-        self.check(self.lib.polee_layout_info(self.h, v, C.c_int32(12)))
+        v = (C.c_int64 * 10)()
+        self.check(self.lib.polee_layout_info(self.h, v, C.c_int32(10)))
         keys = ("ec_rows", "ec_nnz", "ec_classes", "ec_tasks", "ec_blob_bytes", "ec_partials", "general_rows",
-                "general_nnz", "general_kind", "ec_row_slots", "tree_bwd_dfs", "tree_bwd_spans")
+                "general_nnz", "general_kind", "ec_row_slots")
         out = dict(zip(keys, (int(x) for x in v)))
         out["general_kind"] = ("none", "split", "fused")[out["general_kind"]]
         return out

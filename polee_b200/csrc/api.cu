@@ -55,13 +55,7 @@ static std::mutex g_err_mu;
     (h)->err.clear();                 \
     if (cudaSetDevice((h)->device) != cudaSuccess) return (h)->fail(POLEE_ECUDA, "cudaSetDevice failed")
 
-constexpr int TREE_BIN_NODES = 512;
-// nodes per bottom bin of the tree schedule (POLEE_TREE_BIN_NODES: experiments)
-static int tree_bin_nodes() {
-    const char *e = getenv("POLEE_TREE_BIN_NODES");
-    const int v = e ? atoi(e) : TREE_BIN_NODES;
-    return v >= 32 && v <= 8192 ? v : TREE_BIN_NODES;
-}
+constexpr int TREE_BIN_NODES = 512;  // nodes per bottom bin of the tree schedule
 
 static void drop_graph(polee_handle *h) {
     if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
@@ -381,7 +375,7 @@ extern "C" int polee_set_tree(polee_handle *h, int64_t n, const int32_t *node_pa
     release_work_buffers(h);
     h->have_tree = false;
     HostPhaseTimer pt;
-    return finish_tree(h, h->th.build_from_parents(n, node_parent_idxs, node_js, tree_bin_nodes()), pt);
+    return finish_tree(h, h->th.build_from_parents(n, node_parent_idxs, node_js, TREE_BIN_NODES), pt);
 }
 
 // One RNASeqSample in one call: what polee_set_matrix_csc + polee_set_efflens + polee_set_tree do, with the host-side
@@ -398,13 +392,12 @@ extern "C" int polee_set_sample(polee_handle *h, int64_t m, int64_t n, const uin
     h->have_tree = false;  // nothing on this thread reads h->th / h->td until the worker has been joined
     HostPhaseTimer pt;
     std::string tree_err;
-    const int bin_nodes = tree_bin_nodes();
     struct Joiner {
         std::thread t;
         ~Joiner() { if (t.joinable()) t.join(); }
     } worker{std::thread([&]() {
         try {
-            tree_err = h->th.build_from_parents(n, node_parent_idxs, node_js, bin_nodes);
+            tree_err = h->th.build_from_parents(n, node_parent_idxs, node_js, TREE_BIN_NODES);
         } catch (const std::exception &e) {
             tree_err = std::string("tree: ") + e.what();
         }
@@ -548,7 +541,7 @@ static int launch_likelihood(polee_handle *h, int KP, int K, bool want_lp) {
         if (h->fused) {
             if ((rc = launch_fused(h, h->x, h->g, want_lp, h->lp_partial, nullptr, KP))) return rc;
         } else {
-            if ((rc = launch_k1(h, h->x, h->xd, h->w, want_lp, h->lp_partial, KP))) return rc;
+            if ((rc = launch_k1(h, h->x, h->w, want_lp, h->lp_partial, KP))) return rc;
             if ((rc = launch_k2(h, h->w, h->g, KP))) return rc;
         }
         if (want_lp && (rc = launch_reduce_lp(h, h->lp_partial, lp_out, KP))) return rc;
@@ -792,7 +785,6 @@ extern "C" int polee_loglik_grad(polee_handle *h, const float *xs, int32_t K, in
     int KP, rc;
     if ((rc = use_kp(h, K, &KP))) return rc;
     if ((rc = upload_kmajor<float>(h, xs, K, KP, h->n, h->x, 1.0f))) return rc;
-    if ((rc = launch_widen_x(h, h->x, h->xd, KP))) return rc;
     if ((rc = launch_likelihood(h, KP, K, !gradonly))) return rc;
     CK(cudaGetLastError());
     if (x_grad && (rc = download_kmajor<double, double>(h, h->g, K, KP, h->n, x_grad))) return rc;
@@ -846,8 +838,7 @@ extern "C" int polee_frag_prob_recip(polee_handle *h, const float *xs, float *w)
         CK(polee::copy_sync(h->stream, wp.data(), d_w, sizeof(float) * wp.size(), cudaMemcpyDeviceToHost));
         for (int64_t i = 0; i < h->gm; ++i) wr[i] = wp[(size_t)i * KP];
     } else {
-        if ((rc = launch_widen_x(h, h->x, h->xd, KP))) return rc;
-        if ((rc = launch_k1(h, h->x, h->xd, h->w, false, h->lp_partial, KP))) return rc;
+        if ((rc = launch_k1(h, h->x, h->w, false, h->lp_partial, KP))) return rc;
         CK(cudaStreamSynchronize(h->stream));
         std::vector<float> wp(h->m_pad);
         std::vector<uint32_t> perm(h->gm);
@@ -1055,11 +1046,9 @@ extern "C" int polee_step_stats(polee_handle *h, double *b1, double *b2, double 
 extern "C" int polee_layout_info(polee_handle *h, int64_t *info, int32_t count) {
     CHECK_H(h);
     if (!info || count < 1) return h->fail(POLEE_EINVAL, "layout_info: bad arguments");
-    const bool dfs_bwd = h->have_tree && h->td.bnodes != nullptr;
-    const int64_t v[12] = {h->ec_rows, h->ec_nnz, h->ec_classes, (int64_t)h->ec_tasks, (int64_t)h->ec_blob_bytes, h->ec_parts,
-                           h->gm, h->gnnz, (int64_t)((h->gm > 0 || h->ec_tasks == 0) ? (h->fused ? 2 : 1) : 0), h->ec_slots,
-                           dfs_bwd ? 1 : 0, dfs_bwd ? (int64_t)h->td.n_bspans : 0};
-    for (int i = 0; i < count && i < 12; ++i) info[i] = v[i];
+    const int64_t v[10] = {h->ec_rows, h->ec_nnz, h->ec_classes, (int64_t)h->ec_tasks, (int64_t)h->ec_blob_bytes, h->ec_parts,
+                           h->gm, h->gnnz, (int64_t)((h->gm > 0 || h->ec_tasks == 0) ? (h->fused ? 2 : 1) : 0), h->ec_slots};
+    for (int i = 0; i < count && i < 10; ++i) info[i] = v[i];
     return POLEE_OK;
 }
 
@@ -1079,7 +1068,7 @@ extern "C" int polee_time_kernel(polee_handle *h, int32_t which, int32_t reps, f
     for (int r = 0; r < reps && !rc; ++r) {
         if (which == 1) {  // the whole likelihood pass, except on the pure split layout (K1 here, K2 under which == 2)
             rc = (h->ec_tasks > 0 || h->fused) ? launch_likelihood(h, KP, K, false)
-                                               : launch_k1(h, h->x, h->xd, h->w, false, h->lp_partial, KP);
+                                               : launch_k1(h, h->x, h->w, false, h->lp_partial, KP);
         } else if (which == 2) {
             if (h->ec_tasks == 0 && !h->fused) rc = launch_k2(h, h->w, h->g, KP);  // otherwise: no second sparse kernel
         } else if (which == 3) {

@@ -184,29 +184,6 @@ struct DNode {
     uint32_t meta;      // depth | (1u << 31 if the node is its parent's LEFT child, i.e. the child that comes second)
 };
 
-// DFS-range backward kernel (k3d_tree_bwd): a CTA owns a span of <= DFS_CTA_NODES consecutive nodes made of whole
-// bottom subtrees (+ the top nodes interleaved between them, which it skips); a thread owns a run of DFS_BRUN nodes.
-//   tier 1: nodes whose subtree lies inside their run -- the thread walks its run backwards with a LIFO stack;
-//   tier 2: the other non-top nodes of the span -- a short level-synchronous sweep over the CTA's shared-memory slots;
-//   top   : nodes with more than DFS_CTA_NODES descendants -- the one-CTA-per-draw top kernel, as before.
-// DNode.meta of a span record: bit 0 internal node of tier 1; bit 1 its G is exported (the parent is not tier 1);
-// bit 2 exported to the global exchange slot (the parent is a top node) instead of a slot of the CTA;
-// bits 3..13 leaves: index among the span's leaves; bits 14..31 the slot.
-constexpr int DFS_BRUN = 32;
-constexpr int DFS_BRUNS = DFS_CTA_NODES / DFS_BRUN;  // runs per span = node slots of a CTA
-constexpr uint32_t BN_T1INT = 1u, BN_EXPORT = 2u, BN_GLOBAL = 4u;
-struct T2Node {
-    int32_t k;        // index among internal nodes
-    int32_t sl, sr;   // CTA slots holding the children's G
-    int32_t out;      // >= 0: CTA slot of this node's G; < 0: global exchange slot -1 - out; INT32_MIN: nobody needs it
-};
-struct BSpan {
-    int32_t s0, nn;        // first node, nodes
-    int32_t k0, nk;        // first internal-node index of the span, internal nodes (tier 1, tier 2 and interleaved top nodes)
-    int32_t t2_off, nt2;   // tier-2 records
-    int32_t lvl_off, nlev; // level offsets (nlev + 1 entries, relative to t2_off)
-};
-
 // Tree node, 0-based; leaf < 0 <=> internal node (then k = index among internal nodes in node order).
 struct TreeNode {
     int32_t left, right, k, leaf;
@@ -237,14 +214,12 @@ struct SSchedHost {
 struct SSchedDev {
     int32_t *bin_off = nullptr, *bin_lvl_ptr = nullptr, *lvl_off = nullptr;
     SNode *recs = nullptr;
-    int32_t *bin_desc = nullptr;  // [nbins][4] = {q0, nb, l0, nlev} (persistent kernels)
     int nbins = 0, max_bin_nodes = 0, max_bin_levels = 0;
 };
 
 struct TreeSchedDev {
     int32_t *bin_lvl_ptr = nullptr, *lvl_off = nullptr, *sch_node = nullptr;
     int nbins = 0;
-    int max_levels = 0;
 };
 
 struct TreeHost {
@@ -256,7 +231,6 @@ struct TreeHost {
     int n_slots = 0;             // exchange slots = bottom subtree roots
     bool caterpillar = false;    // list tree: internal node k at index 2k, right child = leaf at 2k+1, left = 2k+2
     std::vector<int32_t> chain_leaf;  // [n]: leaf id hanging off spine node k (k < n-1), [n-1] = the last leaf
-    int top_nodes = 0;
     int max_depth = 0;
     // Root -> node paths for the path-product forward kernel, per group of PATH_GROUP consecutive nodes (neighbours in
     // DFS order share most of their ancestors): the group's distinct ancestors `ganc` -- first the gcp[g] entries of the
@@ -270,13 +244,6 @@ struct TreeHost {
     // above are not built): per node a DNode; per run of DFS_RUN nodes the ancestors of its first node, root first, as
     // (k << 1) | 1 if the path continues into the LEFT child; per CTA the number of internal nodes before its first node
     bool preorder = false;
-    // DFS-range backward (built together with the DFS-run forward when the tree qualifies; then s_bottom is not built)
-    bool dfs_bwd = false;
-    std::vector<DNode> bnodes;     // [N + 2] by node id
-    std::vector<BSpan> bspans;
-    std::vector<T2Node> t2nodes;
-    std::vector<int32_t> t2_lvl;
-    int bwd_max_nk = 0, bwd_max_leaves = 0, bwd_max_slots = 0, bwd_max_stack = 0, bwd_max_t2 = 0, bwd_max_lev = 0;
     std::vector<DNode> dnodes;
     std::vector<uint32_t> drun_anc_ptr, drun_anc;
     std::vector<int32_t> dcta_k0;
@@ -295,15 +262,9 @@ struct TreeDev {
     int n_slots = 0;
     bool caterpillar = false;
     int32_t *chain_leaf = nullptr;
-    bool smem_path = false;  // shared-memory kernels usable (top part fits one CTA per draw)
     uint32_t *ganc_ptr = nullptr, *ganc = nullptr, *gcp = nullptr, *nsuf_ptr = nullptr;  // root paths (nullptr: not built)
     uint16_t *nsuf = nullptr;
     int n_groups = 0, max_ganc = 0, max_gsuf = 0;
-    DNode *bnodes = nullptr;  // DFS-range backward (nullptr: not available for this tree)
-    BSpan *bspans = nullptr;
-    T2Node *t2nodes = nullptr;
-    int32_t *t2_lvl = nullptr;
-    int n_bspans = 0, bwd_max_nk = 0, bwd_max_leaves = 0, bwd_max_slots = 0, bwd_max_stack = 0, bwd_max_t2 = 0, bwd_max_lev = 0;
     DNode *dnodes = nullptr;  // DFS-run forward (nullptr: not available for this tree)
     uint32_t *drun_anc_ptr = nullptr, *drun_anc = nullptr;
     int32_t *dcta_k0 = nullptr;
@@ -429,7 +390,6 @@ struct polee_handle {
     double *root_us = nullptr;            // [n_slots][KP] top -> bottom exchange (shared-memory tree kernels)
     float2 *root_G = nullptr;             // [n_slots][KP] bottom -> top exchange
     float *x = nullptr;                   // [n][KP]
-    double *xd = nullptr;                 // [n][KP] Float64(x): K1's gather table
     float *w = nullptr;                   // [m_pad][KP]
     double *g = nullptr;                  // [n][KP]  (all-reduced across ranks)
     float *g32 = nullptr;                 // [n][KP]  Float32 image of g for the all-reduce (multi-rank only)
@@ -533,15 +493,14 @@ int launch_ec(polee_handle *h, const float *x, double *g, bool add_to_g, bool wa
               bool lik_only = false);  // lik_only: the class kernel without its second stage (measurement)
 void preload_ec_kernels(const polee_handle *h, int KP, int K);  // lazy-loading warm-up, see tree_kernels.cu
 void preload_tree_kernels(int KP);
-bool ec_math_f32(const polee_handle *h);  // opts.exact_accumulation / POLEE_EC_MATH
+bool ec_math_f32(const polee_handle *h);  // opts.exact_accumulation != 2
 
 // fused_kernels.cu
 int fused_grid(polee_handle *h, int KP);
 int launch_fused(polee_handle *h, const float *x, double *g, bool want_lp, double *lp_partial, float *w_out, int KP);
 
 // sparse_kernels.cu
-int launch_k1(polee_handle *h, const float *x, const double *xd, float *w, bool want_lp, double *lp_partial, int KP);
-int launch_widen_x(polee_handle *h, const float *x, double *xd, int KP);
+int launch_k1(polee_handle *h, const float *x, float *w, bool want_lp, double *lp_partial, int KP);
 int launch_narrow(polee_handle *h, const double *in, float *out, size_t count);
 int launch_widen(polee_handle *h, const float *in, double *out, size_t count);
 int launch_k2(polee_handle *h, const float *w, double *g, int KP);

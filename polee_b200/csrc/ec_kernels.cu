@@ -14,7 +14,7 @@
 // its slot of the transcript-ordered partial array; k_ec_combine1/2 add each transcript's partials in Float64 in a
 // fixed order (no atomics anywhere).
 //
-// Arithmetic, template parameter T (POLEE_EC_MATH, see launch_ec):
+// Arithmetic, template parameter T (opts.exact_accumulation, see ec_math_f32):
 //   double: values and x widened exactly, every product and every sum in Float64 -- at least the reference's
 //           "Float32 product, Float64 accumulation" (SURVEY App. A); 1/p = MUFU.RCP64H + one Newton step (8.5e-13).
 //   float : FFMA2 (two draws per instruction); a row's sum (<= 64 terms) and a lane's column sums over the task's
@@ -25,7 +25,6 @@
 // depend on scheduling), and never synchronises with another warp.
 #include <algorithm>
 #include <cstdlib>
-#include <cstring>
 
 #include "common.cuh"
 #include "device_utils.cuh"
@@ -689,14 +688,8 @@ void preload_ec_kernels(const polee_handle *h, int KP, int K) {
 }
 
 // The arithmetic of the class kernel (see the header of this file): Float32 runs by default, Float64 with
-// opts.exact_accumulation == 2; POLEE_EC_MATH=f32|f64 overrides both (experiments).
-bool ec_math_f32(const polee_handle *h) {
-    static const int env = [] {
-        const char *e = getenv("POLEE_EC_MATH");
-        return !e ? -1 : (!strcmp(e, "f32") ? 1 : 0);
-    }();
-    return env >= 0 ? env == 1 : h->o.exact_accumulation != 2;
-}
+// opts.exact_accumulation == 2.
+bool ec_math_f32(const polee_handle *h) { return h->o.exact_accumulation != 2; }
 
 int ec_grid(polee_handle *h, int KP) {
     (void)KP;

@@ -19,7 +19,6 @@
 // reduction trees.  Tensor cores are not used: nothing here is a dense contraction.
 #include <algorithm>
 #include <cstdlib>
-#include <cstring>
 
 #include "common.cuh"
 #include "device_utils.cuh"
@@ -199,25 +198,6 @@ __device__ __forceinline__ void k1_short_row(const uint32_t (*sidx)[ROW_TILE], c
     Vec<KP>::st(wout, facc);
 }
 
-template <int KP>
-struct VecD {  // KP doubles; 256-bit requests (sm_100) where KP allows
-    static __device__ __forceinline__ void ld(const double *p, double *v) {
-        if constexpr (KP >= 4) {
-#pragma unroll
-            for (int q = 0; q < KP / 4; ++q)
-                asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];"
-                             : "=d"(v[4 * q]), "=d"(v[4 * q + 1]), "=d"(v[4 * q + 2]), "=d"(v[4 * q + 3])
-                             : "l"(p + 4 * q));
-        } else if constexpr (KP == 2) {
-            double2 t = __ldg(reinterpret_cast<const double2 *>(p));
-            v[0] = t.x;
-            v[1] = t.y;
-        } else {
-            v[0] = __ldg(p);
-        }
-    }
-};
-
 constexpr int V2_CONSUMER_WARPS = 8;
 constexpr int V2_THREADS = (V2_CONSUMER_WARPS + 1) * 32;
 constexpr int K1_TC = 8;      // entries of a row per ring stage
@@ -230,14 +210,13 @@ struct K1Smem {
     uint64_t full[K1_STAGES], empty[K1_STAGES];
 };
 
-// K1 v2.  x is read from a Float64 copy of the Float32 x table (xd[j][k] = Float64(x[j][k])), so the
-// row sum is one DFMA per (entry, draw): p = sum_j Float64(v) * Float64(x) accumulated in Float64.
+// K1 v2.  Rows of <= 4 entries: k1_short_row, all Float32.  Longer rows: batches of <= 4 products summed in Float32,
+// each batch widened once and added to a Float64 row sum.
 // (EXACT builds keep the v1 kernel, whose products are rounded to Float32 first as in the reference.)
-template <int KP, bool LP, bool WEIGHTED, bool XF32>
+template <int KP, bool LP, bool WEIGHTED>
 __global__ void __launch_bounds__(V2_THREADS, 3)
     k1_sell_fwd_tma(const RowTile *__restrict__ tiles, int n_tiles, const uint32_t *__restrict__ idx,
-                    const float *__restrict__ val, const double *__restrict__ xd, const float *__restrict__ xf,
-                    float *__restrict__ w,
+                    const float *__restrict__ val, const float *__restrict__ xf, float *__restrict__ w,
                     const float *__restrict__ row_weight, double *__restrict__ lp_partial) {
     extern __shared__ __align__(128) unsigned char smraw[];
     K1Smem &sm = *reinterpret_cast<K1Smem *>(smraw);
@@ -280,46 +259,44 @@ __global__ void __launch_bounds__(V2_THREADS, 3)
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const RowTile t = tiles[tile];
         const bool active = r < t.nrows;
-        if constexpr (XF32) {
-            if (t.len <= 4) {  // warp-uniform: the whole tile is one ring item
-                const int stage = item % K1_STAGES;
-                mbar_wait(&sm.full[stage], (item / K1_STAGES) & 1);
-                float pv[KP];
+        if (t.len <= 4) {  // warp-uniform: the whole tile is one ring item
+            const int stage = item % K1_STAGES;
+            mbar_wait(&sm.full[stage], (item / K1_STAGES) & 1);
+            float pv[KP];
 #pragma unroll
-                for (int k = 0; k < KP; ++k) pv[k] = 1.0f;
-                float wt = 1.0f;
-                if (active) {
-                    if (WEIGHTED) wt = row_weight[t.row0 + r];
-                    float *wout = w + (size_t)(t.row0 + r) * KP;
-                    float *pp = LP ? pv : nullptr;
-                    switch (t.len) {
-                        case 1: k1_short_row<KP, 1, WEIGHTED>(sm.idx[stage], sm.val[stage], r, xf, wout, wt, pp); break;
-                        case 2: k1_short_row<KP, 2, WEIGHTED>(sm.idx[stage], sm.val[stage], r, xf, wout, wt, pp); break;
-                        case 3: k1_short_row<KP, 3, WEIGHTED>(sm.idx[stage], sm.val[stage], r, xf, wout, wt, pp); break;
-                        default: k1_short_row<KP, 4, WEIGHTED>(sm.idx[stage], sm.val[stage], r, xf, wout, wt, pp); break;
-                    }
+            for (int k = 0; k < KP; ++k) pv[k] = 1.0f;
+            float wt = 1.0f;
+            if (active) {
+                if (WEIGHTED) wt = row_weight[t.row0 + r];
+                float *wout = w + (size_t)(t.row0 + r) * KP;
+                float *pp = LP ? pv : nullptr;
+                switch (t.len) {
+                    case 1: k1_short_row<KP, 1, WEIGHTED>(sm.idx[stage], sm.val[stage], r, xf, wout, wt, pp); break;
+                    case 2: k1_short_row<KP, 2, WEIGHTED>(sm.idx[stage], sm.val[stage], r, xf, wout, wt, pp); break;
+                    case 3: k1_short_row<KP, 3, WEIGHTED>(sm.idx[stage], sm.val[stage], r, xf, wout, wt, pp); break;
+                    default: k1_short_row<KP, 4, WEIGHTED>(sm.idx[stage], sm.val[stage], r, xf, wout, wt, pp); break;
                 }
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&sm.empty[stage]);
-                ++item;
-                if constexpr (LP) {
-#pragma unroll
-                    for (int k = 0; k < KP; ++k) {
-                        double v = active ? (WEIGHTED ? log((double)pv[k]) * (double)wt : log((double)pv[k])) : 0.0;
-#pragma unroll
-                        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-                        if (lane == 0) sm.lpsm[warp][k] = v;
-                    }
-                    consumer_bar_sync();
-                    if (threadIdx.x < KP) {
-                        double sacc = 0.0;
-                        for (int wi = 0; wi < V2_CONSUMER_WARPS; ++wi) sacc += sm.lpsm[wi][threadIdx.x];
-                        lp_partial[(size_t)tile * KP + threadIdx.x] = sacc;
-                    }
-                    consumer_bar_sync();
-                }
-                continue;
             }
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&sm.empty[stage]);
+            ++item;
+            if constexpr (LP) {
+#pragma unroll
+                for (int k = 0; k < KP; ++k) {
+                    double v = active ? (WEIGHTED ? log((double)pv[k]) * (double)wt : log((double)pv[k])) : 0.0;
+#pragma unroll
+                    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+                    if (lane == 0) sm.lpsm[warp][k] = v;
+                }
+                consumer_bar_sync();
+                if (threadIdx.x < KP) {
+                    double sacc = 0.0;
+                    for (int wi = 0; wi < V2_CONSUMER_WARPS; ++wi) sacc += sm.lpsm[wi][threadIdx.x];
+                    lp_partial[(size_t)tile * KP + threadIdx.x] = sacc;
+                }
+                consumer_bar_sync();
+            }
+            continue;
         }
         double acc[KP];
 #pragma unroll
@@ -329,55 +306,26 @@ __global__ void __launch_bounds__(V2_THREADS, 3)
             mbar_wait(&sm.full[stage], (item / K1_STAGES) & 1);
             const uint32_t tc = min((uint32_t)K1_TC, t.len - t0);
             if (active) {
-                if constexpr (XF32) {
-                    // Float32 x table: a batch of <= 4 products is summed in Float32 (one FFMA each), then
-                    // widened once and added to the Float64 row sum
-                    constexpr int U = 4;
-                    for (uint32_t tt = 0; tt < tc; tt += U) {
-                        float xv[U][KP];
-                        float v[U];
+                constexpr int U = 4;
+                for (uint32_t tt = 0; tt < tc; tt += U) {
+                    float xv[U][KP];
+                    float v[U];
 #pragma unroll
-                        for (int u = 0; u < U; ++u) {
-                            const bool ok = tt + u < tc;
-                            const uint32_t c = ok ? sm.idx[stage][tt + u][r] : 0u;
-                            v[u] = ok ? sm.val[stage][tt + u][r] : 0.0f;
-                            Vec<KP>::ld(xf + (size_t)c * KP, xv[u]);
-                        }
-                        float facc[KP];
-#pragma unroll
-                        for (int k = 0; k < KP; ++k) facc[k] = v[0] * xv[0][k];
-#pragma unroll
-                        for (int u = 1; u < U; ++u)
-#pragma unroll
-                            for (int k = 0; k < KP; ++k) facc[k] = fmaf(v[u], xv[u][k], facc[k]);
-#pragma unroll
-                        for (int k = 0; k < KP; ++k) acc[k] += (double)facc[k];
+                    for (int u = 0; u < U; ++u) {
+                        const bool ok = tt + u < tc;
+                        const uint32_t c = ok ? sm.idx[stage][tt + u][r] : 0u;
+                        v[u] = ok ? sm.val[stage][tt + u][r] : 0.0f;
+                        Vec<KP>::ld(xf + (size_t)c * KP, xv[u]);
                     }
-                } else {
-                    constexpr int U = (KP >= 8) ? 2 : 4;
-                    uint32_t tt = 0;
-                    for (; tt + U <= tc; tt += U) {
-                        double xv[U][KP];
-                        double dv[U];
+                    float facc[KP];
 #pragma unroll
-                        for (int u = 0; u < U; ++u) {
-                            const uint32_t c = sm.idx[stage][tt + u][r];
-                            dv[u] = (double)sm.val[stage][tt + u][r];
-                            VecD<KP>::ld(xd + (size_t)c * KP, xv[u]);
-                        }
+                    for (int k = 0; k < KP; ++k) facc[k] = v[0] * xv[0][k];
 #pragma unroll
-                        for (int u = 0; u < U; ++u)
+                    for (int u = 1; u < U; ++u)
 #pragma unroll
-                            for (int k = 0; k < KP; ++k) acc[k] = fma(dv[u], xv[u][k], acc[k]);
-                    }
-                    for (; tt < tc; ++tt) {
-                        const uint32_t c = sm.idx[stage][tt][r];
-                        const double dv = (double)sm.val[stage][tt][r];
-                        double xv[KP];
-                        VecD<KP>::ld(xd + (size_t)c * KP, xv);
+                        for (int k = 0; k < KP; ++k) facc[k] = fmaf(v[u], xv[u][k], facc[k]);
 #pragma unroll
-                        for (int k = 0; k < KP; ++k) acc[k] = fma(dv, xv[k], acc[k]);
-                    }
+                    for (int k = 0; k < KP; ++k) acc[k] += (double)facc[k];
                 }
             }
             __syncwarp();
@@ -437,7 +385,7 @@ struct K2Smem {
 // segment wi of the item.  FAST: the lane's <= COL_SEG/32 products are accumulated in Float32, then widened
 // and reduced in Float64 (lane -> warp butterfly -> segments of a column inside the CTA -> k2_combine);
 // EXACT: every product is a Float64 FMA.  Fixed order everywhere: deterministic, no atomics.
-template <int KP, bool EXACT, bool PREFETCH>
+template <int KP, bool EXACT>
 __global__ void __launch_bounds__(V2_THREADS, 3)
     k2_csc_grad_tma(const ColSeg *__restrict__ segs, int n_segs, const uint32_t *__restrict__ csc_row,
                     const float *__restrict__ csc_val, const float *__restrict__ w, double *__restrict__ g,
@@ -457,20 +405,17 @@ __global__ void __launch_bounds__(V2_THREADS, 3)
     const int n_items = (n_segs + K2_WARPS - 1) / K2_WARPS;
 
     if (warp == K2_WARPS) {
-        // producer warp.  Lane 0 keeps the ring full; then the whole warp walks the row ids of the item that
-        // landed one iteration earlier and issues L2 prefetches for the w rows the consumers are about to gather:
-        // prefetches hold no registers, so they add memory-level parallelism the register file cannot.
-        int j = 0;
-        uint32_t prev_a0 = 0, prev_cnt = 0;
-        for (int it = blockIdx.x; it < n_items; it += gridDim.x, ++j) {
-            const int stage = j % K2_STAGES;
-            const ColSeg first = segs[it * K2_WARPS];
-            const ColSeg last = segs[min(it * K2_WARPS + K2_WARPS - 1, n_segs - 1)];
-            const uint32_t a0 = first.start & ~3u;
-            const uint32_t cnt = last.start + (last.len & 0xffffu) - a0;
-            const uint32_t bytes = (cnt * 4u + 15u) & ~15u;
-            const uint32_t nseg = (uint32_t)min(K2_WARPS, n_segs - it * K2_WARPS);
-            if (lane == 0) {
+        // ------------------------------ producer warp (one lane)
+        if (lane == 0) {
+            int j = 0;
+            for (int it = blockIdx.x; it < n_items; it += gridDim.x, ++j) {
+                const int stage = j % K2_STAGES;
+                const ColSeg first = segs[it * K2_WARPS];
+                const ColSeg last = segs[min(it * K2_WARPS + K2_WARPS - 1, n_segs - 1)];
+                const uint32_t a0 = first.start & ~3u;
+                const uint32_t cnt = last.start + (last.len & 0xffffu) - a0;
+                const uint32_t bytes = (cnt * 4u + 15u) & ~15u;
+                const uint32_t nseg = (uint32_t)min(K2_WARPS, n_segs - it * K2_WARPS);
                 mbar_wait(&sm.empty[stage], ((j / K2_STAGES) & 1) ^ 1);
                 mbar_expect_tx(&sm.full[stage], 2u * bytes + nseg * (uint32_t)sizeof(ColSeg));
                 bulk_g2s(&sm.seg[stage][0], segs + (size_t)it * K2_WARPS, nseg * (uint32_t)sizeof(ColSeg), &sm.full[stage]);
@@ -479,19 +424,7 @@ __global__ void __launch_bounds__(V2_THREADS, 3)
                     bulk_g2s(&sm.val[stage][0], csc_val + a0, bytes, &sm.full[stage]);
                 }
             }
-            __syncwarp();
-            if (PREFETCH && j > 0) {
-                const int ps = (j - 1) % K2_STAGES;
-                mbar_wait(&sm.full[ps], ((j - 1) / K2_STAGES) & 1);
-                for (uint32_t e = lane; e < prev_cnt; e += 32) {
-                    const uint32_t r = sm.row[ps][e];
-                    asm volatile("prefetch.global.L2 [%0];" ::"l"(w + (size_t)r * KP));
-                }
-            }
-            prev_a0 = a0;
-            prev_cnt = cnt;
         }
-        (void)prev_a0;
         return;
     }
 
@@ -597,7 +530,7 @@ __global__ void k_narrow_f64(const double *__restrict__ in, float *__restrict__ 
 }
 
 template <int KP>
-int launch_k1_t(polee_handle *h, const float *x, const double *xd, float *w, bool want_lp, double *lp_partial) {
+int launch_k1_t(polee_handle *h, const float *x, float *w, bool want_lp, double *lp_partial) {
     if (h->n_row_tiles == 0) return POLEE_OK;
     const bool wt = h->row_weight != nullptr;
     if (h->o.exact_accumulation) {
@@ -615,17 +548,11 @@ int launch_k1_t(polee_handle *h, const float *x, const double *xd, float *w, boo
     }
     const int grid = std::min(h->n_row_tiles, h->num_sms * 3);
     const size_t smem = sizeof(K1Smem);
-    static const bool x_f64 = getenv("POLEE_K1_X") && !strcmp(getenv("POLEE_K1_X"), "f64");
-#define K1_LAUNCH3(LPF, WF, XF)                                                                                    \
-    do {                                                                                                           \
-        allow_max_smem(k1_sell_fwd_tma<KP, LPF, WF, XF>);                                                              \
-        k1_sell_fwd_tma<KP, LPF, WF, XF><<<grid, V2_THREADS, smem, h->stream>>>(                                   \
-            h->row_tiles, h->n_row_tiles, h->sell_idx, h->sell_val, xd, x, w, h->row_weight, lp_partial);          \
-    } while (0)
-#define K1_LAUNCH2(LPF, WF)                                \
-    do {                                                   \
-        if (x_f64) K1_LAUNCH3(LPF, WF, false);             \
-        else K1_LAUNCH3(LPF, WF, true);                    \
+#define K1_LAUNCH2(LPF, WF)                                                                                 \
+    do {                                                                                                    \
+        allow_max_smem(k1_sell_fwd_tma<KP, LPF, WF>);                                                       \
+        k1_sell_fwd_tma<KP, LPF, WF><<<grid, V2_THREADS, smem, h->stream>>>(                                \
+            h->row_tiles, h->n_row_tiles, h->sell_idx, h->sell_val, x, w, h->row_weight, lp_partial);       \
     } while (0)
     if (want_lp) {
         if (wt) K1_LAUNCH2(true, true); else K1_LAUNCH2(true, false);
@@ -633,7 +560,6 @@ int launch_k1_t(polee_handle *h, const float *x, const double *xd, float *w, boo
         if (wt) K1_LAUNCH2(false, true); else K1_LAUNCH2(false, false);
     }
 #undef K1_LAUNCH2
-#undef K1_LAUNCH3
     return POLEE_OK;
 }
 
@@ -644,19 +570,14 @@ int launch_k2_t(polee_handle *h, const float *w, double *g) {
         static const int k2_ctas = getenv("POLEE_K2_CTAS") ? atoi(getenv("POLEE_K2_CTAS")) : 3;
         const int grid = std::min(n_items, h->num_sms * k2_ctas);
         const size_t smem = sizeof(K2Smem);
-        // the producer-warp L2 prefetch of w rows measured SLOWER on B200 (0.508 vs 0.483 ms at C3): opt-in only
-        static const bool no_pf = !(getenv("POLEE_K2_PREFETCH") && !strcmp(getenv("POLEE_K2_PREFETCH"), "1"));
-#define K2_LAUNCH(EX, PF)                                                                                           \
-    do {                                                                                                            \
-        allow_max_smem(k2_csc_grad_tma<KP, EX, PF>);                                                               \
-        k2_csc_grad_tma<KP, EX, PF><<<grid, V2_THREADS, smem, h->stream>>>(h->segs, h->n_segs, h->csc_row, h->csc_val, \
-                                                                           w, g, h->seg_partial);                  \
+#define K2_LAUNCH(EX)                                                                                           \
+    do {                                                                                                        \
+        allow_max_smem(k2_csc_grad_tma<KP, EX>);                                                                \
+        k2_csc_grad_tma<KP, EX><<<grid, V2_THREADS, smem, h->stream>>>(h->segs, h->n_segs, h->csc_row, h->csc_val, \
+                                                                       w, g, h->seg_partial);                  \
     } while (0)
-        if (h->o.exact_accumulation) {
-            if (no_pf) K2_LAUNCH(true, false); else K2_LAUNCH(true, true);
-        } else {
-            if (no_pf) K2_LAUNCH(false, false); else K2_LAUNCH(false, true);
-        }
+        if (h->o.exact_accumulation) K2_LAUNCH(true);
+        else K2_LAUNCH(false);
 #undef K2_LAUNCH
     }
     if (h->n_multi > 0) {
@@ -679,9 +600,9 @@ int launch_k2_t(polee_handle *h, const float *w, double *g) {
         default: return h->fail(POLEE_EINVAL, "unsupported number of MC draws (1..16)"); \
     }
 
-int launch_k1(polee_handle *h, const float *x, const double *xd, float *w, bool want_lp, double *lp_partial, int KP) {
+int launch_k1(polee_handle *h, const float *x, float *w, bool want_lp, double *lp_partial, int KP) {
     int rc = POLEE_OK;
-    DISPATCH_KP(KP, rc = launch_k1_t<KPC>(h, x, xd, w, want_lp, lp_partial));
+    DISPATCH_KP(KP, rc = launch_k1_t<KPC>(h, x, w, want_lp, lp_partial));
     return rc;
 }
 
@@ -689,12 +610,6 @@ int launch_k2(polee_handle *h, const float *w, double *g, int KP) {
     int rc = POLEE_OK;
     DISPATCH_KP(KP, rc = launch_k2_t<KPC>(h, w, g));
     return rc;
-}
-
-int launch_widen_x(polee_handle *h, const float *x, double *xd, int KP) {
-    const size_t count = (size_t)h->n * KP;
-    k_widen_f32<<<(unsigned)std::min<size_t>((count + 255) / 256, 4096), 256, 0, h->stream>>>(x, xd, count);
-    return POLEE_OK;
 }
 
 // the gradient crosses NVLink as Float32 (half the bytes of the all-reduce): narrow before, widen after

@@ -44,8 +44,7 @@ struct Affine {  // G -> a * G + b
 template <int KP>
 __global__ void __launch_bounds__(CH_THREADS)
     k3c_chain_fwd(int64_t n, const int32_t *__restrict__ chain_leaf, const double *__restrict__ ys,
-                  double *__restrict__ us /* [2n-1][KP] by node id */, float *__restrict__ x, double *__restrict__ xd,
-                  int clamp_x, const float *__restrict__ efflen, double *__restrict__ S_partial, int want_ladj,
+                  double *__restrict__ us /* [2n-1][KP] by node id */, float *__restrict__ x, int clamp_x, const float *__restrict__ efflen, double *__restrict__ S_partial, int want_ladj,
                   double *__restrict__ ladj_partial) {
     __shared__ double sm[CH_THREADS];
     const int k = blockIdx.x;  // draw
@@ -66,7 +65,6 @@ __global__ void __launch_bounds__(CH_THREADS)
             xv = (float)d;
         }
         x[(size_t)leaf * KP + k] = xv;
-        xd[(size_t)leaf * KP + k] = (double)xv;
         if (efflen) sacc += (double)__fdiv_rn(xv, efflen[leaf]);
     };
     for (int64_t j = s; j < e; ++j) {
@@ -162,8 +160,7 @@ __global__ void __launch_bounds__(CH_THREADS)
     }
 
 int launch_chain_fwd(polee_handle *h, int KP, int clamp_x, const float *eff, double *Sp, int want_ladj, double *ladj_tree) {
-    DISPATCH_KP(KP, (k3c_chain_fwd<KPC><<<KP, CH_THREADS, 0, h->stream>>>(h->td.n, h->td.chain_leaf, h->ys, h->us, h->x, h->xd,
-                                                                        clamp_x, eff, Sp, want_ladj, ladj_tree)));
+    DISPATCH_KP(KP, (k3c_chain_fwd<KPC><<<KP, CH_THREADS, 0, h->stream>>>(h->td.n, h->td.chain_leaf, h->ys, h->us, h->x, clamp_x, eff, Sp, want_ladj, ladj_tree)));
     return POLEE_OK;
 }
 

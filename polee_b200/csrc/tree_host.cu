@@ -30,11 +30,10 @@ int pad_k(int K) {
 }
 
 static void make_sched(const std::vector<std::vector<int32_t>> &bins_nodes, const std::vector<int32_t> &level_of,
-                       TreeSchedHost &out, int &max_levels) {
+                       TreeSchedHost &out) {
     out.bin_lvl_ptr.assign(1, 0);
     out.lvl_off.clear();
     out.sch_node.clear();
-    max_levels = 0;
     size_t total = 0;
     for (const auto &bn : bins_nodes) total += bn.size();
     out.sch_node.reserve(total);
@@ -51,7 +50,6 @@ static void make_sched(const std::vector<std::vector<int32_t>> &bins_nodes, cons
         for (int32_t v : bn) out.sch_node[base + cur[level_of[v]]++] = v;
         for (int l = 0; l <= nl; ++l) out.lvl_off.push_back(base + cnt[l]);
         out.bin_lvl_ptr.push_back((int32_t)out.lvl_off.size());
-        max_levels = std::max(max_levels, nl);
     }
 }
 
@@ -144,8 +142,6 @@ std::string TreeHost::build_from_lrf(int64_t n_, const int32_t *left, const int3
     // ---- root -> node paths, grouped (see TreeHost); not needed when the DFS-run kernel serves the tree
     ganc_ptr.clear(); ganc.clear(); gcp.clear(); nsuf_ptr.clear(); nsuf.clear();
     max_ganc = max_gsuf = 0;
-    static const bool dfs_off = getenv("POLEE_TREE_FWD") && strcmp(getenv("POLEE_TREE_FWD"), "dfs") != 0;
-    if (dfs_off) { preorder = false; dnodes.clear(); drun_anc_ptr.clear(); drun_anc.clear(); dcta_k0.clear(); }
     if (!preorder) {
         int64_t total = 0;
         for (int64_t i = 0; i < N; ++i) total += depth[i];
@@ -223,14 +219,7 @@ std::string TreeHost::build_from_lrf(int64_t n_, const int32_t *left, const int3
         caterpillar = nodes[N - 1].leaf >= 0;
     }
 
-    // ---- cut: top = nodes whose subtree exceeds bin_nodes (the DFS-range backward kernel works on spans of
-    // DFS_CTA_NODES nodes: trees that qualify for it are cut there)
-    // (measured at C3: 80 us against 47.5 us for the level-synchronous bottom kernel -- 11 warps per SM at 75 KB of shared
-    // memory per CTA, profiles/r02_tree_bwd_dfs_v1_ncu_c3.csv -- so it is an experiment: POLEE_TREE_BWD=dfs turns it on)
-    const char *bwd_env = getenv("POLEE_TREE_BWD");  // read per tree, so that a test can switch it
-    const bool bwd_on = bwd_env && !strcmp(bwd_env, "dfs");
-    const bool want_dfs_bwd = preorder && bwd_on;
-    if (want_dfs_bwd) bin_nodes = DFS_CTA_NODES;
+    // ---- cut: top = nodes whose subtree exceeds bin_nodes
     std::vector<char> is_top(N, 0);
     std::vector<int32_t> top_list;
     for (int64_t i = 0; i < N; ++i)
@@ -238,7 +227,6 @@ std::string TreeHost::build_from_lrf(int64_t n_, const int32_t *left, const int3
             is_top[i] = 1;
             top_list.push_back((int32_t)i);
         }
-    top_nodes = (int)top_list.size();
 
     std::vector<int32_t> level_of(N, 0);
     std::vector<std::vector<int32_t>> bins;
@@ -272,14 +260,13 @@ std::string TreeHost::build_from_lrf(int64_t n_, const int32_t *left, const int3
         }
     }
     mark("cut + bins");
-    int ml = 0;
-    make_sched(bins, level_of, bottom, ml);
+    make_sched(bins, level_of, bottom);
     std::vector<std::vector<int32_t>> tb;
     if (!top_list.empty()) {
         tb.push_back(top_list);
         for (int32_t v : top_list) level_of[v] = depth[v];
     }
-    make_sched(tb, level_of, top, ml);
+    make_sched(tb, level_of, top);
 
     mark("global-memory schedules");
     // ---- schedule-order records for the shared-memory kernels
@@ -349,128 +336,7 @@ std::string TreeHost::build_from_lrf(int64_t n_, const int32_t *left, const int3
             out.max_bin_levels = std::max(out.max_bin_levels, nl);
         }
     };
-    // ---- DFS-range backward schedule (see common.cuh)
-    dfs_bwd = false;
-    bnodes.clear(); bspans.clear(); t2nodes.clear(); t2_lvl.clear();
-    bwd_max_nk = bwd_max_leaves = bwd_max_slots = bwd_max_stack = bwd_max_t2 = bwd_max_lev = 0;
-    if (want_dfs_bwd) {
-        dfs_bwd = true;
-        bnodes.assign(N + 2, DNode{-1, 0xffffffffu});  // meta all ones: not a node of any span (a top node, padding)
-        std::vector<int32_t> kbefore(N + 1, 0);  // internal nodes before node i
-        for (int64_t i = 0; i < N; ++i) kbefore[i + 1] = kbefore[i] + (nodes[i].leaf < 0 ? 1 : 0);
-        // spans: consecutive bottom roots (whole subtrees, each a contiguous index range) while the range stays short
-        std::vector<std::pair<int32_t, int32_t>> spans;
-        for (int64_t r = 0; r < N; ++r) {
-            if (is_top[r] || (parent[r] >= 0 && !is_top[parent[r]])) continue;  // r is a bottom root
-            const int32_t e = (int32_t)(r + size[r]);
-            if (spans.empty() || e - spans.back().first > DFS_CTA_NODES) spans.emplace_back((int32_t)r, e);
-            else spans.back().second = e;
-            r = e - 1;  // the nodes of this subtree are no roots
-        }
-        std::vector<int8_t> tier(N, 3);
-        std::vector<int32_t> lslot(N, -1), lvl2(N, 0);
-        for (const auto &sp : spans) {
-            const int32_t s0 = sp.first, s1 = sp.second;
-            BSpan B{};
-            B.s0 = s0; B.nn = s1 - s0;
-            B.k0 = kbefore[s0]; B.nk = kbefore[s1] - kbefore[s0];
-            // tiers
-            for (int32_t i = s0; i < s1; ++i) {
-                if (is_top[i]) { tier[i] = 3; continue; }
-                const int32_t run_end = std::min(s1, s0 + ((i - s0) / DFS_BRUN + 1) * DFS_BRUN);
-                tier[i] = i + size[i] <= run_end ? 1 : 2;
-            }
-            // CTA slots: G of the non-top nodes whose parent is a tier-2 node
-            int32_t nslots = 0, nleaves = 0;
-            for (int32_t i = s0; i < s1; ++i) {
-                if (tier[i] == 3) continue;
-                const int ptier = (parent[i] < 0 || is_top[parent[i]]) ? 3 : tier[parent[i]];
-                if (ptier == 2) lslot[i] = nslots++;
-                uint32_t meta = 0;
-                if (nodes[i].leaf < 0 && tier[i] == 1) meta |= BN_T1INT;
-                if (tier[i] == 1 && ptier >= 2 && parent[i] >= 0) {
-                    meta |= BN_EXPORT;
-                    if (ptier == 3) {
-                        if (slot_of[i] >= 0) meta |= BN_GLOBAL | ((uint32_t)slot_of[i] << 14);
-                        else meta &= ~BN_EXPORT;  // the root of the whole tree: nobody reads its G
-                    } else {
-                        meta |= (uint32_t)lslot[i] << 14;
-                    }
-                }
-                if (nodes[i].leaf >= 0) meta |= (uint32_t)(nleaves++) << 3;
-                bnodes[i].k_or_leaf = nodes[i].leaf >= 0 ? -1 - nodes[i].leaf : nodes[i].k;
-                bnodes[i].meta = meta;
-            }
-            if (nleaves > 2047 || nslots >= (1 << 17) || n_slots >= (1 << 17)) dfs_bwd = false;
-            // the stack a run needs
-            for (int32_t r0 = s0; r0 < s1; r0 += DFS_BRUN) {
-                int sp_now = 0;
-                for (int32_t i = std::min(s1, r0 + DFS_BRUN) - 1; i >= r0; --i) {
-                    if (tier[i] == 3 || (nodes[i].leaf < 0 && tier[i] != 1)) continue;
-                    if (nodes[i].leaf < 0) sp_now -= 2;
-                    if (!(bnodes[i].meta & BN_EXPORT)) ++sp_now;
-                    bwd_max_stack = std::max(bwd_max_stack, sp_now);
-                }
-            }
-            // tier 2: levels (children have larger indices), records in level order
-            B.t2_off = (int32_t)t2nodes.size();
-            int nlev = 0;
-            std::vector<int32_t> t2list;
-            for (int32_t i = s1 - 1; i >= s0; --i) {
-                if (tier[i] != 2) continue;
-                int l = 0;
-                for (int32_t c : {nodes[i].left, nodes[i].right})
-                    if (tier[c] == 2) l = std::max(l, lvl2[c] + 1);
-                lvl2[i] = l;
-                nlev = std::max(nlev, l + 1);
-                t2list.push_back(i);
-            }
-            std::vector<int32_t> cnt(nlev + 1, 0);
-            for (int32_t i : t2list) cnt[lvl2[i] + 1]++;
-            for (int l = 0; l < nlev; ++l) cnt[l + 1] += cnt[l];
-            B.lvl_off = (int32_t)t2_lvl.size();
-            B.nlev = nlev;
-            for (int l = 0; l <= nlev; ++l) t2_lvl.push_back(cnt[l]);
-            t2nodes.resize(t2nodes.size() + t2list.size());
-            std::vector<int32_t> cur(cnt.begin(), cnt.end());
-            for (auto it = t2list.rbegin(); it != t2list.rend(); ++it) {  // ascending node order inside a level
-                const int32_t i = *it;
-                T2Node t;
-                t.k = nodes[i].k;
-                t.sl = lslot[nodes[i].left];
-                t.sr = lslot[nodes[i].right];
-                const int ptier = (parent[i] < 0 || is_top[parent[i]]) ? 3 : 2;
-                t.out = ptier == 2 ? lslot[i] : (slot_of[i] >= 0 ? -1 - slot_of[i] : INT32_MIN);
-                t2nodes[B.t2_off + cur[lvl2[i]]++] = t;
-            }
-            B.nt2 = (int32_t)t2list.size();
-            bspans.push_back(B);
-            bwd_max_nk = std::max(bwd_max_nk, B.nk);
-            bwd_max_leaves = std::max(bwd_max_leaves, nleaves);
-            bwd_max_slots = std::max(bwd_max_slots, nslots);
-            bwd_max_t2 = std::max(bwd_max_t2, B.nt2);
-            bwd_max_lev = std::max(bwd_max_lev, nlev);
-        }
-        if (bwd_max_stack > 32) dfs_bwd = false;
-        {   // shared memory of a CTA with 4 draws (the most the kernel takes), see dfs_bwd_smem in tree_kernels.cu
-            const size_t kpc = 4, threads = (size_t)DFS_BRUNS * kpc;
-            const size_t smem = (size_t)std::max(bwd_max_stack, 1) * threads * 8 + 2 * (size_t)std::max(bwd_max_nk, 1) * kpc * 8 +
-                                (size_t)std::max(bwd_max_slots, 1) * kpc * 8 + (size_t)std::max(bwd_max_t2, 1) * sizeof(T2Node) +
-                                (size_t)DFS_CTA_NODES * sizeof(DNode) + (size_t)std::max(bwd_max_leaves, 1) * kpc * 4 +
-                                4 * (size_t)(bwd_max_lev + 2);
-            if (smem > 200 * 1024) dfs_bwd = false;
-        }
-        if (!dfs_bwd) { bnodes.clear(); bspans.clear(); t2nodes.clear(); t2_lvl.clear(); }
-    }
-
-    mark("dfs-range backward");
-    if (dfs_bwd) {  // the level-synchronous bottom kernels are not used for this tree
-        s_bottom = SSchedHost();
-        s_bottom.bin_off.assign(1, 0);
-        s_bottom.bin_lvl_ptr.assign(1, 0);
-    } else {
-        make_ssched(bins, false, s_bottom);
-    }
+    make_ssched(bins, false, s_bottom);
     make_ssched(tb, true, s_top);
     mark("shared-memory schedules");
     return "";
@@ -516,9 +382,6 @@ void TreeDev::release() {
     nsuf = nullptr;
     polee::dfree(dnodes); polee::dfree(drun_anc_ptr); polee::dfree(drun_anc); polee::dfree(dcta_k0);
     dnodes = nullptr; drun_anc_ptr = drun_anc = nullptr; dcta_k0 = nullptr;
-    polee::dfree(bnodes); polee::dfree(bspans); polee::dfree(t2nodes); polee::dfree(t2_lvl);
-    bnodes = nullptr; bspans = nullptr; t2nodes = nullptr; t2_lvl = nullptr;
-    n_bspans = bwd_max_nk = bwd_max_leaves = bwd_max_slots = bwd_max_stack = bwd_max_t2 = bwd_max_lev = 0;
     dfs_ctas = dfs_max_nk = 0;
     n_groups = max_ganc = max_gsuf = 0;
     for (SSchedDev *s : {&s_top, &s_bottom}) {
@@ -526,13 +389,11 @@ void TreeDev::release() {
         polee::dfree(s->bin_lvl_ptr);
         polee::dfree(s->lvl_off);
         polee::dfree(s->recs);
-        polee::dfree(s->bin_desc);
         *s = SSchedDev();
     }
     nodes = nullptr;
     n = N = 0;
     n_slots = 0;
-    smem_path = false;
 }
 
 static cudaError_t up(const std::vector<int32_t> &v, int32_t **d) {
@@ -557,10 +418,6 @@ std::string upload_tree(const TreeHost &th, TreeDev &td) {
         if (e == cudaSuccess) e = up(hs[s]->lvl_off, &ds[s]->lvl_off);
         if (e == cudaSuccess) e = up(hs[s]->sch_node, &ds[s]->sch_node);
         ds[s]->nbins = hs[s]->nbins();
-        int ml = 0;
-        for (int b = 0; b < hs[s]->nbins(); ++b)
-            ml = std::max(ml, hs[s]->bin_lvl_ptr[b + 1] - hs[s]->bin_lvl_ptr[b] - 1);
-        ds[s]->max_levels = ml;
     }
     const SSchedHost *hss[2] = {&th.s_top, &th.s_bottom};
     SSchedDev *dss[2] = {&td.s_top, &td.s_bottom};
@@ -573,16 +430,6 @@ std::string upload_tree(const TreeHost &th, TreeDev &td) {
             e = polee::dmalloc((void **)&dss[s]->recs, bytes);
             if (e == cudaSuccess && !hss[s]->recs.empty())
                 e = cudaMemcpy(dss[s]->recs, hss[s]->recs.data(), hss[s]->recs.size() * sizeof(SNode), cudaMemcpyHostToDevice);
-        }
-        if (e == cudaSuccess) {
-            std::vector<int32_t> desc;
-            for (int b = 0; b < hss[s]->nbins(); ++b) {
-                desc.push_back(hss[s]->bin_off[b]);
-                desc.push_back(hss[s]->bin_off[b + 1] - hss[s]->bin_off[b]);
-                desc.push_back(hss[s]->bin_lvl_ptr[b]);
-                desc.push_back(hss[s]->bin_lvl_ptr[b + 1] - 1 - hss[s]->bin_lvl_ptr[b]);
-            }
-            e = up(desc, &dss[s]->bin_desc);
         }
         dss[s]->nbins = hss[s]->nbins();
         dss[s]->max_bin_nodes = hss[s]->max_bin_nodes;
@@ -617,20 +464,6 @@ std::string upload_tree(const TreeHost &th, TreeDev &td) {
         td.dfs_ctas = (int)th.dcta_k0.size() - 1;
         td.dfs_max_nk = th.dfs_max_nk;
         td.n_groups = std::max(td.n_groups, td.dfs_ctas);  // sizes the per-CTA partial sums (S, ladj)
-    }
-    if (e == cudaSuccess && th.dfs_bwd) {
-        auto upv = [&](const void *src, size_t bytes, void **dst) {
-            cudaError_t ee = polee::dmalloc(dst, std::max<size_t>(bytes, 16));
-            if (ee == cudaSuccess && bytes) ee = cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice);
-            return ee;
-        };
-        e = upv(th.bnodes.data(), sizeof(DNode) * th.bnodes.size(), (void **)&td.bnodes);
-        if (e == cudaSuccess) e = upv(th.bspans.data(), sizeof(BSpan) * th.bspans.size(), (void **)&td.bspans);
-        if (e == cudaSuccess) e = upv(th.t2nodes.data(), sizeof(T2Node) * th.t2nodes.size(), (void **)&td.t2nodes);
-        if (e == cudaSuccess) e = upv(th.t2_lvl.data(), 4 * th.t2_lvl.size(), (void **)&td.t2_lvl);
-        td.n_bspans = (int)th.bspans.size();
-        td.bwd_max_nk = th.bwd_max_nk; td.bwd_max_leaves = th.bwd_max_leaves; td.bwd_max_slots = th.bwd_max_slots;
-        td.bwd_max_stack = th.bwd_max_stack; td.bwd_max_t2 = th.bwd_max_t2; td.bwd_max_lev = th.bwd_max_lev;
     }
     td.n_slots = th.n_slots;
     td.caterpillar = th.caterpillar;

@@ -19,7 +19,6 @@
 
 #include <climits>
 #include <cstdlib>
-#include <cstring>
 
 #include "common.cuh"
 #include "device_utils.cuh"
@@ -74,8 +73,7 @@ template <int KP, int THREADS>
 __global__ void __launch_bounds__(THREADS)
     k3_tree_fwd(const int32_t *__restrict__ bin_lvl_ptr, const int32_t *__restrict__ lvl_off,
                 const int32_t *__restrict__ sch_node, const TreeNode *__restrict__ nodes,
-                const double *__restrict__ ys, double *__restrict__ us, float *__restrict__ x, double *__restrict__ xd,
-                int clamp_x,
+                const double *__restrict__ ys, double *__restrict__ us, float *__restrict__ x, int clamp_x,
                 const float *__restrict__ efflen, double *__restrict__ S_partial, int part_base, int want_ladj,
                 double *__restrict__ ladj_partial) {
     __shared__ double sm[THREADS];
@@ -99,7 +97,6 @@ __global__ void __launch_bounds__(THREADS)
                     xv = (float)d;
                 }
                 x[(size_t)nd.leaf * KP + k] = xv;
-                xd[(size_t)nd.leaf * KP + k] = (double)xv;
                 if (efflen) sacc = __dadd_rn(sacc, (double)__fdiv_rn(xv, efflen[nd.leaf]));
             } else {
                 const double y = ys[(size_t)nd.k * KP + k];
@@ -291,7 +288,7 @@ template <int KP, int KPC, int THREADS, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB)
     k3s_tree_fwd(const int32_t *__restrict__ bin_off, const int32_t *__restrict__ bin_lvl_ptr,
                  const int32_t *__restrict__ lvl_off, const SNode *__restrict__ recs, const double *__restrict__ ys,
-                 double *__restrict__ root_us, float *__restrict__ x, double *__restrict__ xd, int clamp_x,
+                 double *__restrict__ root_us, float *__restrict__ x, int clamp_x,
                  const float *__restrict__ efflen, double *__restrict__ S_partial, int part_base, int want_ladj,
                  double *__restrict__ ladj_partial) {
     extern __shared__ __align__(16) unsigned char smraw[];
@@ -359,7 +356,6 @@ __global__ void __launch_bounds__(THREADS, MINB)
                     xv = (float)d;
                 }
                 x[(size_t)leaf * KP + k] = xv;
-                xd[(size_t)leaf * KP + k] = (double)xv;
                 if (efflen) sacc = __dadd_rn(sacc, (double)__fdiv_rn(xv, __int_as_float(r.left)));
             }
         }
@@ -496,7 +492,7 @@ __global__ void __launch_bounds__(PATH_SLOTS *KP, 2048 / (PATH_SLOTS * KP) > 16 
     k3p_tree_fwd(int64_t N, const TreeNode *__restrict__ nodes, const uint32_t *__restrict__ ganc_ptr,
                  const uint32_t *__restrict__ ganc, const uint32_t *__restrict__ gcp, const uint32_t *__restrict__ nsuf_ptr,
                  const uint16_t *__restrict__ nsuf, const double *__restrict__ ys, double *__restrict__ us_k,
-                 float *__restrict__ x, double *__restrict__ xd, int clamp_x, const float *__restrict__ efflen,
+                 float *__restrict__ x, int clamp_x, const float *__restrict__ efflen,
                  double *__restrict__ S_partial, int want_ladj, double *__restrict__ ladj_partial) {
     constexpr int THREADS = PATH_SLOTS * KP, NPT = PATH_GROUP / PATH_SLOTS;
     extern __shared__ __align__(16) unsigned char smraw[];
@@ -558,7 +554,6 @@ __global__ void __launch_bounds__(PATH_SLOTS *KP, 2048 / (PATH_SLOTS * KP) > 16 
                 xv = (float)d;
             }
             x[(size_t)nd[j].leaf * KP + k] = xv;
-            xd[(size_t)nd[j].leaf * KP + k] = (double)xv;
             if (efflen) sacc = __dadd_rn(sacc, (double)__fdiv_rn(xv, ef[j]));
         } else {
             us_k[(size_t)nd[j].k * KP + k] = u;
@@ -583,7 +578,7 @@ template <int KP>
 __global__ void __launch_bounds__(DFS_RUNS_PER_CTA *KP)
     k3d_tree_fwd(int64_t N, const DNode *__restrict__ dnodes, const uint32_t *__restrict__ run_anc_ptr,
                  const uint32_t *__restrict__ run_anc, const int32_t *__restrict__ cta_k0, const double *__restrict__ ys,
-                 double *__restrict__ us_k, float *__restrict__ x, double *__restrict__ xd, int clamp_x, int want_ladj,
+                 double *__restrict__ us_k, float *__restrict__ x, int clamp_x, int want_ladj,
                  double *__restrict__ ladj_partial, int stack_levels, int max_nk) {
     constexpr int THREADS = DFS_RUNS_PER_CTA * KP, RS = DFS_RUN + 2;  // record stride of a run: 16-byte aligned, 4 banks apart
     extern __shared__ __align__(16) unsigned char smraw[];
@@ -679,153 +674,9 @@ __global__ void __launch_bounds__(DFS_RUNS_PER_CTA *KP)
             float xv = fmaxf((float)u, (float)1e-16);
             if (clamp_x) xv = fminf(fmaxf(xv, (float)1e-10), 1.0f);
             x[(size_t)leaf * KP + k] = xv;
-            if (xd) xd[(size_t)leaf * KP + k] = (double)xv;
         }
     }
     if (want_ladj) block_reduce_kc<KP, THREADS>(lacc, red, ladj_partial + (size_t)blockIdx.x * KP);
-}
-
-// One node of transform_gradients! (ptt.jl:167-209; WITH_LADJ false: transform_gradients_no_ladj!, :217-251): the same
-// operations in the same association as k3s_tree_bwd, so whoever calls it produces the reference's bits.
-template <bool WITH_LADJ>
-__device__ __forceinline__ float2 bwd_node(double y, double ui, float2 gl, float2 gr, double &yg) {
-    const double omy = __dsub_rn(1.0, y);
-    float2 out;
-    out.x = (float)__dadd_rn(__dmul_rn(y, (double)gl.x), __dmul_rn(omy, (double)gr.x));
-    if (WITH_LADJ) {
-        const float d = __fsub_rn(__fadd_rn(gl.x, gl.y), __fadd_rn(gr.x, gr.y));
-        yg = (double)(float)__dmul_rn(ui, (double)d);
-        out.y = (float)__dadd_rn(__dadd_rn(__ddiv_rn(1.0, ui), __dmul_rn(y, (double)gl.y)), __dmul_rn(omy, (double)gr.y));
-    } else {
-        const float d = __fsub_rn(gl.x, gr.x);
-        yg = __dmul_rn(ui, (double)d);
-        out.y = 0.0f;
-    }
-    return out;
-}
-
-// transform_gradients! for trees in DFS pre-order, bottom part (see common.cuh, "DFS-range backward").  A CTA owns a span
-// of <= DFS_CTA_NODES consecutive nodes (whole bottom subtrees) and KPC draws; thread = (run of DFS_BRUN nodes, draw).
-//   staging : the span's records, the y and u of its internal nodes (consecutive k: contiguous rows of ys / us), the
-//             tier-2 records, and the leaves' gradients g - adj / S (likelihood.jl:105) rounded to Float32
-//   tier 1  : every thread walks its run backwards -- the reference's own order -- with a LIFO stack in shared memory:
-//             a leaf pushes its G, an internal node whose subtree lies inside the run pops its children (right on top)
-//             and pushes its own; a node whose parent is not tier 1 stores its G in a CTA slot (or, under a top node, in
-//             the global exchange array) instead of pushing it.  No barrier, no idle level sweeps.
-//   tier 2  : the span's remaining nodes (ancestors of run boundaries: ~13 % of a balanced tree), level by level from
-//             the CTA slots.
-// The top nodes follow in the one-CTA-per-draw kernel (k3s_tree_bwd over s_top), as before.
-template <int KP, int KPC, bool WITH_LADJ>
-__global__ void __launch_bounds__(DFS_BRUNS *KPC)
-    k3d_tree_bwd(const BSpan *__restrict__ spans, const DNode *__restrict__ bnodes, const T2Node *__restrict__ t2nodes,
-                 const int32_t *__restrict__ t2_lvl, const double *__restrict__ ys, const double *__restrict__ us_k,
-                 const double *__restrict__ g, const float *__restrict__ efflen_adj, const double *__restrict__ S,
-                 float2 *__restrict__ root_G, double *__restrict__ ygrad, double *__restrict__ xgrad_out, int stack_levels,
-                 int max_nk, int max_leaves, int max_slots, int max_t2, int max_lev) {
-    constexpr int THREADS = DFS_BRUNS * KPC;
-    extern __shared__ __align__(16) unsigned char smraw[];
-    float2 *stack = reinterpret_cast<float2 *>(smraw);                                  // [stack_levels][THREADS]
-    double *ys_s = reinterpret_cast<double *>(stack + (size_t)stack_levels * THREADS);  // [max_nk][KPC]
-    double *us_s = ys_s + (size_t)max_nk * KPC;                                         // [max_nk][KPC]
-    float2 *slot_s = reinterpret_cast<float2 *>(us_s + (size_t)max_nk * KPC);           // [max_slots][KPC]
-    T2Node *t2_s = reinterpret_cast<T2Node *>(slot_s + (size_t)max_slots * KPC);        // [max_t2]
-    DNode *rec_s = reinterpret_cast<DNode *>(t2_s + max_t2);                            // [DFS_CTA_NODES]
-    float *gl_s = reinterpret_cast<float *>(rec_s + DFS_CTA_NODES);                     // [max_leaves][KPC]
-    int *lvl_s = reinterpret_cast<int *>(gl_s + (size_t)max_leaves * KPC);              // [max_lev + 1]
-    const int kk = threadIdx.x % KPC, rl = threadIdx.x / KPC, k = blockIdx.y * KPC + kk;
-    const BSpan B = spans[blockIdx.x];
-
-    // ---- staging
-    for (int p = threadIdx.x; p < B.nn; p += THREADS) rec_s[p] = bnodes[B.s0 + p];
-    for (int q = threadIdx.x; q < B.nt2; q += THREADS) t2_s[q] = t2nodes[B.t2_off + q];
-    for (int l = threadIdx.x; l <= B.nlev; l += THREADS) lvl_s[l] = t2_lvl[B.lvl_off + l];
-    {
-        const double *ysrc = ys + (size_t)B.k0 * KP + blockIdx.y * KPC, *usrc = us_k + (size_t)B.k0 * KP + blockIdx.y * KPC;
-        const int cnt = B.nk * KPC;
-#pragma unroll 4
-        for (int idx = threadIdx.x; idx < cnt; idx += THREADS) {
-            const int r = idx / KPC, c = idx - r * KPC;
-            ys_s[idx] = ysrc[(size_t)r * KP + c];
-            us_s[idx] = usrc[(size_t)r * KP + c];
-        }
-    }
-    __syncthreads();
-    // leaves: g - adj / S, four independent gathers per thread in flight
-    const double Sk = efflen_adj ? S[k] : 1.0;
-    for (int base = rl; base < B.nn; base += 4 * DFS_BRUNS) {
-        double gv[4];
-        float adj[4];
-        int leaf[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int p = base + u * DFS_BRUNS;
-            leaf[u] = (p < B.nn && rec_s[p].k_or_leaf < 0 && rec_s[p].meta != 0xffffffffu) ? -1 - rec_s[p].k_or_leaf : -1;
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            gv[u] = 0.0; adj[u] = 0.0f;
-            if (leaf[u] >= 0) {
-                gv[u] = g[(size_t)leaf[u] * KP + k];
-                if (efflen_adj) adj[u] = efflen_adj[leaf[u]];
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            if (leaf[u] < 0) continue;
-            const int p = base + u * DFS_BRUNS;
-            double v = gv[u];
-            if (efflen_adj) v = __dsub_rn(v, __ddiv_rn((double)adj[u], Sk));  // likelihood.jl:105
-            if (xgrad_out) xgrad_out[(size_t)leaf[u] * KP + k] = v;
-            gl_s[((rec_s[p].meta >> 3) & 0x7ffu) * KPC + kk] = (float)v;
-        }
-    }
-    __syncthreads();
-
-    // ---- tier 1: the run, backwards
-    {
-        const int p0 = rl * DFS_BRUN, p1 = p0 + DFS_BRUN < B.nn ? p0 + DFS_BRUN : B.nn;
-        float2 *st = stack + threadIdx.x;
-        int sp = 0;
-        for (int p = p1 - 1; p >= p0; --p) {
-            const DNode r = rec_s[p];
-            float2 G;
-            if (r.k_or_leaf < 0) {
-                if (r.meta == 0xffffffffu) continue;  // a top node inside the span
-                G = make_float2(gl_s[((r.meta >> 3) & 0x7ffu) * KPC + kk], 0.0f);
-            } else {
-                if (!(r.meta & BN_T1INT)) continue;   // tier 2
-                const float2 gr = st[(size_t)(sp - 1) * THREADS], gl = st[(size_t)(sp - 2) * THREADS];
-                sp -= 2;
-                const int kr = r.k_or_leaf - B.k0;
-                double yg;
-                G = bwd_node<WITH_LADJ>(ys_s[kr * KPC + kk], us_s[kr * KPC + kk], gl, gr, yg);
-                ygrad[(size_t)r.k_or_leaf * KP + k] = yg;
-            }
-            if (r.meta & BN_EXPORT) {
-                if (r.meta & BN_GLOBAL) root_G[(size_t)(r.meta >> 14) * KP + k] = G;
-                else slot_s[(r.meta >> 14) * KPC + kk] = G;
-            } else {
-                st[(size_t)sp * THREADS] = G;
-                ++sp;
-            }
-        }
-    }
-    __syncthreads();
-
-    // ---- tier 2: level by level from the CTA slots
-    for (int l = 0; l < B.nlev; ++l) {
-        for (int q = lvl_s[l] + rl; q < lvl_s[l + 1]; q += DFS_BRUNS) {
-            const T2Node t = t2_s[q];
-            const int kr = t.k - B.k0;
-            double yg;
-            const float2 G = bwd_node<WITH_LADJ>(ys_s[kr * KPC + kk], us_s[kr * KPC + kk], slot_s[t.sl * KPC + kk],
-                                                 slot_s[t.sr * KPC + kk], yg);
-            ygrad[(size_t)t.k * KP + k] = yg;
-            if (t.out >= 0) slot_s[t.out * KPC + kk] = G;
-            else if (t.out != INT32_MIN) root_G[(size_t)(-1 - t.out) * KP + k] = G;
-        }
-        __syncthreads();
-    }
 }
 
 // S_k = sum_j x_jk / efflen_j (effective_length_jacobian_adjustment!, likelihood.jl:96-100: Float32 quotients, Float64
@@ -1120,13 +971,13 @@ __global__ void __launch_bounds__(256) k3_elbo(int K, int KP, const double *__re
 #define CK(expr) POLEE_CUDA_CHECK(h, expr)
 
 void release_work_buffers(polee_handle *h) {
-    void *ptrs[] = {h->zs0, h->zs, h->ys, h->ygrad, h->us, h->G, h->root_us, h->root_G, h->x, h->xd, h->w, h->g, h->seg_partial, h->S_partial,
+    void *ptrs[] = {h->zs0, h->zs, h->ys, h->ygrad, h->us, h->G, h->root_us, h->root_G, h->x, h->w, h->g, h->seg_partial, h->S_partial,
                     h->S, h->lp_partial, h->ladj_partial, h->grad_out, h->ft_partial, h->ft_lvl2, h->g32,
                     h->ec_partial, h->ec_lvl2, h->ec_lp_partial};
     for (void *p : ptrs) polee::dfree(p);
     h->ft_partial = nullptr; h->ft_lvl2 = nullptr; h->g32 = nullptr;
     h->ec_partial = h->ec_lvl2 = h->ec_lp_partial = nullptr;
-    h->zs0 = h->zs = nullptr; h->ys = h->ygrad = h->us = nullptr; h->G = nullptr; h->x = h->w = nullptr; h->xd = nullptr; h->root_us = nullptr; h->root_G = nullptr;
+    h->zs0 = h->zs = nullptr; h->ys = h->ygrad = h->us = nullptr; h->G = nullptr; h->x = h->w = nullptr; h->root_us = nullptr; h->root_G = nullptr;
     h->g = h->seg_partial = h->S_partial = h->S = h->lp_partial = h->ladj_partial = nullptr;
     h->grad_out = nullptr;
     h->work_KP = 0;
@@ -1153,7 +1004,6 @@ int ensure_work_buffers(polee_handle *h, int KP) {
     CK(polee::dmalloc((void **)&h->root_us, sizeof(double) * std::max(h->td.n_slots, 1) * KP));
     CK(polee::dmalloc((void **)&h->root_G, sizeof(float2) * std::max(h->td.n_slots, 1) * KP));
     CK(polee::dmalloc((void **)&h->x, sizeof(float) * n * KP));
-    CK(polee::dmalloc((void **)&h->xd, sizeof(double) * n * KP));
     CK(polee::dmalloc((void **)&h->g, sizeof(double) * (n + 1) * KP));
     CK(polee::dmalloc((void **)&h->S_partial, sizeof(double) * h->n_tree_ctas * KP));
     CK(polee::dmalloc((void **)&h->S, sizeof(double) * KP));
@@ -1225,40 +1075,17 @@ int launch_reparam_fwd(polee_handle *h, int KP, int K, const float *noise, int64
 }
 
 constexpr int S_TOP_THREADS = 1024;
-
-template <typename F>
-static void set_smem_attr(F func, size_t bytes) {
-    (void)bytes;
-    allow_max_smem(func);  // per-function, process-wide: see common.cuh
-}
+// bottom forests: draws per CTA and min CTAs per SM of the TREE_THREADS-thread CTAs (KP = 8: the shape that measured
+// fastest, profiles/r02_k3_sweep.log)
+constexpr int bottom_kpc(int KP) { return KP == 8 ? 4 : (KP < 8 ? KP : 8); }
+constexpr int bottom_minb(int KP) { return KP == 8 ? 3 : 2; }
 
 // the path-product forward kernel (k3p_tree_fwd) is used whenever the tree's root paths were built (not for very deep
-// trees) and the shared-memory backward kernels, which read its u, are; POLEE_TREE_FWD=levels keeps the level kernels
+// trees) and the shared-memory backward kernels, which read its u, are
 static bool smem_path_ok(const polee_handle *h, int KP);
 static bool chain_path(const polee_handle *h);
 static bool path_fwd_ok(const polee_handle *h) {
-    static const bool off = getenv("POLEE_TREE_FWD") && !strcmp(getenv("POLEE_TREE_FWD"), "levels");
-    return !off && h->td.ganc_ptr != nullptr && !chain_path(h) && smem_path_ok(h, h->work_KP);
-}
-// the DFS-range backward kernel (k3d_tree_bwd) goes with the DFS-run forward (it reads its u by k)
-static int dfs_bwd_kpc(int KP) { return KP < 4 ? KP : 4; }
-static size_t dfs_bwd_smem(const polee_handle *h, int KP) {
-    const TreeDev &td = h->td;
-    const size_t kpc = (size_t)dfs_bwd_kpc(KP), threads = (size_t)DFS_BRUNS * kpc;
-    return (size_t)std::max(td.bwd_max_stack, 1) * threads * 8 + 2 * (size_t)std::max(td.bwd_max_nk, 1) * kpc * 8 +
-           (size_t)std::max(td.bwd_max_slots, 1) * kpc * 8 + (size_t)std::max(td.bwd_max_t2, 1) * sizeof(T2Node) +
-           (size_t)DFS_CTA_NODES * sizeof(DNode) + (size_t)std::max(td.bwd_max_leaves, 1) * kpc * 4 + 4 * (size_t)(td.bwd_max_lev + 2);
-}
-
-
-// bottom-forest launch variants (draws per CTA, threads, min CTAs/SM); POLEE_TREE_VARIANT picks one at run time
-static int tree_variant() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("POLEE_TREE_VARIANT");
-        v = e ? atoi(e) : 0;
-    }
-    return v;
+    return h->td.ganc_ptr != nullptr && !chain_path(h) && smem_path_ok(h, h->work_KP);
 }
 // the DFS-run forward kernel (k3d_tree_fwd): trees in DFS pre-order of moderate depth (tree_host.cu builds its inputs
 // only then); like the path-product kernel it leaves u by k for the shared-memory backward kernels
@@ -1268,33 +1095,10 @@ static size_t dfs_fwd_smem(const polee_handle *h, int KP) {
            (size_t)DFS_RUNS_PER_CTA * (DFS_RUN + 2) * sizeof(DNode);
 }
 static bool dfs_fwd_ok(const polee_handle *h) {
-    // a tree cut for the DFS-range backward kernel has no level-synchronous bottom schedule: both or neither
     return h->td.dnodes != nullptr && !chain_path(h) && smem_path_ok(h, h->work_KP) && h->work_KP <= 16 &&
-           dfs_fwd_smem(h, h->work_KP) <= 200 * 1024 &&
-           (h->td.bnodes == nullptr || dfs_bwd_smem(h, h->work_KP) <= 200 * 1024);
+           dfs_fwd_smem(h, h->work_KP) <= 200 * 1024;
 }
-static bool dfs_bwd_ok(const polee_handle *h) { return h->td.bnodes != nullptr && dfs_fwd_ok(h); }
 static bool fwd_leaves_us_by_k(const polee_handle *h) { return dfs_fwd_ok(h) || path_fwd_ok(h); }
-template <int KP, int KPC, int THREADS, int MINB>
-static void launch_fwd_bottom_v(polee_handle *h, int clamp_x, const float *eff, double *Sp, int want_ladj, double *ladj_tree) {
-    const TreeDev &td = h->td;
-    const size_t smem = (size_t)td.s_bottom.max_bin_nodes * (sizeof(SNode) + 16 * KPC) + 4 * (td.s_bottom.max_bin_levels + 2);
-    auto fn = k3s_tree_fwd<KP, KPC, THREADS, MINB>;
-    set_smem_attr(fn, smem);
-    fn<<<dim3(td.s_bottom.nbins, KP / KPC), THREADS, smem, h->stream>>>(
-        td.s_bottom.bin_off, td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->root_us, h->x, h->xd,
-        clamp_x, eff, Sp, 1, want_ladj, ladj_tree);
-}
-template <int KP, int KPC, int THREADS, int MINB, bool WITH_LADJ>
-static void launch_bwd_bottom_v(polee_handle *h, const float *adj, double *xgrad_out) {
-    const TreeDev &td = h->td;
-    const size_t smem = (size_t)td.s_bottom.max_bin_nodes * (sizeof(SNode) + 24 * KPC) + 4 * (td.s_bottom.max_bin_levels + 2);
-    auto fn = k3s_tree_bwd<KP, KPC, THREADS, MINB, WITH_LADJ>;
-    set_smem_attr(fn, smem);
-    fn<<<dim3(td.s_bottom.nbins, KP / KPC), THREADS, smem, h->stream>>>(
-        td.s_bottom.bin_off, td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->root_us, h->root_G, h->g,
-        adj, h->S, h->ygrad, xgrad_out, fwd_leaves_us_by_k(h) ? h->us : nullptr);
-}
 
 template <int KP>
 static int launch_tree_fwd_smem(polee_handle *h, int clamp_x, const float *eff, double *Sp, int want_ladj, double *ladj_tree) {
@@ -1302,21 +1106,19 @@ static int launch_tree_fwd_smem(polee_handle *h, int clamp_x, const float *eff, 
     if (td.s_top.nbins > 0) {
         const size_t smem = (size_t)td.s_top.max_bin_nodes * (sizeof(SNode) + 16) + 4 * (td.s_top.max_bin_levels + 2);
         auto fn = k3s_tree_fwd<KP, 1, S_TOP_THREADS, 1>;
-        set_smem_attr(fn, smem);
+        allow_max_smem(fn);  // per-function, process-wide: see common.cuh
         fn<<<dim3(td.s_top.nbins, KP), S_TOP_THREADS, smem, h->stream>>>(
-            td.s_top.bin_off, td.s_top.bin_lvl_ptr, td.s_top.lvl_off, td.s_top.recs, h->ys, h->root_us, h->x, h->xd, clamp_x,
+            td.s_top.bin_off, td.s_top.bin_lvl_ptr, td.s_top.lvl_off, td.s_top.recs, h->ys, h->root_us, h->x, clamp_x,
             eff, Sp, 0, want_ladj, ladj_tree);
     }
     if (td.s_bottom.nbins > 0) {
-        if constexpr (KP == 8) {
-            const int v = tree_variant();
-            if (v == 1) launch_fwd_bottom_v<8, 8, 512, 1>(h, clamp_x, eff, Sp, want_ladj, ladj_tree);
-            else if (v == 2) launch_fwd_bottom_v<8, 2, 256, 6>(h, clamp_x, eff, Sp, want_ladj, ladj_tree);
-            else if (v == 3) launch_fwd_bottom_v<8, 8, 256, 2>(h, clamp_x, eff, Sp, want_ladj, ladj_tree);
-            else launch_fwd_bottom_v<8, 4, 256, 3>(h, clamp_x, eff, Sp, want_ladj, ladj_tree);
-        } else {
-            launch_fwd_bottom_v<KP, (KP < 8 ? KP : 8), 256, 2>(h, clamp_x, eff, Sp, want_ladj, ladj_tree);
-        }
+        constexpr int KPC = bottom_kpc(KP);
+        const size_t smem = (size_t)td.s_bottom.max_bin_nodes * (sizeof(SNode) + 16 * KPC) + 4 * (td.s_bottom.max_bin_levels + 2);
+        auto fn = k3s_tree_fwd<KP, KPC, TREE_THREADS, bottom_minb(KP)>;
+        allow_max_smem(fn);
+        fn<<<dim3(td.s_bottom.nbins, KP / KPC), TREE_THREADS, smem, h->stream>>>(
+            td.s_bottom.bin_off, td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->root_us, h->x,
+            clamp_x, eff, Sp, 1, want_ladj, ladj_tree);
     }
     return POLEE_OK;
 }
@@ -1324,33 +1126,23 @@ static int launch_tree_fwd_smem(polee_handle *h, int clamp_x, const float *eff, 
 template <int KP, bool WITH_LADJ>
 static int launch_tree_bwd_smem(polee_handle *h, const float *adj, double *xgrad_out) {
     const TreeDev &td = h->td;
-    if (dfs_bwd_ok(h)) {
-        constexpr int KPC = KP < 4 ? KP : 4;
-        const size_t smem = dfs_bwd_smem(h, KP);
-        auto fn = k3d_tree_bwd<KP, KPC, WITH_LADJ>;
-        set_smem_attr(fn, smem);
-        fn<<<dim3(td.n_bspans, KP / KPC), DFS_BRUNS * KPC, smem, h->stream>>>(
-            td.bspans, td.bnodes, td.t2nodes, td.t2_lvl, h->ys, h->us, h->g, adj, h->S, h->root_G, h->ygrad, xgrad_out,
-            std::max(td.bwd_max_stack, 1), std::max(td.bwd_max_nk, 1), std::max(td.bwd_max_leaves, 1),
-            std::max(td.bwd_max_slots, 1), std::max(td.bwd_max_t2, 1), td.bwd_max_lev);
-    } else if (td.s_bottom.nbins > 0) {
-        if constexpr (KP == 8) {
-            const int v = tree_variant();
-            if (v == 1) launch_bwd_bottom_v<8, 8, 512, 1, WITH_LADJ>(h, adj, xgrad_out);
-            else if (v == 2) launch_bwd_bottom_v<8, 2, 256, 6, WITH_LADJ>(h, adj, xgrad_out);
-            else if (v == 3) launch_bwd_bottom_v<8, 8, 256, 2, WITH_LADJ>(h, adj, xgrad_out);
-            else launch_bwd_bottom_v<8, 4, 256, 3, WITH_LADJ>(h, adj, xgrad_out);
-        } else {
-            launch_bwd_bottom_v<KP, (KP < 8 ? KP : 8), 256, 2, WITH_LADJ>(h, adj, xgrad_out);
-        }
+    const double *us_k = fwd_leaves_us_by_k(h) ? h->us : nullptr;
+    if (td.s_bottom.nbins > 0) {
+        constexpr int KPC = bottom_kpc(KP);
+        const size_t smem = (size_t)td.s_bottom.max_bin_nodes * (sizeof(SNode) + 24 * KPC) + 4 * (td.s_bottom.max_bin_levels + 2);
+        auto fn = k3s_tree_bwd<KP, KPC, TREE_THREADS, bottom_minb(KP), WITH_LADJ>;
+        allow_max_smem(fn);
+        fn<<<dim3(td.s_bottom.nbins, KP / KPC), TREE_THREADS, smem, h->stream>>>(
+            td.s_bottom.bin_off, td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->root_us, h->root_G, h->g,
+            adj, h->S, h->ygrad, xgrad_out, us_k);
     }
     if (td.s_top.nbins > 0) {
         const size_t smem = (size_t)td.s_top.max_bin_nodes * (sizeof(SNode) + 24) + 4 * (td.s_top.max_bin_levels + 2);
         auto fn = k3s_tree_bwd<KP, 1, S_TOP_THREADS, 1, WITH_LADJ>;
-        set_smem_attr(fn, smem);
+        allow_max_smem(fn);
         fn<<<dim3(td.s_top.nbins, KP), S_TOP_THREADS, smem, h->stream>>>(
             td.s_top.bin_off, td.s_top.bin_lvl_ptr, td.s_top.lvl_off, td.s_top.recs, h->ys, h->root_us, h->root_G, h->g, adj,
-            h->S, h->ygrad, xgrad_out, fwd_leaves_us_by_k(h) ? h->us : nullptr);
+            h->S, h->ygrad, xgrad_out, us_k);
     }
     return POLEE_OK;
 }
@@ -1362,8 +1154,6 @@ static bool smem_path_ok(const polee_handle *h, int KP) {
     const TreeDev &td = h->td;
     const int KPC = KP < 8 ? KP : 8;
     const size_t limit = 200 * 1024;
-    const char *env = getenv("POLEE_TREE_PATH");
-    if (env && !strcmp(env, "global")) return false;
     return (size_t)td.s_bottom.max_bin_nodes * (sizeof(SNode) + 24 * KPC) + 4 * (td.s_bottom.max_bin_levels + 2) <= limit &&
            (size_t)td.s_top.max_bin_nodes * (sizeof(SNode) + 24) + 4 * (td.s_top.max_bin_levels + 2) <= limit;
 }
@@ -1382,12 +1172,10 @@ int launch_tree_fwd(polee_handle *h, int KP, int clamp_x, int want_S, int want_l
     double *Sp = want_S ? h->S_partial : nullptr;
     if (chain_path(h)) return launch_chain_fwd(h, KP, clamp_x, eff, Sp, want_ladj, ladj_tree);
     if (dfs_fwd_ok(h)) {
-        // the Float64 copy of x is the gather table of the split layout's K1 only
-        double *xd = (!h->have_matrix || ((h->gm > 0 || h->ec_tasks == 0) && !h->fused)) ? h->xd : nullptr;
         const size_t smem = dfs_fwd_smem(h, KP);
         if (smem > 40 * 1024) DISPATCH_KP(KP, allow_max_smem(k3d_tree_fwd<KPC>));
         DISPATCH_KP(KP, (k3d_tree_fwd<KPC><<<td.dfs_ctas, DFS_RUNS_PER_CTA * KPC, smem, h->stream>>>(
-                            td.N, td.dnodes, td.drun_anc_ptr, td.drun_anc, td.dcta_k0, h->ys, h->us, h->x, xd, clamp_x,
+                            td.N, td.dnodes, td.drun_anc_ptr, td.drun_anc, td.dcta_k0, h->ys, h->us, h->x, clamp_x,
                             want_ladj, ladj_tree, td.max_depth + 2, (std::max(td.dfs_max_nk, 1) + 1) & ~1)));
         h->S_deferred = want_S != 0;  // launch_mid adds S = sum_j x_j / efflen_j (k3_leaf_S) beside the likelihood pass
         return POLEE_OK;
@@ -1396,24 +1184,24 @@ int launch_tree_fwd(polee_handle *h, int KP, int clamp_x, int want_S, int want_l
         const size_t smem = (size_t)td.max_ganc * (16 * KP + 2) + 16 + 2 * (size_t)td.max_gsuf;
         if (smem > 40 * 1024) DISPATCH_KP(KP, allow_max_smem(k3p_tree_fwd<KPC>));
         DISPATCH_KP(KP, (k3p_tree_fwd<KPC><<<td.n_groups, PATH_SLOTS * KPC, smem, h->stream>>>(
-                            td.N, td.nodes, td.ganc_ptr, td.ganc, td.gcp, td.nsuf_ptr, td.nsuf, h->ys, h->us, h->x, h->xd, clamp_x,
+                            td.N, td.nodes, td.ganc_ptr, td.ganc, td.gcp, td.nsuf_ptr, td.nsuf, h->ys, h->us, h->x, clamp_x,
                             eff, Sp, want_ladj, ladj_tree)));
         return POLEE_OK;
     }
-    if (smem_path_ok(h, KP) && td.bnodes == nullptr) {
+    if (smem_path_ok(h, KP)) {
         int rc = POLEE_OK;
         DISPATCH_KP(KP, rc = launch_tree_fwd_smem<KPC>(h, clamp_x, eff, Sp, want_ladj, ladj_tree));
         return rc;
     }
     if (td.top.nbins > 0) {
         DISPATCH_KP(KP, (k3_tree_fwd<KPC, TOP_THREADS><<<td.top.nbins, TOP_THREADS, 0, h->stream>>>(
-                            td.top.bin_lvl_ptr, td.top.lvl_off, td.top.sch_node, td.nodes, h->ys, h->us, h->x, h->xd, clamp_x,
+                            td.top.bin_lvl_ptr, td.top.lvl_off, td.top.sch_node, td.nodes, h->ys, h->us, h->x, clamp_x,
                             eff, Sp, 0, want_ladj, ladj_tree)));
     }
     if (td.bottom.nbins > 0) {
         DISPATCH_KP(KP, (k3_tree_fwd<KPC, TREE_THREADS><<<td.bottom.nbins, TREE_THREADS, 0, h->stream>>>(
                             td.bottom.bin_lvl_ptr, td.bottom.lvl_off, td.bottom.sch_node, td.nodes, h->ys, h->us, h->x,
-                            h->xd, clamp_x, eff, Sp, 1, want_ladj, ladj_tree)));
+                            clamp_x, eff, Sp, 1, want_ladj, ladj_tree)));
     }
     return POLEE_OK;
 }
@@ -1436,7 +1224,7 @@ int launch_tree_bwd(polee_handle *h, int KP, bool with_ladj, bool apply_efflen, 
     const TreeDev &td = h->td;
     const float *adj = apply_efflen ? h->efflen_adj : nullptr;
     if (chain_path(h)) return launch_chain_bwd(h, KP, with_ladj, adj, xgrad_out);
-    if (smem_path_ok(h, KP) && (td.bnodes == nullptr || dfs_bwd_ok(h))) {
+    if (smem_path_ok(h, KP)) {
         int rc = POLEE_OK;
         if (with_ladj) {
             DISPATCH_KP(KP, (rc = launch_tree_bwd_smem<KPC, true>(h, adj, xgrad_out)));
@@ -1471,8 +1259,7 @@ static void preload_tree_kernels_kp() {
     cudaFuncGetAttributes(&a, k3_elem<KP>);
     cudaFuncGetAttributes(&a, k3d_tree_fwd<KP>);
     cudaFuncGetAttributes(&a, k3_leaf_S<KP>);
-    if constexpr (KP == 8) cudaFuncGetAttributes(&a, k3s_tree_bwd<8, 4, 256, 3, true>);
-    else cudaFuncGetAttributes(&a, k3s_tree_bwd<KP, (KP < 8 ? KP : 8), 256, 2, true>);
+    cudaFuncGetAttributes(&a, k3s_tree_bwd<KP, bottom_kpc(KP), TREE_THREADS, bottom_minb(KP), true>);
     cudaFuncGetAttributes(&a, k3s_tree_bwd<KP, 1, S_TOP_THREADS, 1, true>);
     cudaGetLastError();
 }

@@ -81,17 +81,20 @@ def _trees(fx):
     from polee_b200 import synth
     from polee_b200.api import sequential_tree
     return {"fixture": (fx.parent_idxs, fx.js), "sequential": sequential_tree(fx.n),
-            "random": synth.random_tree(fx.n, 3), "balanced": synth.balanced_tree(fx.n)}
+            "random": synth.random_tree(fx.n, 3), "balanced": synth.balanced_tree(fx.n),
+            # large trees: several bottom bins and a top part
+            "balanced_20001": synth.balanced_tree(20001), "random_6000": synth.random_tree(6000, 9)}
 
 
-@pytest.mark.parametrize("tree", ["fixture", "sequential", "random", "balanced"])
+@pytest.mark.parametrize("tree", ["fixture", "sequential", "random", "balanced", "balanced_20001", "random_6000"])
 def test_tree_forward_backward_bit_exact(pb, fx, oracle, tree):
     pi, js = _trees(fx)[tree]
+    n = (len(pi) + 1) // 2
     K = 4
     rng = np.random.default_rng(1)
     lo = 0.3 if tree == "sequential" else 0.01       # keep a depth-312 product inside the Float32 range
-    ys = rng.uniform(lo, 0.99, (K, fx.n - 1))
-    x_grad = rng.normal(size=(K, fx.n)) * 1000
+    ys = rng.uniform(lo, 0.99, (K, n - 1))
+    x_grad = rng.normal(size=(K, n)) * 1000
     t = pb.PolyaTreeTransform(pi, js)
     to = oracle.PTT(pi, js)
     xs, ladj = t.transform(ys, compute_ladj=True)
@@ -104,7 +107,7 @@ def test_tree_forward_backward_bit_exact(pb, fx, oracle, tree):
         assert np.array_equal(yg[k], to.transform_gradients(ys[k], x_grad[k]), equal_nan=True)
         assert np.array_equal(yg0[k], to.transform_gradients_no_ladj(ys[k], x_grad[k]).astype(np.float32), equal_nan=True)
     # transform!(inverse_transform!(x)) = x   (KAT 1 of SURVEY 8c)
-    x = rng.dirichlet(np.ones(fx.n)).astype(np.float32)
+    x = rng.dirichlet(np.ones(n)).astype(np.float32)
     y_inv, ladj_inv = t.inverse_transform(x)
     yo, lo_ = to.inverse_transform(x)
     # y: one Float64 add and one divide per node in the reference's association -> the same bits; ladj: the device's logf
@@ -353,15 +356,15 @@ def test_optimize_ptt(pb, fx, oracle, exact):
     xo = oracle.fit_optimize_ptt(fx.m, fx.n, fx.colptr, fx.rowval, fx.nzval, fx.efflens, steps)
     h = pb.Handle(approx=1, num_steps=steps, exact_accumulation=exact)
     h.set_sample(_sample(pb, fx))
-    xd = h.fit_optimize_ptt()
+    x_dev = h.fit_optimize_ptt()
     h.close()
-    assert abs(xd.astype(np.float64).sum() - 1.0) < 1e-4
+    assert abs(x_dev.astype(np.float64).sum() - 1.0) < 1e-4
     M = oracle.Model(fx.m, fx.n, fx.colptr, fx.rowval, fx.nzval)
-    lp_d, _ = M.log_likelihood(xd, gradonly=False)
+    lp_d, _ = M.log_likelihood(x_dev, gradonly=False)
     lp_o, _ = M.log_likelihood(xo, gradonly=False)
     assert abs(lp_d - lp_o) <= 1e-4 * abs(lp_o)
     big = xo > 1e-4
-    assert np.median(np.abs(xd[big] - xo[big]) / xo[big]) < (1e-3 if exact else 1e-2)
+    assert np.median(np.abs(x_dev[big] - xo[big]) / xo[big]) < (1e-3 if exact else 1e-2)
 
 
 @pytest.mark.parametrize("exact", [0, 1])
@@ -372,9 +375,9 @@ def test_optimize_ptt_first_steps_tight(pb, fx, oracle, exact):
         xo = oracle.fit_optimize_ptt(fx.m, fx.n, fx.colptr, fx.rowval, fx.nzval, fx.efflens, steps)
         h = pb.Handle(approx=1, num_steps=steps, exact_accumulation=exact)
         h.set_sample(_sample(pb, fx))
-        xd = h.fit_optimize_ptt()
+        x_dev = h.fit_optimize_ptt()
         h.close()
-        err = np.abs(xd.astype(np.float64) - xo) / np.maximum(xo, 1e-30)
+        err = np.abs(x_dev.astype(np.float64) - xo) / np.maximum(xo, 1e-30)
         # the first ADAM step moves every coordinate by ~ +-lr g / (|g| + 1e-8): coordinates whose gradient is ~ 0 are
         # sensitive to its last bits, hence a looser bound on the maximum than on the bulk
         assert np.median(err) <= 1e-6 and err.max() <= 2e-4, (steps, np.median(err), err.max())
@@ -505,11 +508,11 @@ def test_optimize_ptt_large_sequential(pb, small_synth, oracle):
         os.environ["POLEE_CHAIN_MIN_NODES"] = env
         h = pb.Handle(approx=1, num_steps=steps)
         h.set_sample(sample)
-        xd = h.fit_optimize_ptt()
+        x_dev = h.fit_optimize_ptt()
         h.close()
-        lp_d, _ = M.log_likelihood(xd, gradonly=False)
+        lp_d, _ = M.log_likelihood(x_dev, gradonly=False)
         assert abs(lp_d - lp_o) <= 2e-4 * abs(lp_o), env
-        assert abs(xd.astype(np.float64).sum() - 1.0) < 1e-4
+        assert abs(x_dev.astype(np.float64).sum() - 1.0) < 1e-4
     os.environ.pop("POLEE_CHAIN_MIN_NODES")
 
 
@@ -674,42 +677,3 @@ def test_exact_factorization_on_device(pb, fx, small_synth, oracle):
         h1.close()
         assert relerr(lp1, lp0) <= 1e-10 and relerr(g1, g0) <= 1e-6
     assert dup[0] > 2 * comp.m * 0.9                                  # the synthetic case really was ~2.5x redundant
-
-
-@pytest.mark.gpu
-def test_dfs_range_backward_experiment_bit_exact(pb, fx, small_synth, oracle, monkeypatch):
-    """The opt-in DFS-range tree backward kernel (POLEE_TREE_BWD=dfs, k3d_tree_bwd: per-thread runs with a LIFO stack,
-    run-crossing nodes level by level from CTA slots, the top part as before) produces the reference's bits, on trees
-    with several spans and a top part, for both ladj variants and through a whole fit (leaf effective-length term)."""
-    from polee_b200 import synth
-    monkeypatch.setenv("POLEE_TREE_BWD", "dfs")
-    rng = np.random.default_rng(5)
-    for name, (pi, js), n in (("balanced", synth.balanced_tree(20001), 20001), ("random", synth.random_tree(6000, 9), 6000),
-                               ("fixture", (fx.parent_idxs, fx.js), fx.n)):
-        t = pb.PolyaTreeTransform(pi, js)
-        info = t.handle.layout_info()
-        assert info["tree_bwd_dfs"] == 1 and (info["tree_bwd_spans"] >= 2 or n < 1000), (name, info)
-        to = oracle.PTT(pi, js)
-        for K in (4, 8):
-            ys = rng.uniform(0.01, 0.99, (K, n - 1))
-            x_grad = rng.normal(size=(K, n)) * 1000
-            t.transform(ys, compute_ladj=False)
-            yg = t.transform_gradients(ys, x_grad)
-            yg0 = t.transform_gradients_no_ladj(ys, x_grad)
-            for k in range(K):
-                to.transform(ys[k], True)   # transform_gradients! reads the us transform! left behind (ptt.jl:167-170)
-                want = to.transform_gradients(ys[k], x_grad[k])
-                assert np.all(np.isfinite(want)) and np.array_equal(yg[k], want), (name, K, k)
-                assert np.array_equal(yg0[k], to.transform_gradients_no_ladj(ys[k], x_grad[k]).astype(np.float32)), (name, K, k)
-    # a whole fit: identical parameters with either backward engine
-    sample, tree = _synth_sample(pb, small_synth), small_synth["tree"]
-    fits = []
-    for engine in ("dfs", "levels"):
-        monkeypatch.setenv("POLEE_TREE_BWD", engine)
-        h = pb.Handle(num_mc_samples=6, num_steps=10, seed=7)
-        h.set_sample(sample, None, tree)
-        assert h.layout_info()["tree_bwd_dfs"] == (1 if engine == "dfs" else 0)
-        fits.append(h.fit())
-        h.close()
-    for k in ("mu", "omega", "alpha"):
-        assert np.array_equal(fits[0][k], fits[1][k]), k

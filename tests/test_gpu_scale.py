@@ -23,7 +23,6 @@ EXACT_MODE = {"exact": 1, "ec64": 2}   # opts.exact_accumulation (include/polee_
 
 def _layout_handle(pb, layout, monkeypatch, K, m, n, colptr, rowval, nzval):
     monkeypatch.delenv("POLEE_LAYOUT", raising=False)
-    monkeypatch.delenv("POLEE_EC_MATH", raising=False)
     for k, v in LAYOUTS[layout].items():
         monkeypatch.setenv(k, v)
     h = pb.Handle(num_mc_samples=K, num_steps=3, exact_accumulation=EXACT_MODE.get(layout, 0))

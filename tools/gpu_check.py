@@ -80,8 +80,8 @@ print('elbo first/last', rd['elbo'][:2], ro['elbo'][:2], rd['elbo'][-1], ro['elb
 t0 = time.time(); rd = pb.approximate_likelihood(pb.LogitSkewNormalPTTApprox(), sample, tree_topology=(pi, js)); print('default 500-step fit s', time.time() - t0)
 mu_ref = np.fromfile(g + 'fixture_prep_mu.f32', np.float32); print('corr mu vs reference prep.h5', np.corrcoef(rd['mu'], mu_ref)[0, 1])
 xo = O.fit_optimize_ptt(m, n, colptr, rowval, nzval, eff, 100)
-h = pb.Handle(approx=1, num_steps=100); h.set_sample(sample); xd = h.fit_optimize_ptt(); h.close()
-print('optimize_ptt rel', rel(xd, xo), xd.sum(), xo.sum())
+h = pb.Handle(approx=1, num_steps=100); h.set_sample(sample); x_dev = h.fit_optimize_ptt(); h.close()
+print('optimize_ptt rel', rel(x_dev, xo), x_dev.sum(), xo.sum())
 # hsb
 l, r, f = pb.make_inverse_ptt_params(pi, js)
 yl = rng.normal(0, 2, (5, n - 1)).astype(np.float32)

@@ -22,9 +22,8 @@ static uint64_t tree_hash(const polee::TreeHost &t) {
         mix(&s->max_bin_nodes, 4); mix(&s->max_bin_levels, 4);
     }
     mixv(t.chain_leaf); mixv(t.ganc_ptr); mixv(t.ganc); mixv(t.gcp); mixv(t.nsuf_ptr); mixv(t.nsuf);
-    mixv(t.bnodes); mixv(t.bspans); mixv(t.t2nodes); mixv(t.t2_lvl); mixv(t.dnodes); mixv(t.drun_anc_ptr); mixv(t.drun_anc); mixv(t.dcta_k0);
-    const int sc[] = {t.n_slots, (int)t.caterpillar, t.top_nodes, t.max_depth, t.max_ganc, t.max_gsuf, (int)t.preorder, (int)t.dfs_bwd,
-                      t.bwd_max_nk, t.bwd_max_leaves, t.bwd_max_slots, t.bwd_max_stack, t.bwd_max_t2, t.bwd_max_lev, t.dfs_max_nk};
+    mixv(t.dnodes); mixv(t.drun_anc_ptr); mixv(t.drun_anc); mixv(t.dcta_k0);
+    const int sc[] = {t.n_slots, (int)t.caterpillar, t.max_depth, t.max_ganc, t.max_gsuf, (int)t.preorder, t.dfs_max_nk};
     mix(sc, sizeof sc);
     return g_h;
 }
@@ -42,8 +41,8 @@ int main(int argc, char **argv) {
         auto t0 = std::chrono::steady_clock::now();
         std::string e = th.build_from_parents(n, buf.data(), buf.data() + N, 512);
         auto t1 = std::chrono::steady_clock::now();
-        printf("rep %d: %.2f ms  err='%s' preorder=%d dfs_bwd=%d hash=%016llx\n", rep,
-               std::chrono::duration<double, std::milli>(t1 - t0).count(), e.c_str(), (int)th.preorder, (int)th.dfs_bwd,
+        printf("rep %d: %.2f ms  err='%s' preorder=%d hash=%016llx\n", rep,
+               std::chrono::duration<double, std::milli>(t1 - t0).count(), e.c_str(), (int)th.preorder,
                (unsigned long long)tree_hash(th));
     }
     return 0;
