@@ -223,6 +223,18 @@ int polee_hsb_device(const polee_hsb_plan *plan, int64_t B, const float *d_y_log
 int polee_inv_hsb_device(const polee_hsb_plan *plan, int64_t B, const float *d_x, double *d_y, float *d_ladj, void *stream);
 int polee_inv_hsb_grad_device(const polee_hsb_plan *plan, int64_t B, const double *d_y_grad, const float *d_ladj_grad,
                               const double *d_y, float *d_backprops, void *stream);
+/* log q(x) of the fitted LogitSkewNormalPTT approximation (definition: DESIGN.md K5) and d log q / dx (as InvHSBGrad
+ * defines it).  x [B][n] on the simplex; mu/omega/alpha [param_batch][n-1], param_batch 1 or B; lp [B] Float64;
+ * x_grad [B][n] Float32 or NULL (then only lp).  For each internal node k (numbered as the fit and the prep file
+ * number them), with y_k = u_left / u_k from the tree inverse, sigma = Float64(expf(omega)),
+ * z = log y - log1p(-y), s = (z - mu) / sigma, w = asinh(s) - alpha, z0 = sinh(w):
+ *   log q(x) = sum_k [ -z0^2/2 - log(2 pi)/2 + log cosh w - log1p(s^2)/2 - log sigma - log y - log1p(-y) ] - sum_k log u_k
+ * in Float64.  A row with some y_k exactly 0 or 1 gets lp = -inf (its x_grad is undefined); other rows are unaffected. */
+int polee_approx_log_prob_with_plan(const polee_hsb_plan *plan, int64_t B, int64_t param_batch, const float *x,
+                                    const float *mu, const float *omega, const float *alpha, double *lp, float *x_grad);
+int polee_approx_log_prob_device(const polee_hsb_plan *plan, int64_t B, int64_t param_batch, const float *d_x,
+                                 const float *d_mu, const float *d_omega, const float *d_alpha, double *d_lp,
+                                 float *d_x_grad, void *stream);
 const char *polee_hsb_last_error(void);
 /* make_inverse_ptt_params(node_parent_idxs, node_js)  src/ptt.jl:293-309 (host helper, exact ints) */
 int polee_make_inverse_ptt_params(int64_t num_nodes, const int32_t *node_parent_idxs, const int32_t *node_js,

@@ -18,6 +18,8 @@ from .api import (  # noqa: F401
     OptimizePTTApprox,
     PolyaTreeTransform,
     RNASeqSample,
+    approx_log_prob,
+    approx_log_prob_torch,
     approximate_likelihood,
     exact_factorization,
     hclust,

@@ -445,17 +445,31 @@ class ApproxLikelihoodSampler:
     def __init__(self, device=0, draws_per_launch=16):
         self.handle = Handle(device=device, num_mc_samples=draws_per_launch)
         self.calls = 0
+        self.plan = None
 
     def set_transform(self, t, mu, sigma, alpha):
         """t: PolyaTreeTransform or (node_parent_idxs, node_js); sigma = exp(omega) as in src/main.jl:833."""
         pi, js = (t.node_parent_idxs, t.node_js) if isinstance(t, PolyaTreeTransform) else t
         self.handle.set_tree(pi, js)
-        self.handle.set_params(mu, np.log(_c(sigma, np.float32)), alpha)
+        omega = np.log(_c(sigma, np.float32))
+        self.handle.set_params(mu, omega, alpha)
+        self.tree = (_c(pi, np.int32), _c(js, np.int32))
+        self.params = (_c(mu, np.float32), omega, _c(alpha, np.float32))
+        if self.plan is not None:
+            self.plan.close()
+            self.plan = None
 
     def rand(self, num_samples=1, seed=None):
         """rand!(als, xs) for num_samples draws at once -> xs[num_samples][n]"""
         self.calls += 1
         return self.handle.sample(num_samples, self.calls if seed is None else seed)
+
+    def log_prob(self, xs, want_grad=False):
+        """log q(xs) of the approximation set_transform holds, in the x space rand() returns (DESIGN.md K5):
+        xs [num_samples][n] -> lp [num_samples], or (lp, x_grad) with want_grad."""
+        if self.plan is None:
+            self.plan = HsbPlan(self.handle.n, *make_inverse_ptt_params(*self.tree), device=self.handle.opts.device)
+        return self.plan.approx_log_prob(xs, *self.params, want_grad=want_grad)
 
 
 def sequential_tree(n):
@@ -685,3 +699,75 @@ class HsbPlan:
     def inv_hsb_grad_device(self, B, d_y_grad, d_ladj_grad, d_y, d_backprops, stream=0):
         _hsb_check(self.lib.polee_inv_hsb_grad_device(self.p, C.c_int64(B), C.c_void_p(d_y_grad), C.c_void_p(d_ladj_grad),
                                                       C.c_void_p(d_y), C.c_void_p(d_backprops), C.c_void_p(stream)))
+
+    def approx_log_prob(self, x, mu, omega, alpha, want_grad=True):
+        """log q(x) of the LogitSkewNormalPTT approximation on this plan's tree(s) (polee_approx_log_prob_with_plan;
+        definition: DESIGN.md K5).  x [B][n]; mu / omega / alpha [param_batch][n-1] (or [n-1]), param_batch 1 or B.
+        Returns lp [B] Float64, or (lp, x_grad [B][n] Float32) with want_grad."""
+        x = np.atleast_2d(_c(x, np.float32))
+        B, n = x.shape
+        mu, omega, alpha = (_c(a, np.float32).reshape(a.size // (n - 1) if n > 1 else 1, n - 1)
+                            for a in (np.asarray(mu), np.asarray(omega), np.asarray(alpha)))
+        if not mu.shape[0] == omega.shape[0] == alpha.shape[0]:
+            raise ValueError("mu, omega and alpha must have the same number of rows")
+        lp = np.zeros(B, np.float64)
+        x_grad = np.zeros((B, n), np.float32) if want_grad else None
+        _hsb_check(self.lib.polee_approx_log_prob_with_plan(self.p, C.c_int64(B), C.c_int64(mu.shape[0]), _p(x), _p(mu),
+                                                            _p(omega), _p(alpha), _p(lp), _p(x_grad)))
+        return (lp, x_grad) if want_grad else lp
+
+    def approx_log_prob_device(self, B, param_batch, d_x, d_mu, d_omega, d_alpha, d_lp, d_x_grad=0, stream=0):
+        """polee_approx_log_prob_device: device pointers; d_x_grad = 0 computes lp only."""
+        _hsb_check(self.lib.polee_approx_log_prob_device(self.p, C.c_int64(B), C.c_int64(param_batch), C.c_void_p(d_x),
+                                                         C.c_void_p(d_mu), C.c_void_p(d_omega), C.c_void_p(d_alpha),
+                                                         C.c_void_p(d_lp), C.c_void_p(d_x_grad or None),
+                                                         C.c_void_p(stream)))
+
+
+def approx_log_prob(x, mu, omega, alpha, left_index, right_index, leaf_index, want_grad=True, device=0):
+    """log q(x) of the fitted LogitSkewNormalPTT approximation (mu, omega = log sigma, alpha: one row, or one per row of
+    x) on the tree(s) given as make_inverse_ptt_params arrays -> lp [B], or (lp, x_grad) with want_grad.  The density
+    the reference evaluates in RNASeqApproxLikelihoodDist._log_prob (src/polee_approx_likelihood.py:367-450), in the
+    fit's own x space (no effective-length rescaling); definition: DESIGN.md K5."""
+    x = np.atleast_2d(_c(x, np.float32))
+    plan = HsbPlan(x.shape[1], left_index, right_index, leaf_index, device)
+    try:
+        return plan.approx_log_prob(x, mu, omega, alpha, want_grad)
+    finally:
+        plan.close()
+
+
+_approx_log_prob_fn = None
+
+
+def approx_log_prob_torch(plan, x, mu, omega, alpha):
+    """Differentiable log q(x) for a torch model: lp [B] (float64) of x [B][n] (float32, on the plan's device), computed
+    by polee_approx_log_prob_device on torch's current stream.  Gradients flow into x only (grad_lp[:, None] * x_grad);
+    mu / omega / alpha ([param_batch][n-1], param_batch 1 or B) are constants here."""
+    global _approx_log_prob_fn
+    if _approx_log_prob_fn is None:
+        import torch
+
+        class ApproxLogProb(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, plan, x, mu, omega, alpha):
+                x = x.detach().to(torch.float32).contiguous()
+                n = x.shape[1]
+                mu, omega, alpha = (a.detach().to(device=x.device, dtype=torch.float32).reshape(-1, n - 1).contiguous()
+                                    for a in (mu, omega, alpha))
+                B = x.shape[0]
+                lp = torch.empty(B, dtype=torch.float64, device=x.device)
+                x_grad = torch.empty_like(x) if ctx.needs_input_grad[1] else None
+                plan.approx_log_prob_device(B, mu.shape[0], x.data_ptr(), mu.data_ptr(), omega.data_ptr(),
+                                            alpha.data_ptr(), lp.data_ptr(), 0 if x_grad is None else x_grad.data_ptr(),
+                                            torch.cuda.current_stream(x.device).cuda_stream)
+                ctx.save_for_backward(x_grad)
+                return lp
+
+            @staticmethod
+            def backward(ctx, grad_lp):
+                (x_grad,) = ctx.saved_tensors
+                return None, (grad_lp[:, None] * x_grad).to(x_grad.dtype), None, None, None
+
+        _approx_log_prob_fn = ApproxLogProb
+    return _approx_log_prob_fn.apply(plan, x, mu, omega, alpha)

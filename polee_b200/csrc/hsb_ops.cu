@@ -25,11 +25,11 @@ struct polee_hsb_plan {
     int nbins[2] = {0, 0};
     int32_t *desc_order = nullptr;  // [ntrees][n-1] internal node ids in descending node order (ladj emulation)
     std::string err;
-    // scratch of the device-resident entry points (u, v / log u per row), grown on demand and kept with the plan so a
-    // training step allocates nothing; calls on one plan are serialised by `mu`
+    // scratch of the device-resident entry points (u, v / log u per row; y, y_grad and row partials of the density),
+    // grown on demand and kept with the plan so a training step allocates nothing; calls on one plan are serialised by `mu`
     mutable std::mutex mu;
-    mutable double *scr[2] = {nullptr, nullptr};
-    mutable size_t scr_count[2] = {0, 0};
+    mutable double *scr[3] = {nullptr, nullptr, nullptr};
+    mutable size_t scr_count[3] = {0, 0, 0};
 };
 
 namespace {
@@ -227,6 +227,70 @@ __global__ void __launch_bounds__(HSB_THREADS)
     }
 }
 
+// K5: log q(x) of the LogitSkewNormalPTT approximation (definition: DESIGN.md K5) from the y and log u that k4_inv_hsb
+// wrote.  One thread per (internal node k, row); a row's terms are summed in Float64 in a fixed order (warp shuffles,
+// then the block's warps, then k5_row_sum over the blocks), so results are run-to-run identical without atomics.
+constexpr int K5_THREADS = 256;
+
+// the block's sum, valid in thread 0; fixed association
+__device__ __forceinline__ double k5_block_sum(double v) {
+    __shared__ double warp_sum[K5_THREADS / 32];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = v;
+    __syncthreads();
+    v = threadIdx.x < K5_THREADS / 32 ? warp_sum[threadIdx.x] : 0.0;
+    if (threadIdx.x < 32) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    }
+    return v;
+}
+
+// node k of row `row`: term = the LSN log density of y_k - log u_k (u_k = the node's subtree sum), y_grad = d term / d y_k
+// (the log u part of the gradient is InvHSBGrad's ladj path).  partial[row][blockIdx.x] = the block's sum of terms.
+__global__ void __launch_bounds__(K5_THREADS)
+    k5_lsn_log_density(int64_t nm1, int per_row_params, const double *__restrict__ yv, const double *__restrict__ logu,
+                       const float *__restrict__ mu, const float *__restrict__ omega, const float *__restrict__ alpha,
+                       double *__restrict__ y_grad, double *__restrict__ partial) {
+    const int64_t row = blockIdx.y, k = (int64_t)blockIdx.x * K5_THREADS + threadIdx.x;
+    double term = 0.0;
+    if (k < nm1) {
+        const size_t i = (size_t)row * nm1 + k, ip = (per_row_params ? (size_t)row * nm1 : 0) + k;
+        const double y = yv[i];
+        // the fit's Float32 sigma = expf(omega) (likelihood-approximation.jl:505-507), correctly rounded: CUDA's expf may be
+        // 2 ulp off, which moves lp by ~1e-9 relative; glibc's expf agrees with this value in all but ~0.1 % of cases
+        const double sigma = (double)(float)exp((double)omega[ip]);
+        const double ly = log(y), l1my = log1p(-y);
+        const double s = (ly - l1my - (double)mu[ip]) / sigma;
+        const double w = asinh(s) - (double)alpha[ip];
+        const double z0 = sinh(w), r = hypot(1.0, s), aw = fabs(w);
+        if (y > 0.0 && y < 1.0) {
+            const double log_cosh_w = aw + log1p(exp(-2.0 * aw)) - 0.69314718055994530942;
+            term = -0.5 * z0 * z0 - 0.91893853320467274178 + log_cosh_w - 0.5 * log1p(s * s) - log(sigma) - ly - l1my - logu[i];
+        } else {
+            term = -INFINITY;  // x is on the boundary of the support (a zero leaf under a non-zero subtree)
+        }
+        const double g_s = (tanh(w) - z0 * cosh(w)) / r - s / (r * r);
+        y_grad[i] = g_s / (sigma * y * (1.0 - y)) + 1.0 / (1.0 - y) - 1.0 / y;
+    }
+    term = k5_block_sum(term);
+    if (threadIdx.x == 0) partial[(size_t)row * gridDim.x + blockIdx.x] = term;
+}
+
+// lp[row] = the sum of the row's block partials; also the ladj_grad = 1 that k4_inv_hsb_grad reads for the gradient
+__global__ void __launch_bounds__(K5_THREADS)
+    k5_row_sum(int nblk, const double *__restrict__ partial, double *__restrict__ lp, float *__restrict__ ladj_grad) {
+    const int64_t row = blockIdx.x;
+    double v = 0.0;
+    for (int b = threadIdx.x; b < nblk; b += K5_THREADS) v += partial[(size_t)row * nblk + b];
+    v = k5_block_sum(v);
+    if (threadIdx.x == 0) {
+        lp[row] = v;
+        ladj_grad[row] = 1.0f;
+    }
+}
+
 template <typename T>
 cudaError_t up_vec(const std::vector<T> &v, T **d) {
     *d = nullptr;
@@ -270,7 +334,7 @@ int polee_hsb_plan_destroy(polee_hsb_plan *p) {
     cudaSetDevice(p->device);
     polee::dfree(p->nodes);
     polee::dfree(p->desc_order);
-    polee::dfree(p->scr[0]); polee::dfree(p->scr[1]);
+    polee::dfree(p->scr[0]); polee::dfree(p->scr[1]); polee::dfree(p->scr[2]);
     for (int s = 0; s < 2; ++s) {
         polee::dfree(p->bin_lvl_ptr[s]); polee::dfree(p->lvl_off[s]); polee::dfree(p->sch_node[s]); polee::dfree(p->bin_tree[s]);
     }
@@ -415,6 +479,46 @@ int polee_inv_hsb_grad_device(const polee_hsb_plan *p, int64_t B, const double *
     return POLEE_OK;
 }
 
+// k4_inv_hsb -> k5_lsn_log_density -> k5_row_sum [-> k4_inv_hsb_grad with ladj_grad = 1].  The Float32 ladj replay
+// (k4_ladj_chain) is not needed: the density sums -log u_j in Float64 with the other terms.
+int polee_approx_log_prob_device(const polee_hsb_plan *p, int64_t B, int64_t param_batch, const float *d_x,
+                                 const float *d_mu, const float *d_omega, const float *d_alpha, double *d_lp,
+                                 float *d_x_grad, void *stream) {
+    int rc = check_plan(p, B);
+    if (rc) return rc;
+    if (param_batch != 1 && param_batch != B) return hsb_fail(POLEE_EINVAL, "approx_log_prob: param_batch must be 1 or B");
+    if (!d_x || !d_mu || !d_omega || !d_alpha || !d_lp) return hsb_fail(POLEE_EINVAL, "approx_log_prob: null pointer");
+    std::lock_guard<std::mutex> lk(p->mu);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int shared = p->ntrees == 1;
+    const int64_t nm1 = p->n - 1;
+    const int nblk = (int)((nm1 + K5_THREADS - 1) / K5_THREADS);
+    double *d_us, *d_logu, *d_k5;
+    if ((rc = plan_scratch(p, 0, (size_t)B * p->N, &d_us))) return rc;
+    if ((rc = plan_scratch(p, 1, (size_t)B * p->N, &d_logu))) return rc;  // log u, then v of the gradient
+    if ((rc = plan_scratch(p, 2, (size_t)B * (2 * nm1 + nblk + 1), &d_k5))) return rc;
+    double *d_y = d_k5, *d_y_grad = d_y + (size_t)B * nm1, *d_part = d_y_grad + (size_t)B * nm1;
+    float *d_ladj_grad = (float *)(d_part + (size_t)B * nblk);
+    for (int s = 1; s >= 0; --s)
+        if (p->nbins[s] > 0) {
+            dim3 grid(p->nbins[s], shared ? (unsigned)B : 1u);
+            k4_inv_hsb<<<grid, HSB_THREADS, 0, st>>>(sched_of(p, s), shared, p->nodes, p->n, p->N, d_x, d_us, d_y, d_logu);
+        }
+    if (nblk > 0)
+        k5_lsn_log_density<<<dim3((unsigned)nblk, (unsigned)B), K5_THREADS, 0, st>>>(nm1, param_batch != 1, d_y, d_logu, d_mu,
+                                                                                     d_omega, d_alpha, d_y_grad, d_part);
+    k5_row_sum<<<(unsigned)B, K5_THREADS, 0, st>>>(nblk, d_part, d_lp, d_ladj_grad);
+    if (d_x_grad)
+        for (int s = 0; s < 2; ++s)
+            if (p->nbins[s] > 0) {
+                dim3 grid(p->nbins[s], shared ? (unsigned)B : 1u);
+                k4_inv_hsb_grad<<<grid, HSB_THREADS, 0, st>>>(sched_of(p, s), shared, p->nodes, p->n, p->N, d_y_grad, d_ladj_grad,
+                                                              d_y, d_us, d_logu, d_x_grad);
+            }
+    HCK(cudaGetLastError());
+    return POLEE_OK;
+}
+
 // ---- host-tensor forms (the DEVICE_CPU registration of the shim): upload, the device form on the legacy stream, download
 int polee_hsb_with_plan(const polee_hsb_plan *p, int64_t B, const float *y_logit, float *x) {
     int rc = check_plan(p, B);
@@ -458,6 +562,28 @@ int polee_inv_hsb_grad_with_plan(const polee_hsb_plan *p, int64_t B, const doubl
     HCK(db.alloc(&d_bp, (size_t)B * p->n));
     if ((rc = polee_inv_hsb_grad_device(p, B, d_yg, d_lg, d_y, d_bp, nullptr))) return rc;
     HCK(cudaMemcpy(backprops, d_bp, sizeof(float) * (size_t)B * p->n, cudaMemcpyDeviceToHost));
+    return POLEE_OK;
+}
+
+int polee_approx_log_prob_with_plan(const polee_hsb_plan *p, int64_t B, int64_t param_batch, const float *x,
+                                    const float *mu, const float *omega, const float *alpha, double *lp, float *x_grad) {
+    int rc = check_plan(p, B);
+    if (rc) return rc;
+    if (param_batch != 1 && param_batch != B) return hsb_fail(POLEE_EINVAL, "approx_log_prob: param_batch must be 1 or B");
+    if (!x || !mu || !omega || !alpha || !lp) return hsb_fail(POLEE_EINVAL, "approx_log_prob: null pointer");
+    const size_t np = (size_t)param_batch * (p->n - 1);
+    DevBuf db;
+    float *d_x, *d_mu, *d_om, *d_al, *d_xg = nullptr;
+    double *d_lp;
+    HCK(db.upload(&d_x, x, (size_t)B * p->n));
+    HCK(db.upload(&d_mu, mu, np));
+    HCK(db.upload(&d_om, omega, np));
+    HCK(db.upload(&d_al, alpha, np));
+    HCK(db.alloc(&d_lp, (size_t)B));
+    if (x_grad) HCK(db.alloc(&d_xg, (size_t)B * p->n));
+    if ((rc = polee_approx_log_prob_device(p, B, param_batch, d_x, d_mu, d_om, d_al, d_lp, d_xg, nullptr))) return rc;
+    HCK(cudaMemcpy(lp, d_lp, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost));
+    if (x_grad) HCK(cudaMemcpy(x_grad, d_xg, sizeof(float) * (size_t)B * p->n, cudaMemcpyDeviceToHost));
     return POLEE_OK;
 }
 
