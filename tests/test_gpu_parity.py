@@ -26,7 +26,7 @@ def _synth_sample(pb, s):
 
 
 @pytest.mark.parametrize("exact", [False, True])
-@pytest.mark.parametrize("K", [1, 2, 6, 8, 16])
+@pytest.mark.parametrize("K", [1, 2, 3, 5, 6, 7, 8, 12, 16])
 def test_loglik_and_gradient_fixture(pb, fx, oracle, K, exact):
     """K1 + K2 vs sparse.jl restated: lp and x_grad <= 1e-5 relative, identity sum_j x_j g_j = m.
     exact=True: reference-order all-Float64 sums (p bit-identical); exact=False: the default fast kernels."""
