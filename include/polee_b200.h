@@ -156,7 +156,10 @@ int polee_step_stats(polee_handle *h, double *bytes_k1, double *bytes_k2, double
 /* which device layouts hold the matrix (a1-a2: replaces Xt = SparseMatrixCSC(transpose(X)),
  * likelihood-approximation.jl:407): info[0..5] = rows, entries, classes, tasks, blob bytes, partials of the
  * equivalence-class layout; info[6..7] = rows, entries of the general layouts; info[8] = their kind (0 none,
- * 1 split, 2 fused); info[9] = padded row slots of the class layout.  count <= 10 values are written. */
+ * 1 split, 2 fused); info[9] = padded row slots of the class layout; info[10] = the kernels the tree takes at the
+ * draw count the work buffers were last sized for (0 chain scans, 1 DFS runs, 2 path products, 3 shared-memory
+ * levels, 4 global-memory levels; -1 without a tree or before the first call that sizes them).  count <= 11 values
+ * are written. */
 int polee_layout_info(polee_handle *h, int64_t *info, int32_t count);
 /* time (ms, CUDA events on the handle's stream) of `reps` launches of one named kernel group:
  * which = 1 (the likelihood pass; K1 alone on the pure split layout), 2 (K2 of the pure split layout),

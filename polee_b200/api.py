@@ -214,12 +214,15 @@ class Handle:
         return {"bytes_k1": b[0].value, "bytes_k2": b[1].value, "bytes_k3": b[2].value, "launches": nl.value}
 
     def layout_info(self):
-        v = (C.c_int64 * 10)()
-        self.check(self.lib.polee_layout_info(self.h, v, C.c_int32(10)))
+        v = (C.c_int64 * 11)()
+        self.check(self.lib.polee_layout_info(self.h, v, C.c_int32(11)))
         keys = ("ec_rows", "ec_nnz", "ec_classes", "ec_tasks", "ec_blob_bytes", "ec_partials", "general_rows",
-                "general_nnz", "general_kind", "ec_row_slots")
+                "general_nnz", "general_kind", "ec_row_slots", "tree_route")
         out = dict(zip(keys, (int(x) for x in v)))
         out["general_kind"] = ("none", "split", "fused")[out["general_kind"]]
+        # the kernels the tree takes at the draw count of the last call (None: no tree, or no call yet)
+        r = out["tree_route"]
+        out["tree_route"] = None if r < 0 else ("chain", "dfs", "path", "levels_smem", "levels_global")[r]
         return out
 
     def time_kernel(self, which, reps):

@@ -1042,13 +1042,16 @@ extern "C" int polee_step_stats(polee_handle *h, double *b1, double *b2, double 
 
 // Which layouts hold the matrix: info[0..9] = {rows, entries, classes, tasks, blob bytes, partials} of the
 // equivalence-class layout, {rows, entries} of the general layouts, general layout kind (0 none, 1 split, 2 fused),
-// padded row slots of the class layout.
+// padded row slots of the class layout; info[10] = the tree route (TreeRoute) at the work buffers' KP, -1 without a tree
+// or work buffers.
 extern "C" int polee_layout_info(polee_handle *h, int64_t *info, int32_t count) {
     CHECK_H(h);
     if (!info || count < 1) return h->fail(POLEE_EINVAL, "layout_info: bad arguments");
-    const int64_t v[10] = {h->ec_rows, h->ec_nnz, h->ec_classes, (int64_t)h->ec_tasks, (int64_t)h->ec_blob_bytes, h->ec_parts,
-                           h->gm, h->gnnz, (int64_t)((h->gm > 0 || h->ec_tasks == 0) ? (h->fused ? 2 : 1) : 0), h->ec_slots};
-    for (int i = 0; i < count && i < 10; ++i) info[i] = v[i];
+    const int64_t route = h->have_tree && h->work_KP > 0 ? (int64_t)tree_route(h->td, h->work_KP) : -1;
+    const int64_t v[11] = {h->ec_rows, h->ec_nnz, h->ec_classes, (int64_t)h->ec_tasks, (int64_t)h->ec_blob_bytes, h->ec_parts,
+                           h->gm, h->gnnz, (int64_t)((h->gm > 0 || h->ec_tasks == 0) ? (h->fused ? 2 : 1) : 0), h->ec_slots,
+                           route};
+    for (int i = 0; i < count && i < 11; ++i) info[i] = v[i];
     return POLEE_OK;
 }
 

@@ -269,10 +269,17 @@ struct TreeDev {
     uint32_t *drun_anc_ptr = nullptr, *drun_anc = nullptr;
     int32_t *dcta_k0 = nullptr;
     int dfs_ctas = 0, dfs_max_nk = 0, max_depth = 0;
+    int64_t chain_min_nodes = 0;  // caterpillar trees of this many nodes or more take the scan kernels of tree_chain.cu
+                                  // (upload_tree: POLEE_CHAIN_MIN_NODES, default 4096)
     void release();
 };
 
 std::string upload_tree(const TreeHost &th, TreeDev &td);
+
+// The kernels that serve a tree's forward, backward and inverse passes (the rules: tree_route, tree_kernels.cu).
+// polee_layout_info reports the route as its integer value, which include/polee_b200.h documents: keep the order.
+enum class TreeRoute { Chain, DfsRun, PathProduct, SmemLevels, GlobalLevels };
+TreeRoute tree_route(const TreeDev &td, int KP);
 
 }  // namespace polee
 
@@ -405,7 +412,6 @@ struct polee_handle {
     float *grad_out = nullptr;            // [3][n-1] averaged grads (polee_lsn_draws)
     int work_KP = 0;                      // KP the work buffers were sized for
     int n_tree_ctas = 0;
-    int tree_grid = 0;  // persistent bottom-tree grid
 
     // ---- graph
     cudaGraph_t graph = nullptr;
@@ -432,6 +438,17 @@ struct polee_handle {
 namespace polee {
 
 int pad_k(int K);
+
+// CALL with the padded draw count KP as the compile-time constant KPC; other KP fail the enclosing launch function
+#define DISPATCH_KP(KP, CALL)                                                   \
+    switch (KP) {                                                               \
+        case 1: { constexpr int KPC = 1; CALL; } break;                         \
+        case 2: { constexpr int KPC = 2; CALL; } break;                         \
+        case 4: { constexpr int KPC = 4; CALL; } break;                         \
+        case 8: { constexpr int KPC = 8; CALL; } break;                         \
+        case 16: { constexpr int KPC = 16; CALL; } break;                       \
+        default: return h->fail(POLEE_EINVAL, "unsupported number of MC draws (1..16)"); \
+    }
 
 // Dynamic shared memory opt-in.  The attribute is per FUNCTION and process-wide, and several handles (host threads)
 // with different tile / tree sizes launch the same kernels: always raise it to the device limit, never to "what this

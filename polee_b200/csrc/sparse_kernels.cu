@@ -590,16 +590,6 @@ int launch_k2_t(polee_handle *h, const float *w, double *g) {
 
 }  // namespace
 
-#define DISPATCH_KP(KP, CALL)                                                   \
-    switch (KP) {                                                               \
-        case 1: { constexpr int KPC = 1; CALL; } break;                         \
-        case 2: { constexpr int KPC = 2; CALL; } break;                         \
-        case 4: { constexpr int KPC = 4; CALL; } break;                         \
-        case 8: { constexpr int KPC = 8; CALL; } break;                         \
-        case 16: { constexpr int KPC = 16; CALL; } break;                       \
-        default: return h->fail(POLEE_EINVAL, "unsupported number of MC draws (1..16)"); \
-    }
-
 int launch_k1(polee_handle *h, const float *x, float *w, bool want_lp, double *lp_partial, int KP) {
     int rc = POLEE_OK;
     DISPATCH_KP(KP, rc = launch_k1_t<KPC>(h, x, w, want_lp, lp_partial));

@@ -149,15 +149,6 @@ __global__ void __launch_bounds__(CH_THREADS)
 }  // namespace
 
 #define CK(expr) POLEE_CUDA_CHECK(h, expr)
-#define DISPATCH_KP(KP, CALL)                                                   \
-    switch (KP) {                                                               \
-        case 1: { constexpr int KPC = 1; CALL; } break;                         \
-        case 2: { constexpr int KPC = 2; CALL; } break;                         \
-        case 4: { constexpr int KPC = 4; CALL; } break;                         \
-        case 8: { constexpr int KPC = 8; CALL; } break;                         \
-        case 16: { constexpr int KPC = 16; CALL; } break;                       \
-        default: return h->fail(POLEE_EINVAL, "unsupported number of MC draws (1..16)"); \
-    }
 
 int launch_chain_fwd(polee_handle *h, int KP, int clamp_x, const float *eff, double *Sp, int want_ladj, double *ladj_tree) {
     DISPATCH_KP(KP, (k3c_chain_fwd<KPC><<<KP, CH_THREADS, 0, h->stream>>>(h->td.n, h->td.chain_leaf, h->ys, h->us, h->x, clamp_x, eff, Sp, want_ladj, ladj_tree)));

@@ -16,6 +16,7 @@
 #include <climits>
 #include <cstdio>
 #include <cstdint>
+#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -463,10 +464,12 @@ std::string upload_tree(const TreeHost &th, TreeDev &td) {
         if (e == cudaSuccess) e = upv(th.dcta_k0.data(), 4 * th.dcta_k0.size(), (void **)&td.dcta_k0);
         td.dfs_ctas = (int)th.dcta_k0.size() - 1;
         td.dfs_max_nk = th.dfs_max_nk;
-        td.n_groups = std::max(td.n_groups, td.dfs_ctas);  // sizes the per-CTA partial sums (S, ladj)
     }
     td.n_slots = th.n_slots;
     td.caterpillar = th.caterpillar;
+    // read once per tree: no launch, graph-captured ones included, looks at the environment
+    const char *chain_env = getenv("POLEE_CHAIN_MIN_NODES");
+    td.chain_min_nodes = chain_env ? atoll(chain_env) : 4096;
     if (e == cudaSuccess && th.caterpillar) e = up(th.chain_leaf, &td.chain_leaf);
     if (e != cudaSuccess) return std::string("upload_tree: ") + cudaGetErrorString(e);
     // the pageable-memory copies above run on the legacy stream, which does not order against the handle's

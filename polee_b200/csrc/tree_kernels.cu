@@ -18,7 +18,6 @@
 #include <math_constants.h>
 
 #include <climits>
-#include <cstdlib>
 
 #include "common.cuh"
 #include "device_utils.cuh"
@@ -271,7 +270,8 @@ __global__ void k3_init_params(int64_t nm1, int KP, const double *__restrict__ y
 // the level loops entirely out of shared memory (one __syncthreads per level, no global load on the critical path)
 // and writes its results back at the end.  grid = (bins, KP / KPC): KPC draws per CTA (8 for the bottom forests,
 // 1 for the top part so that a few thousand nodes fit).  Bottom subtree roots exchange u (top -> bottom) and G
-// (bottom -> top) through [slot][KP] arrays.  The backward kernel recomputes u from ys instead of reading it back.
+// (bottom -> top) through [slot][KP] arrays.  The forward kernel also leaves u of every internal node by k in us_k,
+// where the backward kernel reads it, as it does after the DFS-run and path-product forward kernels.
 template <int KPC, int THREADS>
 __device__ __forceinline__ void block_reduce_kc(double v, double *red, double *out /* [KPC] */) {
     red[threadIdx.x] = v;
@@ -288,7 +288,7 @@ template <int KP, int KPC, int THREADS, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB)
     k3s_tree_fwd(const int32_t *__restrict__ bin_off, const int32_t *__restrict__ bin_lvl_ptr,
                  const int32_t *__restrict__ lvl_off, const SNode *__restrict__ recs, const double *__restrict__ ys,
-                 double *__restrict__ root_us, float *__restrict__ x, int clamp_x,
+                 double *__restrict__ root_us, double *__restrict__ us_k, float *__restrict__ x, int clamp_x,
                  const float *__restrict__ efflen, double *__restrict__ S_partial, int part_base, int want_ladj,
                  double *__restrict__ ladj_partial) {
     extern __shared__ __align__(16) unsigned char smraw[];
@@ -342,6 +342,7 @@ __global__ void __launch_bounds__(THREADS, MINB)
                 const double y = ys_s[p * KPC + kk];
                 us_s[r.left * KPC + kk] = __dmul_rn(y, ui);
                 us_s[r.right * KPC + kk] = __dmul_rn(__dsub_rn(1.0, y), ui);
+                us_k[(size_t)r.k_or_leaf * KP + k] = ui;
                 if (want_ladj) lacc += log(ui);
             } else if (r.k_or_leaf == INT32_MIN) {
                 root_us[(size_t)r.slot * KP + k] = ui;  // a bottom subtree root: hand u over
@@ -371,11 +372,10 @@ template <int KP, int KPC, int THREADS, int MINB, bool WITH_LADJ>
 __global__ void __launch_bounds__(THREADS, MINB)
     k3s_tree_bwd(const int32_t *__restrict__ bin_off, const int32_t *__restrict__ bin_lvl_ptr,
                  const int32_t *__restrict__ lvl_off, const SNode *__restrict__ recs, const double *__restrict__ ys,
-                 const double *__restrict__ root_us, float2 *__restrict__ root_G, const double *__restrict__ g,
+                 const double *__restrict__ us_k, float2 *__restrict__ root_G, const double *__restrict__ g,
                  const float *__restrict__ efflen_adj, const double *__restrict__ S, double *__restrict__ ygrad,
-                 double *__restrict__ xgrad_out, const double *__restrict__ us_k) {
-    // us_k != nullptr: u of every internal node by k, as the path-product forward kernel left it (then nothing is
-    // recomputed here and root_us is not read)
+                 double *__restrict__ xgrad_out) {
+    // us_k: u of every internal node by k, as the forward kernel left it
     extern __shared__ __align__(16) unsigned char smraw[];
     const int q0 = bin_off[blockIdx.x], nb = bin_off[blockIdx.x + 1] - q0;
     SNode *rec_s = reinterpret_cast<SNode *>(smraw);
@@ -407,7 +407,7 @@ __global__ void __launch_bounds__(THREADS, MINB)
             v0[u] = 0.0; uv[u] = 1.0; adj[u] = 0.0f; gx[u] = make_float2(0.f, 0.f);
             if (r[u].k_or_leaf >= 0) {
                 v0[u] = ys[(size_t)r[u].k_or_leaf * KP + k];
-                if (us_k) uv[u] = us_k[(size_t)r[u].k_or_leaf * KP + k];
+                uv[u] = us_k[(size_t)r[u].k_or_leaf * KP + k];
             } else if (r[u].k_or_leaf == INT32_MIN) {
                 gx[u] = root_G[(size_t)r[u].slot * KP + k];
             } else if (r[u].k_or_leaf != INT32_MIN + 1) {
@@ -415,7 +415,6 @@ __global__ void __launch_bounds__(THREADS, MINB)
                 v0[u] = g[(size_t)leaf * KP + k];
                 if (efflen_adj) adj[u] = __int_as_float(r[u].right);
             }
-            if (!us_k && r[u].slot >= 0 && r[u].k_or_leaf != INT32_MIN) uv[u] = root_us[(size_t)r[u].slot * KP + k];
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
@@ -423,6 +422,7 @@ __global__ void __launch_bounds__(THREADS, MINB)
             if (p >= nb) continue;
             if (r[u].k_or_leaf >= 0) {
                 ys_s[p * KPC + kk] = v0[u];
+                us_s[p * KPC + kk] = uv[u];
             } else if (r[u].k_or_leaf == INT32_MIN) {
                 G_s[p * KPC + kk] = gx[u];
             } else {
@@ -432,24 +432,10 @@ __global__ void __launch_bounds__(THREADS, MINB)
                 if (xgrad_out) xgrad_out[(size_t)leaf * KP + k] = gv;
                 G_s[p * KPC + kk] = make_float2((float)gv, 0.0f);
             }
-            if (us_k ? r[u].k_or_leaf >= 0 : (r[u].slot >= -1 && r[u].k_or_leaf != INT32_MIN)) us_s[p * KPC + kk] = uv[u];
         }
     }
     __syncthreads();
 
-    // forward recompute of u (same operations as k3s_tree_fwd -> same bits)
-    for (int l = 0; l < (us_k ? 0 : nlev); ++l) {
-        const int lo = lvl_s[l], hi = lvl_s[l + 1];
-        for (int p = lo + slot_t; p < hi; p += NPP) {
-            const SNode r = rec_s[p];
-            if (r.k_or_leaf >= 0) {
-                const double ui = us_s[p * KPC + kk], y = ys_s[p * KPC + kk];
-                us_s[r.left * KPC + kk] = __dmul_rn(y, ui);
-                us_s[r.right * KPC + kk] = __dmul_rn(__dsub_rn(1.0, y), ui);
-            }
-        }
-        __syncthreads();
-    }
     // backward sweep
     for (int l = nlev - 1; l >= 0; --l) {
         const int lo = lvl_s[l], hi = lvl_s[l + 1];
@@ -992,9 +978,19 @@ int ensure_work_buffers(polee_handle *h, int KP) {
     if (h->work_KP == KP) return POLEE_OK;
     release_work_buffers(h);
     const int64_t n = h->n, nm1 = std::max<int64_t>(n - 1, 1), N = 2 * n - 1;
-    h->tree_grid = std::max(1, std::min(h->td.s_bottom.nbins * std::max(1, KP / std::min(KP, 4)), 2 * h->num_sms));
-    h->n_tree_ctas = std::max(1 + std::max(h->td.bottom.nbins, h->tree_grid), h->td.n_groups);
-    h->n_tree_ctas = std::max(h->n_tree_ctas, (int)((n + LEAF_S_PER_WARP - 1) / LEAF_S_PER_WARP));  // k3_leaf_S: a row per warp
+    // rows of the per-CTA partial sums (S_partial and the tree part of ladj_partial): those the route's forward kernels
+    // write, or one per warp of k3_leaf_S.  k3_mid, k3_elbo and polee_ptt_transform add them all in a fixed order; the
+    // rows a route does not write stay 0
+    const TreeDev &td = h->td;
+    int rows = 1;  // k3c_chain_fwd: one
+    switch (tree_route(td, KP)) {
+        case TreeRoute::Chain: break;
+        case TreeRoute::DfsRun: rows = td.dfs_ctas; break;
+        case TreeRoute::PathProduct: rows = td.n_groups; break;
+        case TreeRoute::SmemLevels: rows = 1 + td.s_bottom.nbins; break;  // the top part, then the bottom bins
+        case TreeRoute::GlobalLevels: rows = 1 + td.bottom.nbins; break;
+    }
+    h->n_tree_ctas = std::max(rows, (int)((n + LEAF_S_PER_WARP - 1) / LEAF_S_PER_WARP));
     CK(polee::dmalloc((void **)&h->zs0, sizeof(float) * nm1 * KP));
     CK(polee::dmalloc((void **)&h->zs, sizeof(float) * nm1 * KP));
     CK(polee::dmalloc((void **)&h->ys, sizeof(double) * nm1 * KP));
@@ -1034,16 +1030,6 @@ int ensure_work_buffers(polee_handle *h, int KP) {
     return POLEE_OK;
 }
 
-#define DISPATCH_KP(KP, CALL)                                                   \
-    switch (KP) {                                                               \
-        case 1: { constexpr int KPC = 1; CALL; } break;                         \
-        case 2: { constexpr int KPC = 2; CALL; } break;                         \
-        case 4: { constexpr int KPC = 4; CALL; } break;                         \
-        case 8: { constexpr int KPC = 8; CALL; } break;                         \
-        case 16: { constexpr int KPC = 16; CALL; } break;                       \
-        default: return h->fail(POLEE_EINVAL, "unsupported number of MC draws (1..16)"); \
-    }
-
 int patch_leaf_records(polee_handle *h) {
     if (!h->have_efflen || !h->have_tree) return POLEE_OK;
     for (SSchedDev *sd : {&h->td.s_top, &h->td.s_bottom}) {
@@ -1080,25 +1066,40 @@ constexpr int S_TOP_THREADS = 1024;
 constexpr int bottom_kpc(int KP) { return KP == 8 ? 4 : (KP < 8 ? KP : 8); }
 constexpr int bottom_minb(int KP) { return KP == 8 ? 3 : 2; }
 
-// the path-product forward kernel (k3p_tree_fwd) is used whenever the tree's root paths were built (not for very deep
-// trees) and the shared-memory backward kernels, which read its u, are
-static bool smem_path_ok(const polee_handle *h, int KP);
-static bool chain_path(const polee_handle *h);
-static bool path_fwd_ok(const polee_handle *h) {
-    return h->td.ganc_ptr != nullptr && !chain_path(h) && smem_path_ok(h, h->work_KP);
-}
-// the DFS-run forward kernel (k3d_tree_fwd): trees in DFS pre-order of moderate depth (tree_host.cu builds its inputs
-// only then); like the path-product kernel it leaves u by k for the shared-memory backward kernels
-static size_t dfs_fwd_smem(const polee_handle *h, int KP) {
+// dynamic shared memory of k3d_tree_fwd: the walks' stacks, the CTA's y slice and its node records
+static size_t dfs_fwd_smem(const TreeDev &td, int KP) {
     const size_t threads = (size_t)DFS_RUNS_PER_CTA * KP;
-    return (size_t)(h->td.max_depth + 2) * threads * 8 + (size_t)((std::max(h->td.dfs_max_nk, 1) + 1) & ~1) * KP * 8 +
+    return (size_t)(td.max_depth + 2) * threads * 8 + (size_t)((std::max(td.dfs_max_nk, 1) + 1) & ~1) * KP * 8 +
            (size_t)DFS_RUNS_PER_CTA * (DFS_RUN + 2) * sizeof(DNode);
 }
-static bool dfs_fwd_ok(const polee_handle *h) {
-    return h->td.dnodes != nullptr && !chain_path(h) && smem_path_ok(h, h->work_KP) && h->work_KP <= 16 &&
-           dfs_fwd_smem(h, h->work_KP) <= 200 * 1024;
+
+// The kernels that serve a tree at KP draws: the first route whose condition holds.
+//
+//   route         condition                                       forward        backward       inverse
+//   Chain         caterpillar, N >= chain_min_nodes               k3c_chain_fwd  k3c_chain_bwd  k3_tree_inv_serial
+//   DfsRun        bins fit, DFS-run inputs built (pre-order,      k3d_tree_fwd   k3s_tree_bwd   k3_tree_inv
+//                 depth <= DFS_MAX_DEPTH), KP <= 16,
+//                 dfs_fwd_smem <= 200 KB
+//   PathProduct   bins fit, root-path tables built                k3p_tree_fwd   k3s_tree_bwd   k3_tree_inv
+//   SmemLevels    bins fit                                        k3s_tree_fwd   k3s_tree_bwd   k3_tree_inv
+//   GlobalLevels  everything else                                 k3_tree_fwd    k3_tree_bwd    k3_tree_inv
+//
+// "Bins fit": the largest bottom bin (min(KP, 8) draws) and the top part (one draw) each fit in 200 KB of shared memory
+// with the records, u, y and G the shared-memory kernels hold per node.  The forward kernels of the three routes that
+// share k3s_tree_bwd all leave u of every internal node by k in h->us, where it reads it; the chain and global-level
+// kernels keep u by node there.
+TreeRoute tree_route(const TreeDev &td, int KP) {
+    if (td.caterpillar && td.N >= td.chain_min_nodes) return TreeRoute::Chain;
+    const size_t limit = 200 * 1024;
+    const int KPC = KP < 8 ? KP : 8;
+    const bool bins_fit =
+        (size_t)td.s_bottom.max_bin_nodes * (sizeof(SNode) + 24 * KPC) + 4 * (td.s_bottom.max_bin_levels + 2) <= limit &&
+        (size_t)td.s_top.max_bin_nodes * (sizeof(SNode) + 24) + 4 * (td.s_top.max_bin_levels + 2) <= limit;
+    if (!bins_fit) return TreeRoute::GlobalLevels;
+    if (td.dnodes && KP <= 16 && dfs_fwd_smem(td, KP) <= limit) return TreeRoute::DfsRun;
+    if (td.ganc_ptr) return TreeRoute::PathProduct;
+    return TreeRoute::SmemLevels;
 }
-static bool fwd_leaves_us_by_k(const polee_handle *h) { return dfs_fwd_ok(h) || path_fwd_ok(h); }
 
 template <int KP>
 static int launch_tree_fwd_smem(polee_handle *h, int clamp_x, const float *eff, double *Sp, int want_ladj, double *ladj_tree) {
@@ -1108,8 +1109,8 @@ static int launch_tree_fwd_smem(polee_handle *h, int clamp_x, const float *eff, 
         auto fn = k3s_tree_fwd<KP, 1, S_TOP_THREADS, 1>;
         allow_max_smem(fn);  // per-function, process-wide: see common.cuh
         fn<<<dim3(td.s_top.nbins, KP), S_TOP_THREADS, smem, h->stream>>>(
-            td.s_top.bin_off, td.s_top.bin_lvl_ptr, td.s_top.lvl_off, td.s_top.recs, h->ys, h->root_us, h->x, clamp_x,
-            eff, Sp, 0, want_ladj, ladj_tree);
+            td.s_top.bin_off, td.s_top.bin_lvl_ptr, td.s_top.lvl_off, td.s_top.recs, h->ys, h->root_us, h->us, h->x,
+            clamp_x, eff, Sp, 0, want_ladj, ladj_tree);
     }
     if (td.s_bottom.nbins > 0) {
         constexpr int KPC = bottom_kpc(KP);
@@ -1117,8 +1118,8 @@ static int launch_tree_fwd_smem(polee_handle *h, int clamp_x, const float *eff, 
         auto fn = k3s_tree_fwd<KP, KPC, TREE_THREADS, bottom_minb(KP)>;
         allow_max_smem(fn);
         fn<<<dim3(td.s_bottom.nbins, KP / KPC), TREE_THREADS, smem, h->stream>>>(
-            td.s_bottom.bin_off, td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->root_us, h->x,
-            clamp_x, eff, Sp, 1, want_ladj, ladj_tree);
+            td.s_bottom.bin_off, td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->root_us, h->us,
+            h->x, clamp_x, eff, Sp, 1, want_ladj, ladj_tree);
     }
     return POLEE_OK;
 }
@@ -1126,43 +1127,24 @@ static int launch_tree_fwd_smem(polee_handle *h, int clamp_x, const float *eff, 
 template <int KP, bool WITH_LADJ>
 static int launch_tree_bwd_smem(polee_handle *h, const float *adj, double *xgrad_out) {
     const TreeDev &td = h->td;
-    const double *us_k = fwd_leaves_us_by_k(h) ? h->us : nullptr;
     if (td.s_bottom.nbins > 0) {
         constexpr int KPC = bottom_kpc(KP);
         const size_t smem = (size_t)td.s_bottom.max_bin_nodes * (sizeof(SNode) + 24 * KPC) + 4 * (td.s_bottom.max_bin_levels + 2);
         auto fn = k3s_tree_bwd<KP, KPC, TREE_THREADS, bottom_minb(KP), WITH_LADJ>;
         allow_max_smem(fn);
         fn<<<dim3(td.s_bottom.nbins, KP / KPC), TREE_THREADS, smem, h->stream>>>(
-            td.s_bottom.bin_off, td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->root_us, h->root_G, h->g,
-            adj, h->S, h->ygrad, xgrad_out, us_k);
+            td.s_bottom.bin_off, td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->us, h->root_G, h->g,
+            adj, h->S, h->ygrad, xgrad_out);
     }
     if (td.s_top.nbins > 0) {
         const size_t smem = (size_t)td.s_top.max_bin_nodes * (sizeof(SNode) + 24) + 4 * (td.s_top.max_bin_levels + 2);
         auto fn = k3s_tree_bwd<KP, 1, S_TOP_THREADS, 1, WITH_LADJ>;
         allow_max_smem(fn);
         fn<<<dim3(td.s_top.nbins, KP), S_TOP_THREADS, smem, h->stream>>>(
-            td.s_top.bin_off, td.s_top.bin_lvl_ptr, td.s_top.lvl_off, td.s_top.recs, h->ys, h->root_us, h->root_G, h->g, adj,
-            h->S, h->ygrad, xgrad_out, us_k);
+            td.s_top.bin_off, td.s_top.bin_lvl_ptr, td.s_top.lvl_off, td.s_top.recs, h->ys, h->us, h->root_G, h->g, adj,
+            h->S, h->ygrad, xgrad_out);
     }
     return POLEE_OK;
-}
-
-// the shared-memory kernels need the largest bin (bottom: <= bin_nodes; top: top nodes + subtree roots, one draw
-// per CTA) to fit in one CTA's shared memory; otherwise (very deep trees, e.g. :sequential) the global-memory
-// kernels above are used
-static bool smem_path_ok(const polee_handle *h, int KP) {
-    const TreeDev &td = h->td;
-    const int KPC = KP < 8 ? KP : 8;
-    const size_t limit = 200 * 1024;
-    return (size_t)td.s_bottom.max_bin_nodes * (sizeof(SNode) + 24 * KPC) + 4 * (td.s_bottom.max_bin_levels + 2) <= limit &&
-           (size_t)td.s_top.max_bin_nodes * (sizeof(SNode) + 24) + 4 * (td.s_top.max_bin_levels + 2) <= limit;
-}
-
-// large caterpillar trees take the scan kernels of tree_chain.cu (POLEE_CHAIN_MIN_NODES overrides the threshold)
-static bool chain_path(const polee_handle *h) {
-    const char *e = getenv("POLEE_CHAIN_MIN_NODES");
-    const int64_t min_nodes = e ? atoll(e) : 4096;
-    return h->td.caterpillar && h->td.N >= min_nodes;
 }
 
 int launch_tree_fwd(polee_handle *h, int KP, int clamp_x, int want_S, int want_ladj) {
@@ -1170,40 +1152,44 @@ int launch_tree_fwd(polee_handle *h, int KP, int clamp_x, int want_S, int want_l
     double *ladj_tree = h->ladj_partial + (size_t)2 * elem_ctas(h, KP) * KP;
     const float *eff = want_S ? h->efflen : nullptr;
     double *Sp = want_S ? h->S_partial : nullptr;
-    if (chain_path(h)) return launch_chain_fwd(h, KP, clamp_x, eff, Sp, want_ladj, ladj_tree);
-    if (dfs_fwd_ok(h)) {
-        const size_t smem = dfs_fwd_smem(h, KP);
-        if (smem > 40 * 1024) DISPATCH_KP(KP, allow_max_smem(k3d_tree_fwd<KPC>));
-        DISPATCH_KP(KP, (k3d_tree_fwd<KPC><<<td.dfs_ctas, DFS_RUNS_PER_CTA * KPC, smem, h->stream>>>(
-                            td.N, td.dnodes, td.drun_anc_ptr, td.drun_anc, td.dcta_k0, h->ys, h->us, h->x, clamp_x,
-                            want_ladj, ladj_tree, td.max_depth + 2, (std::max(td.dfs_max_nk, 1) + 1) & ~1)));
-        h->S_deferred = want_S != 0;  // launch_mid adds S = sum_j x_j / efflen_j (k3_leaf_S) beside the likelihood pass
-        return POLEE_OK;
+    int rc = POLEE_OK;
+    switch (tree_route(td, KP)) {
+        case TreeRoute::Chain:
+            return launch_chain_fwd(h, KP, clamp_x, eff, Sp, want_ladj, ladj_tree);
+        case TreeRoute::DfsRun: {
+            const size_t smem = dfs_fwd_smem(td, KP);
+            if (smem > 40 * 1024) DISPATCH_KP(KP, allow_max_smem(k3d_tree_fwd<KPC>));
+            DISPATCH_KP(KP, (k3d_tree_fwd<KPC><<<td.dfs_ctas, DFS_RUNS_PER_CTA * KPC, smem, h->stream>>>(
+                                td.N, td.dnodes, td.drun_anc_ptr, td.drun_anc, td.dcta_k0, h->ys, h->us, h->x, clamp_x,
+                                want_ladj, ladj_tree, td.max_depth + 2, (std::max(td.dfs_max_nk, 1) + 1) & ~1)));
+            h->S_deferred = want_S != 0;  // launch_mid adds S = sum_j x_j / efflen_j (k3_leaf_S) beside the likelihood pass
+            break;
+        }
+        case TreeRoute::PathProduct: {
+            const size_t smem = (size_t)td.max_ganc * (16 * KP + 2) + 16 + 2 * (size_t)td.max_gsuf;
+            if (smem > 40 * 1024) DISPATCH_KP(KP, allow_max_smem(k3p_tree_fwd<KPC>));
+            DISPATCH_KP(KP, (k3p_tree_fwd<KPC><<<td.n_groups, PATH_SLOTS * KPC, smem, h->stream>>>(
+                                td.N, td.nodes, td.ganc_ptr, td.ganc, td.gcp, td.nsuf_ptr, td.nsuf, h->ys, h->us, h->x, clamp_x,
+                                eff, Sp, want_ladj, ladj_tree)));
+            break;
+        }
+        case TreeRoute::SmemLevels:
+            DISPATCH_KP(KP, rc = launch_tree_fwd_smem<KPC>(h, clamp_x, eff, Sp, want_ladj, ladj_tree));
+            break;
+        case TreeRoute::GlobalLevels:
+            if (td.top.nbins > 0) {
+                DISPATCH_KP(KP, (k3_tree_fwd<KPC, TOP_THREADS><<<td.top.nbins, TOP_THREADS, 0, h->stream>>>(
+                                    td.top.bin_lvl_ptr, td.top.lvl_off, td.top.sch_node, td.nodes, h->ys, h->us, h->x, clamp_x,
+                                    eff, Sp, 0, want_ladj, ladj_tree)));
+            }
+            if (td.bottom.nbins > 0) {
+                DISPATCH_KP(KP, (k3_tree_fwd<KPC, TREE_THREADS><<<td.bottom.nbins, TREE_THREADS, 0, h->stream>>>(
+                                    td.bottom.bin_lvl_ptr, td.bottom.lvl_off, td.bottom.sch_node, td.nodes, h->ys, h->us, h->x,
+                                    clamp_x, eff, Sp, 1, want_ladj, ladj_tree)));
+            }
+            break;
     }
-    if (path_fwd_ok(h)) {
-        const size_t smem = (size_t)td.max_ganc * (16 * KP + 2) + 16 + 2 * (size_t)td.max_gsuf;
-        if (smem > 40 * 1024) DISPATCH_KP(KP, allow_max_smem(k3p_tree_fwd<KPC>));
-        DISPATCH_KP(KP, (k3p_tree_fwd<KPC><<<td.n_groups, PATH_SLOTS * KPC, smem, h->stream>>>(
-                            td.N, td.nodes, td.ganc_ptr, td.ganc, td.gcp, td.nsuf_ptr, td.nsuf, h->ys, h->us, h->x, clamp_x,
-                            eff, Sp, want_ladj, ladj_tree)));
-        return POLEE_OK;
-    }
-    if (smem_path_ok(h, KP)) {
-        int rc = POLEE_OK;
-        DISPATCH_KP(KP, rc = launch_tree_fwd_smem<KPC>(h, clamp_x, eff, Sp, want_ladj, ladj_tree));
-        return rc;
-    }
-    if (td.top.nbins > 0) {
-        DISPATCH_KP(KP, (k3_tree_fwd<KPC, TOP_THREADS><<<td.top.nbins, TOP_THREADS, 0, h->stream>>>(
-                            td.top.bin_lvl_ptr, td.top.lvl_off, td.top.sch_node, td.nodes, h->ys, h->us, h->x, clamp_x,
-                            eff, Sp, 0, want_ladj, ladj_tree)));
-    }
-    if (td.bottom.nbins > 0) {
-        DISPATCH_KP(KP, (k3_tree_fwd<KPC, TREE_THREADS><<<td.bottom.nbins, TREE_THREADS, 0, h->stream>>>(
-                            td.bottom.bin_lvl_ptr, td.bottom.lvl_off, td.bottom.sch_node, td.nodes, h->ys, h->us, h->x,
-                            clamp_x, eff, Sp, 1, want_ladj, ladj_tree)));
-    }
-    return POLEE_OK;
+    return rc;
 }
 
 int launch_mid(polee_handle *h, int KP, int advance, cudaStream_t st) {
@@ -1223,16 +1209,7 @@ int launch_mid(polee_handle *h, int KP, int advance, cudaStream_t st) {
 int launch_tree_bwd(polee_handle *h, int KP, bool with_ladj, bool apply_efflen, double *xgrad_out) {
     const TreeDev &td = h->td;
     const float *adj = apply_efflen ? h->efflen_adj : nullptr;
-    if (chain_path(h)) return launch_chain_bwd(h, KP, with_ladj, adj, xgrad_out);
-    if (smem_path_ok(h, KP)) {
-        int rc = POLEE_OK;
-        if (with_ladj) {
-            DISPATCH_KP(KP, (rc = launch_tree_bwd_smem<KPC, true>(h, adj, xgrad_out)));
-        } else {
-            DISPATCH_KP(KP, (rc = launch_tree_bwd_smem<KPC, false>(h, adj, xgrad_out)));
-        }
-        return rc;
-    }
+    int rc = POLEE_OK;
 #define BWD(SCHED, THREADS)                                                                                          \
     if (with_ladj) {                                                                                                 \
         DISPATCH_KP(KP, (k3_tree_bwd<KPC, THREADS, true><<<SCHED.nbins, THREADS, 0, h->stream>>>(                    \
@@ -1243,10 +1220,25 @@ int launch_tree_bwd(polee_handle *h, int KP, bool with_ladj, bool apply_efflen, 
                             SCHED.bin_lvl_ptr, SCHED.lvl_off, SCHED.sch_node, td.nodes, h->ys, h->us, h->g, adj, h->S, \
                             h->G, h->ygrad, xgrad_out)));                                                            \
     }
-    if (td.bottom.nbins > 0) { BWD(td.bottom, TREE_THREADS) }
-    if (td.top.nbins > 0) { BWD(td.top, TOP_THREADS) }
+    switch (tree_route(td, KP)) {
+        case TreeRoute::Chain:
+            return launch_chain_bwd(h, KP, with_ladj, adj, xgrad_out);
+        case TreeRoute::DfsRun:
+        case TreeRoute::PathProduct:
+        case TreeRoute::SmemLevels:
+            if (with_ladj) {
+                DISPATCH_KP(KP, (rc = launch_tree_bwd_smem<KPC, true>(h, adj, xgrad_out)));
+            } else {
+                DISPATCH_KP(KP, (rc = launch_tree_bwd_smem<KPC, false>(h, adj, xgrad_out)));
+            }
+            break;
+        case TreeRoute::GlobalLevels:
+            if (td.bottom.nbins > 0) { BWD(td.bottom, TREE_THREADS) }
+            if (td.top.nbins > 0) { BWD(td.top, TOP_THREADS) }
+            break;
+    }
 #undef BWD
-    return POLEE_OK;
+    return rc;
 }
 
 // Under CUDA's lazy module loading a kernel's code is loaded at its first launch (a few hundred microseconds to
@@ -1293,7 +1285,7 @@ int launch_tree_inv(polee_handle *h, int KP, const float *x_dev, double *us_tmp,
     const TreeDev &td = h->td;
     float *logu = ladj_out ? logu_tmp : nullptr;
     if (td.n < 2) return POLEE_OK;
-    if (chain_path(h)) {
+    if (tree_route(td, KP) == TreeRoute::Chain) {
         k3_tree_inv_serial<<<1, 32, 0, h->stream>>>(td.N, KP, td.nodes, x_dev, us_tmp, ys_out, logu);
     } else {
         if (td.bottom.nbins > 0) {

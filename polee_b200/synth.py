@@ -196,3 +196,33 @@ def random_tree(n, seed=0):
         b = items[j]
         items[j] = (a, b)
     return tree_from_nested(items[0], n)
+
+
+def spine_tree(n_spine, every):
+    """(node_parent_idxs, node_js) of a caterpillar of n_spine internal nodes in which every `every`-th right-hand leaf
+    is replaced by a 3-leaf subtree, in DFS pre-order.  With n_spine above 1 024 it is deep (no DFS-run inputs, more
+    than 1 024 ancestors per path group, so no root-path tables) and not a caterpillar (no chain scans), and its top
+    part fits in shared memory: the tree kernels' shared-memory level route."""
+    pi, js = [], []
+
+    def add(parent, leaf):
+        pi.append(parent)
+        js.append(leaf)
+        return len(pi)                                # 1-based index of the new node
+
+    leaves, parent = 0, 0
+    for s in range(n_spine):
+        me = add(parent, 0)
+        if s % every == every - 1:                    # the first child of a node is its right child
+            a = add(me, 0)
+            add(a, leaves + 1)
+            b = add(a, 0)
+            add(b, leaves + 2)
+            add(b, leaves + 3)
+            leaves += 3
+        else:
+            leaves += 1
+            add(me, leaves)
+        parent = me
+    add(parent, leaves + 1)
+    return np.array(pi, np.int32), np.array(js, np.int32)

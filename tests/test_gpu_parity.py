@@ -83,21 +83,41 @@ def _trees(fx):
     return {"fixture": (fx.parent_idxs, fx.js), "sequential": sequential_tree(fx.n),
             "random": synth.random_tree(fx.n, 3), "balanced": synth.balanced_tree(fx.n),
             # large trees: several bottom bins and a top part
-            "balanced_20001": synth.balanced_tree(20001), "random_6000": synth.random_tree(6000, 9)}
+            "balanced_20001": synth.balanced_tree(20001), "random_6000": synth.random_tree(6000, 9),
+            "random_6000_K16": synth.random_tree(6000, 9),
+            "spine_1225": synth.spine_tree(1200, 100), "sequential_6000": sequential_tree(6000)}
 
 
-@pytest.mark.parametrize("tree", ["fixture", "sequential", "random", "balanced", "balanced_20001", "random_6000"])
-def test_tree_forward_backward_bit_exact(pb, fx, oracle, tree):
+# the kernels each tree of test_tree_forward_backward_bit_exact takes (Handle.layout_info()["tree_route"]);
+# sequential_6000 runs with POLEE_CHAIN_MIN_NODES raised, so that it does not take the chain scans
+_TREE_ROUTES = {"fixture": "dfs", "sequential": "path", "random": "dfs", "balanced": "dfs", "balanced_20001": "dfs",
+                "random_6000": "dfs", "random_6000_K16": "dfs", "spine_1225": "levels_smem",
+                "sequential_6000": "levels_global"}
+
+
+@pytest.mark.parametrize("tree", list(_TREE_ROUTES))
+def test_tree_forward_backward_bit_exact(pb, fx, oracle, tree, monkeypatch):
+    """transform!, both transform_gradients and inverse_transform! bit for bit against the oracle, on every route but
+    the chain scans (test_large_sequential_tree_scan_path); random_6000_K16 runs 16 draws, where the DFS-run kernel
+    needs 4 times the shared memory of K = 4."""
     pi, js = _trees(fx)[tree]
     n = (len(pi) + 1) // 2
-    K = 4
+    K = 16 if tree.endswith("_K16") else 4
     rng = np.random.default_rng(1)
-    lo = 0.3 if tree == "sequential" else 0.01       # keep a depth-312 product inside the Float32 range
-    ys = rng.uniform(lo, 0.99, (K, n - 1))
-    x_grad = rng.normal(size=(K, n)) * 1000
-    t = pb.PolyaTreeTransform(pi, js)
     to = oracle.PTT(pi, js)
+    if tree in ("spine_1225", "sequential_6000"):
+        # ys of a near-uniform composition: u stays O(1/n) along paths of 1200 or 6000 nodes
+        x0 = rng.dirichlet(np.ones(n) * 5.0, K).astype(np.float32)
+        ys = np.stack([to.inverse_transform(x0[k])[0] for k in range(K)])
+    else:
+        lo = 0.3 if tree == "sequential" else 0.01   # keep a depth-312 product inside the Float32 range
+        ys = rng.uniform(lo, 0.99, (K, n - 1))
+    x_grad = rng.normal(size=(K, n)) * 1000
+    if tree == "sequential_6000":
+        monkeypatch.setenv("POLEE_CHAIN_MIN_NODES", str(10 ** 9))
+    t = pb.PolyaTreeTransform(pi, js)
     xs, ladj = t.transform(ys, compute_ladj=True)
+    assert t.handle.layout_info()["tree_route"] == _TREE_ROUTES[tree]
     yg = t.transform_gradients(ys, x_grad)
     yg0 = t.transform_gradients_no_ladj(ys, x_grad)
     for k in range(K):
@@ -481,6 +501,9 @@ def test_large_sequential_tree_scan_path(pb, oracle):
     ys = np.stack([to.inverse_transform(x0[k])[0] for k in range(K)])
     t = pb.PolyaTreeTransform(pi, js)
     xs, ladj = t.transform(ys, compute_ladj=True)
+    assert t.handle.layout_info()["tree_route"] == "chain"
+    # with the trees of test_tree_forward_backward_bit_exact, every route is taken
+    assert set(_TREE_ROUTES.values()) | {"chain"} == {"chain", "dfs", "path", "levels_smem", "levels_global"}
     x_grad = rng.normal(size=(K, n)) * 100
     yg = t.transform_gradients(ys, x_grad)
     yg0 = t.transform_gradients_no_ladj(ys, x_grad)
