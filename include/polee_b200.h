@@ -158,8 +158,9 @@ int polee_step_stats(polee_handle *h, double *bytes_k1, double *bytes_k2, double
  * equivalence-class layout; info[6..7] = rows, entries of the general layouts; info[8] = their kind (0 none,
  * 1 split, 2 fused); info[9] = padded row slots of the class layout; info[10] = the kernels the tree takes at the
  * draw count the work buffers were last sized for (0 chain scans, 1 DFS runs, 2 path products, 3 shared-memory
- * levels, 4 global-memory levels; -1 without a tree or before the first call that sizes them).  count <= 11 values
- * are written. */
+ * levels, 4 global-memory levels; -1 without a tree or before the first call that sizes them); info[11], info[12] =
+ * programmatic edges (PDL launches of consecutive step kernels) in the captured one-step and multi-step graphs of
+ * polee_run_steps, -1 while that graph is not captured.  count <= 13 values are written. */
 int polee_layout_info(polee_handle *h, int64_t *info, int32_t count);
 /* time (ms, CUDA events on the handle's stream) of `reps` launches of one named kernel group:
  * which = 1 (the likelihood pass; K1 alone on the pure split layout), 2 (K2 of the pure split layout),

@@ -214,10 +214,11 @@ class Handle:
         return {"bytes_k1": b[0].value, "bytes_k2": b[1].value, "bytes_k3": b[2].value, "launches": nl.value}
 
     def layout_info(self):
-        v = (C.c_int64 * 11)()
-        self.check(self.lib.polee_layout_info(self.h, v, C.c_int32(11)))
+        v = (C.c_int64 * 13)()
+        self.check(self.lib.polee_layout_info(self.h, v, C.c_int32(13)))
         keys = ("ec_rows", "ec_nnz", "ec_classes", "ec_tasks", "ec_blob_bytes", "ec_partials", "general_rows",
-                "general_nnz", "general_kind", "ec_row_slots", "tree_route")
+                "general_nnz", "general_kind", "ec_row_slots", "tree_route", "graph_programmatic_edges",
+                "multi_step_graph_programmatic_edges")
         out = dict(zip(keys, (int(x) for x in v)))
         out["general_kind"] = ("none", "split", "fused")[out["general_kind"]]
         # the kernels the tree takes at the draw count of the last call (None: no tree, or no call yet)

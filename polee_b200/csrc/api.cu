@@ -56,12 +56,20 @@ static std::mutex g_err_mu;
     if (cudaSetDevice((h)->device) != cudaSuccess) return (h)->fail(POLEE_ECUDA, "cudaSetDevice failed")
 
 constexpr int TREE_BIN_NODES = 512;  // nodes per bottom bin of the tree schedule
+// steps per launch of the multi-step graph: inside it the step boundary (k3_elem -> tree forward) is a programmatic edge
+// too, and one graph launch replaces STEP_GRAPH_STEPS
+constexpr int STEP_GRAPH_STEPS = 8;
+constexpr int STEP_GRAPH_LEAD = 3;  // steps queued before the multi-step graph is captured (polee_run_steps)
 
 static void drop_graph(polee_handle *h) {
     if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
     if (h->graph) cudaGraphDestroy(h->graph);
+    if (h->graph_multi_exec) cudaGraphExecDestroy(h->graph_multi_exec);
+    if (h->graph_multi) cudaGraphDestroy(h->graph_multi);
     h->graph_exec = nullptr;
     h->graph = nullptr;
+    h->graph_multi_exec = nullptr;
+    h->graph_multi = nullptr;
     h->graph_warm = false;
 }
 
@@ -140,6 +148,7 @@ extern "C" int polee_create(polee_handle **out, const polee_opts *opts) {
     h->num_sms = sm_count;
     h->K = o.num_mc_samples;
     h->KP = pad_k(h->K);
+    h->pdl = !(getenv("POLEE_PDL") && !strcmp(getenv("POLEE_PDL"), "0"));
     if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaStreamCreateWithFlags(&h->side_stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
@@ -625,6 +634,37 @@ static int ensure_reparam(polee_handle *h) {
     return POLEE_OK;
 }
 
+// nsteps consecutive steps captured into one graph.  The step number and the learning rate live in device memory
+// (StepCtl), so a replay is the same as enqueueing the steps one by one.
+static int capture_steps(polee_handle *h, int nsteps, cudaGraph_t *graph, cudaGraphExec_t *exec) {
+    const float *noise = h->o.noise_mode == POLEE_NOISE_INJECTED ? h->noise : nullptr;
+    // Relaxed: other host threads (one handle per thread in `polee prep`) may allocate, free or synchronise while
+    // this thread records; the handle's streams are non-blocking, so nothing they do can join this capture.
+    std::shared_lock<std::shared_mutex> cap(polee::capture_mutex());  // no device-wide sync anywhere meanwhile
+    CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeRelaxed));
+    int rc = POLEE_OK;
+    for (int s = 0; s < nsteps && !rc; ++s)
+        rc = launch_step_sequence(h, true, true, nullptr, nullptr, noise, std::max<int64_t>(h->noise_steps, 1));
+    cudaError_t e = cudaStreamEndCapture(h->stream, graph);
+    if (rc) return rc;
+    if (e != cudaSuccess) return h->fail(POLEE_ECUDA, std::string("graph capture: ") + cudaGetErrorString(e));
+    CK(cudaGraphInstantiate(exec, *graph, 0));
+    return POLEE_OK;
+}
+
+// STEP_GRAPH_STEPS steps in one graph launch; the caller has run enqueue_step at least once
+static int enqueue_step_chunk(polee_handle *h) {
+    int rc = ensure_reparam(h);  // init_params, set_params, polee_sample ... leave ys / zs0 for the graph to redo
+    if (rc) return rc;
+    if (!h->graph_multi_exec) {
+        HostPhaseTimer pt;
+        if ((rc = capture_steps(h, STEP_GRAPH_STEPS, &h->graph_multi, &h->graph_multi_exec))) return rc;
+        pt.mark("multi-step graph: capture + inst.");
+    }
+    CK(cudaGraphLaunch(h->graph_multi_exec, h->stream));
+    return POLEE_OK;
+}
+
 static int enqueue_step(polee_handle *h) {
     const float *noise = h->o.noise_mode == POLEE_NOISE_INJECTED ? h->noise : nullptr;
     int rc = ensure_reparam(h);
@@ -647,18 +687,9 @@ static int enqueue_step(polee_handle *h) {
         return POLEE_OK;
     }
     if (!h->graph_exec) {
-        // Relaxed: other host threads (one handle per thread in `polee prep`) may allocate, free or synchronise while
-        // this thread records; the handle's streams are non-blocking, so nothing they do can join this capture.
         HostPhaseTimer pt;
-        std::shared_lock<std::shared_mutex> cap(polee::capture_mutex());  // no device-wide sync anywhere meanwhile
-        CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeRelaxed));
-        rc = launch_step_sequence(h, true, true, nullptr, nullptr, noise, std::max<int64_t>(h->noise_steps, 1));
-        cudaError_t e = cudaStreamEndCapture(h->stream, &h->graph);
-        if (rc) return rc;
-        if (e != cudaSuccess) return h->fail(POLEE_ECUDA, std::string("graph capture: ") + cudaGetErrorString(e));
-        pt.mark("second step: capture");
-        CK(cudaGraphInstantiate(&h->graph_exec, h->graph, 0));
-        pt.mark("graph instantiate");
+        if ((rc = capture_steps(h, 1, &h->graph, &h->graph_exec))) return rc;
+        pt.mark("second step: capture + instantiate");
     }
     CK(cudaGraphLaunch(h->graph_exec, h->stream));
     return POLEE_OK;
@@ -671,10 +702,22 @@ extern "C" int polee_run_steps(polee_handle *h, int32_t nsteps) {
     int rc = ready_for_steps(h);
     if (rc) return rc;
     pt.mark("run_steps: work buffers");
-    for (int s = 0; s < nsteps; ++s) {
-        if ((rc = enqueue_step(h))) return rc;
-        h->steps_enqueued++;
-        if (h->progress_cb && h->progress_every > 0 && (h->steps_enqueued % h->progress_every == 0 || s + 1 == nsteps)) {
+    const bool progress = h->progress_cb && h->progress_every > 0;
+    for (int s = 0; s < nsteps;) {
+        // the multi-step graph once the one-step graph exists, while a whole chunk remains and no progress report
+        // falls inside it (one may fall on its last step).  It is captured only after this call has queued
+        // STEP_GRAPH_LEAD steps: its capture and instantiation (~1 ms of host time) then overlap their execution
+        // instead of leaving the device idle.
+        int chunk = 1;
+        if (h->graph_exec && (h->graph_multi_exec || s >= STEP_GRAPH_LEAD) && nsteps - s >= STEP_GRAPH_STEPS) {
+            chunk = STEP_GRAPH_STEPS;
+            for (int j = 1; progress && j < STEP_GRAPH_STEPS; ++j)
+                if ((h->steps_enqueued + j) % h->progress_every == 0) chunk = 1;
+        }
+        if ((rc = chunk > 1 ? enqueue_step_chunk(h) : enqueue_step(h))) return rc;
+        h->steps_enqueued += chunk;
+        s += chunk;
+        if (progress && (h->steps_enqueued % h->progress_every == 0 || s == nsteps)) {
             CK(cudaStreamSynchronize(h->stream));  // the bar reports finished steps, not enqueued ones
             h->progress_cb(h->steps_enqueued, h->o.num_steps, h->progress_user);
         }
@@ -1040,18 +1083,32 @@ extern "C" int polee_step_stats(polee_handle *h, double *b1, double *b2, double 
     return POLEE_OK;
 }
 
+// programmatic edges of a captured graph (the PDL launches between consecutive step kernels), -1 without a graph
+static int64_t programmatic_edges(cudaGraph_t g) {
+    if (!g) return -1;
+    size_t n = 0;
+    if (cudaGraphGetEdges_v2(g, nullptr, nullptr, nullptr, &n) != cudaSuccess) return -1;
+    std::vector<cudaGraphNode_t> from(n), to(n);
+    std::vector<cudaGraphEdgeData> data(n);
+    if (n > 0 && cudaGraphGetEdges_v2(g, from.data(), to.data(), data.data(), &n) != cudaSuccess) return -1;
+    int64_t count = 0;
+    for (size_t i = 0; i < n; ++i) count += data[i].type == cudaGraphDependencyTypeProgrammatic;
+    return count;
+}
+
 // Which layouts hold the matrix: info[0..9] = {rows, entries, classes, tasks, blob bytes, partials} of the
 // equivalence-class layout, {rows, entries} of the general layouts, general layout kind (0 none, 1 split, 2 fused),
 // padded row slots of the class layout; info[10] = the tree route (TreeRoute) at the work buffers' KP, -1 without a tree
-// or work buffers.
+// or work buffers; info[11], info[12] = programmatic edges of the captured one-step and multi-step graphs, -1 while
+// not captured.
 extern "C" int polee_layout_info(polee_handle *h, int64_t *info, int32_t count) {
     CHECK_H(h);
     if (!info || count < 1) return h->fail(POLEE_EINVAL, "layout_info: bad arguments");
     const int64_t route = h->have_tree && h->work_KP > 0 ? (int64_t)tree_route(h->td, h->work_KP) : -1;
-    const int64_t v[11] = {h->ec_rows, h->ec_nnz, h->ec_classes, (int64_t)h->ec_tasks, (int64_t)h->ec_blob_bytes, h->ec_parts,
+    const int64_t v[13] = {h->ec_rows, h->ec_nnz, h->ec_classes, (int64_t)h->ec_tasks, (int64_t)h->ec_blob_bytes, h->ec_parts,
                            h->gm, h->gnnz, (int64_t)((h->gm > 0 || h->ec_tasks == 0) ? (h->fused ? 2 : 1) : 0), h->ec_slots,
-                           route};
-    for (int i = 0; i < count && i < 11; ++i) info[i] = v[i];
+                           route, programmatic_edges(h->graph), programmatic_edges(h->graph_multi)};
+    for (int i = 0; i < count && i < 13; ++i) info[i] = v[i];
     return POLEE_OK;
 }
 

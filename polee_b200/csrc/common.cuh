@@ -6,6 +6,7 @@
 #include <stdint.h>
 
 #include <shared_mutex>
+#include <utility>
 #include <string>
 #include <vector>
 
@@ -413,10 +414,13 @@ struct polee_handle {
     int work_KP = 0;                      // KP the work buffers were sized for
     int n_tree_ctas = 0;
 
-    // ---- graph
+    // ---- graph: one step, and STEP_GRAPH_STEPS consecutive steps (api.cu)
     cudaGraph_t graph = nullptr;
     cudaGraphExec_t graph_exec = nullptr;
+    cudaGraph_t graph_multi = nullptr;
+    cudaGraphExec_t graph_multi_exec = nullptr;
     bool graph_warm = false;  // one uncaptured step has run with the current layouts
+    bool pdl = true;          // step kernels launched with programmatic stream serialization (POLEE_PDL=0: plainly)
 
 #ifdef POLEE_WITH_NCCL
     ncclComm_t comm = nullptr;
@@ -468,6 +472,26 @@ inline cudaError_t allow_max_smem(F func) {
     cudaError_t e = cudaFuncGetAttributes(&a, func);
     if (e != cudaSuccess) return e;
     return cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM_PER_CTA - (int)a.sharedSizeBytes);
+}
+
+// Launch of a kernel that follows the pdl_wait() rule (device_utils.cuh) with programmatic stream serialization: it may
+// start, and run its part before pdl_wait(), while the kernel before it on the stream drains.  Under stream capture the
+// launch becomes a programmatic graph edge.  Only kernels that contain the wait go through here.  As with <<< >>>, a
+// launch error surfaces through cudaGetLastError.
+template <typename... P, typename... A>
+inline void launch_pdl(const polee_handle *h, void (*kern)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                       A &&...args) {
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr.val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cfg.attrs = &attr;
+    cfg.numAttrs = h->pdl ? 1 : 0;
+    cudaLaunchKernelEx(&cfg, kern, std::forward<A>(args)...);
 }
 
 // Device-wide synchronisation (explicit, or implied by cudaFree / cudaMalloc) is not permitted while ANY stream of the

@@ -103,6 +103,21 @@ __device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t by
 }
 __device__ __forceinline__ void consumer_bar_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
 
+// ---------------------------------------------------------------- programmatic dependent launch
+// A kernel launched through launch_pdl (common.cuh) may start while the kernel before it on the stream is still running;
+// pdl_wait() returns once that kernel has completed and its writes are visible.  The rule every such kernel follows:
+//   - before pdl_wait() it reads only data that no kernel of the step loop writes: layouts, node records, schedules,
+//     unit / task descriptors, the class blob, the seed and its arguments;
+//   - x, ys, us, g, the partial sums, S, the StepCtl counters, the parameters and the ADAM state are read only after it,
+//     and every write to global memory comes after it;
+//   - every CTA executes pdl_wait(), on paths that exit early and write nothing too: a kernel's completion must still
+//     imply the completion of every kernel before it, or a chain of early launches could run ahead of a kernel two
+//     launches back.
+// pdl_trigger() lets the next kernel's CTAs be scheduled once every CTA of this one has triggered or exited; it orders
+// nothing, so where it stands is a matter of speed only.  Both are no-ops in a kernel launched without the attribute.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
 __device__ __forceinline__ float rcp_approx(float x) {
     float r;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));

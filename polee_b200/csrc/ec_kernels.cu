@@ -501,7 +501,10 @@ __global__ void __launch_bounds__(EcCfg<T>::WARPS * 32, 1)
     W.G = gridDim.x * Cfg::WARPS;
     W.tk = blockIdx.x * Cfg::WARPS + warp;
     W.n_tasks = n_tasks;
-    if (W.tk >= n_tasks) return;
+    if (W.tk >= n_tasks) {
+        pdl_wait();
+        return;
+    }
     W.mine_u32 = smem_u32(mine);
     W.bar_u32 = smem_u32(bars);
     if (lane == 0) {
@@ -518,6 +521,8 @@ __global__ void __launch_bounds__(EcCfg<T>::WARPS * 32, 1)
         }
     }
     __syncwarp();
+    // the copies above read only the constant blob; x is the tree forward's output
+    pdl_wait();
     W.s = 0;
     mbar_wait_u32(W.bar_u32, 0u);
     W.phase = 1u;
@@ -526,6 +531,8 @@ __global__ void __launch_bounds__(EcCfg<T>::WARPS * 32, 1)
     if (W.tk < kinds.end[i]) ec_run<T, KD, 8 - (i), FULL>(W, kinds.end[i], mine, xbuf, desc, blob, A, lane)
     EC_KIND(0); EC_KIND(1); EC_KIND(2); EC_KIND(3); EC_KIND(4); EC_KIND(5); EC_KIND(6); EC_KIND(7);
 #undef EC_KIND
+    // not at the start: the next kernel's waiting CTAs would take SM space k3_leaf_S uses beside this kernel
+    pdl_trigger();
 }
 
 // g[col] (or a level-2 slot) = [g[col] +] sum of <= FT_UNIT partials of one column, in task order, in Float64
@@ -537,8 +544,11 @@ __global__ void __launch_bounds__(256)
     const int warp_global = (int)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5);
     const int lane = threadIdx.x & 31;
     const int unit = warp_global * GP + lane / KP, k = lane % KP;
+    pdl_trigger();
+    FusedUnit u{};
+    if (unit < n_units) u = units[unit];
+    pdl_wait();
     if (unit >= n_units) return;
-    const FusedUnit u = units[unit];
     double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
     uint32_t i = u.begin;
     for (; i + 4 <= u.end; i += 4) {
@@ -562,11 +572,14 @@ __global__ void __launch_bounds__(256)
     k_ec_combine2(const FusedMulti *__restrict__ multi, int n_multi, const double *__restrict__ lvl2, double *__restrict__ g,
                   int add_to_g) {
     const int idx = (int)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5);
+    pdl_trigger();
+    FusedMulti mc{};
+    if (idx < n_multi) mc = multi[idx];
+    pdl_wait();
     if (idx >= n_multi) return;
     const int lane = threadIdx.x & 31;
     constexpr int GP = 32 / KP;
     const int grp = lane / KP, k = lane % KP;
-    const FusedMulti mc = multi[idx];
     double a = 0.0;
     for (uint32_t i = grp; i < mc.count; i += GP) a += lvl2[(size_t)(mc.first + i) * KP + k];
 #pragma unroll
@@ -601,7 +614,7 @@ int launch_lik_full(polee_handle *h, const EcArgs &A) {
     const int grid = std::max(1, std::min(h->ec_grid, (h->ec_tasks + EcCfg<T>::WARPS - 1) / EcCfg<T>::WARPS));
     EcKinds kinds;
     for (int i = 0; i < 8; ++i) kinds.end[i] = h->ec_kind_end[i];
-    kern<<<grid, EcCfg<T>::WARPS * 32, EcCfg<T>::SMEM, h->stream>>>(h->ec_desc, h->ec_tasks, h->ec_blob, A, kinds);
+    launch_pdl(h, kern, grid, EcCfg<T>::WARPS * 32, EcCfg<T>::SMEM, h->stream, h->ec_desc, h->ec_tasks, h->ec_blob, A, kinds);
     return POLEE_OK;
 }
 
@@ -628,12 +641,12 @@ void launch_combine(polee_handle *h, double *g, bool add_to_g) {
     if (h->ec_nunits > 0) {
         const int units_per_block = 8 * (32 / KP);
         const int blocks = (h->ec_nunits + units_per_block - 1) / units_per_block;
-        k_ec_combine1<P, KP><<<blocks, 256, 0, h->stream>>>(h->ec_units, h->ec_nunits, reinterpret_cast<const P *>(h->ec_partial), g,
-                                                            h->ec_lvl2, add_to_g ? 1 : 0);
+        launch_pdl(h, k_ec_combine1<P, KP>, blocks, 256, 0, h->stream, h->ec_units, h->ec_nunits,
+                   reinterpret_cast<const P *>(h->ec_partial), g, h->ec_lvl2, add_to_g ? 1 : 0);
     }
     if (h->ec_nmulti > 0) {
         const int blocks = (h->ec_nmulti + 7) / 8;
-        k_ec_combine2<KP><<<blocks, 256, 0, h->stream>>>(h->ec_multi, h->ec_nmulti, h->ec_lvl2, g, add_to_g ? 1 : 0);
+        launch_pdl(h, k_ec_combine2<KP>, blocks, 256, 0, h->stream, h->ec_multi, h->ec_nmulti, h->ec_lvl2, g, add_to_g ? 1 : 0);
     }
 }
 

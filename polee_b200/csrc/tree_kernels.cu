@@ -387,8 +387,10 @@ __global__ void __launch_bounds__(THREADS, MINB)
     constexpr int NPP = THREADS / KPC;
     const int l0 = bin_lvl_ptr[blockIdx.x], nlev = bin_lvl_ptr[blockIdx.x + 1] - 1 - l0;
 
+    pdl_trigger();
     for (int p = threadIdx.x; p < nb; p += THREADS) rec_s[p] = recs[q0 + p];
     for (int l = threadIdx.x; l <= nlev; l += THREADS) lvl_s[l] = lvl_off[l0 + l] - q0;
+    pdl_wait();  // the schedule above is constant; ys, us_k, g, root_G and S come from this step's kernels
     __syncthreads();
     const double Sk = efflen_adj ? S[k] : 1.0;
     for (int base = slot_t; base < nb; base += 4 * NPP) {
@@ -576,8 +578,10 @@ __global__ void __launch_bounds__(DFS_RUNS_PER_CTA *KP)
     const int64_t c0 = (int64_t)blockIdx.x * DFS_CTA_NODES;
     const int nn = (int)(N - c0 < DFS_CTA_NODES ? N - c0 : DFS_CTA_NODES);
     const int k0 = cta_k0[blockIdx.x], nk = cta_k0[blockIdx.x + 1] - k0;
-    // ---- stage the CTA's y slice (one contiguous piece of ys) and node records with 1-D bulk copies (TMA) completing
-    // on an mbarrier; they are in flight while the threads walk the root paths
+    pdl_trigger();
+    // ---- stage the CTA's node records and y slice (one contiguous piece of ys) with 1-D bulk copies (TMA) completing
+    // on an mbarrier; they are in flight while the threads walk the root paths.  The records (and the first batch of
+    // each run's ancestor list below) are constant and requested before pdl_wait(); ys is the previous step's output.
     __shared__ uint64_t bar;
     const bool bulk = KP >= 2;  // 16-byte granularity: k0 KP and nk KP doubles are even then
     if (bulk) {
@@ -590,30 +594,41 @@ __global__ void __launch_bounds__(DFS_RUNS_PER_CTA *KP)
             // 8-byte records, 16-byte copies: an odd tail takes the padding record the host appended
             const int nn2 = (nn + 1) & ~1;
             mbar_expect_tx(&bar, (uint32_t)(nk * KP * 8 + nn2 * (int)sizeof(DNode)));
-            if (nk > 0) bulk_g2s(ys_s, ys + (size_t)k0 * KP, (uint32_t)(nk * KP * 8), &bar);
             for (int q = 0; q * DFS_RUN < nn2; ++q) {
                 const int len = nn2 - q * DFS_RUN < DFS_RUN ? nn2 - q * DFS_RUN : DFS_RUN;
                 bulk_g2s(rec_s + q * RS, dnodes + c0 + (int64_t)q * DFS_RUN, (uint32_t)(len * sizeof(DNode)), &bar);
             }
         }
     } else {
-        for (int idx = threadIdx.x; idx < nk * KP; idx += THREADS) ys_s[idx] = ys[(size_t)k0 * KP + idx];
         for (int idx = threadIdx.x; idx < nn; idx += THREADS) rec_s[(idx / DFS_RUN) * RS + idx % DFS_RUN] = dnodes[c0 + idx];
     }
     // ---- the run's starting state: down the root path of its first node
+    constexpr int AB = 16;  // ancestors per batch: their y are all requested before the first product
     const int64_t i0 = c0 + (int64_t)rl * DFS_RUN;
     const int cnt = i0 < N ? (int)(N - i0 < DFS_RUN ? N - i0 : DFS_RUN) : 0;
+    uint32_t a0 = 0, na = 0, en[AB];
+    if (cnt > 0) {
+        const int64_t run = i0 / DFS_RUN;
+        a0 = run_anc_ptr[run];
+        na = run_anc_ptr[run + 1] - a0;
+    }
+#pragma unroll
+    for (int j = 0; j < AB; ++j) en[j] = j < (int)na ? run_anc[a0 + j] : 0u;
+    pdl_wait();
+    if (bulk) {
+        if (threadIdx.x == 0 && nk > 0) bulk_g2s(ys_s, ys + (size_t)k0 * KP, (uint32_t)(nk * KP * 8), &bar);
+    } else {
+        for (int idx = threadIdx.x; idx < nk * KP; idx += THREADS) ys_s[idx] = ys[(size_t)k0 * KP + idx];
+    }
     double *st = stack + threadIdx.x;
     double u = 1.0;
     if (cnt > 0) {
-        constexpr int AB = 16;  // ancestors per batch: their y are all requested before the first product
-        const int64_t run = i0 / DFS_RUN;
-        const uint32_t a0 = run_anc_ptr[run], na = run_anc_ptr[run + 1] - a0;
         for (uint32_t a = 0; a < na; a += AB) {
-            uint32_t en[AB];
             double yv[AB];
+            if (a > 0) {
 #pragma unroll
-            for (int j = 0; j < AB; ++j) en[j] = a + j < na ? run_anc[a0 + a + j] : 0u;
+                for (int j = 0; j < AB; ++j) en[j] = a + j < na ? run_anc[a0 + a + j] : 0u;
+            }
 #pragma unroll
             for (int j = 0; j < AB; ++j) yv[j] = a + j < na ? ys[(size_t)(en[j] >> 1) * KP + k] : 0.0;
 #pragma unroll
@@ -789,6 +804,8 @@ __global__ void __launch_bounds__(ELEM_THREADS)
             const float *__restrict__ noise, int64_t noise_steps, uint64_t seed, int fast_noise, int want_ladj,
             double *__restrict__ ladj_partial /* [2][gridDim.x][KP] */, int step0_fixed, int clamp_y) {
     __shared__ double sm[ELEM_THREADS];
+    pdl_trigger();
+    pdl_wait();  // everything this kernel reads, the step counters included, is written inside the step loop
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     const bool live = i < nm1;
     float p_mu = 0.f, p_om = 0.f, p_al = 0.f;
@@ -1048,11 +1065,11 @@ int launch_elem(polee_handle *h, int KP, int K, bool do_update, bool do_adam, bo
     const int mode = h->o.approx == POLEE_APPROX_OPTIMIZE_PTT ? 1 : 0;
     AdamCfg cfg{h->o.max_step_mu, h->o.max_step_omega, h->o.max_step_alpha, h->o.max_step_z};
     const int ctas = elem_ctas(h, KP);
-    DISPATCH_KP(KP, (k3_elem<KPC><<<ctas, ELEM_THREADS, 0, h->stream>>>(
+    DISPATCH_KP(KP, launch_pdl(h, k3_elem<KPC>, ctas, ELEM_THREADS, 0, h->stream,
                         nm1, K, mode, do_update ? 1 : 0, do_adam ? 1 : 0, do_reparam ? 1 : 0, h->mu, h->omega, h->alpha, h->m_mu,
                         h->m_omega, h->m_alpha, h->v_mu, h->v_omega, h->v_alpha, h->zs0, h->ys, h->ygrad, h->d_step, cfg,
                         h->d_bad_step, grad_out, noise, std::max<int64_t>(noise_steps, 1),
-                        step0_fixed >= 0 ? seed_override : h->o.seed, 1, want_ladj, h->ladj_partial, step0_fixed, clamp_y)));
+                        step0_fixed >= 0 ? seed_override : h->o.seed, 1, want_ladj, h->ladj_partial, step0_fixed, clamp_y));
     return POLEE_OK;
 }
 
@@ -1132,17 +1149,16 @@ static int launch_tree_bwd_smem(polee_handle *h, const float *adj, double *xgrad
         const size_t smem = (size_t)td.s_bottom.max_bin_nodes * (sizeof(SNode) + 24 * KPC) + 4 * (td.s_bottom.max_bin_levels + 2);
         auto fn = k3s_tree_bwd<KP, KPC, TREE_THREADS, bottom_minb(KP), WITH_LADJ>;
         allow_max_smem(fn);
-        fn<<<dim3(td.s_bottom.nbins, KP / KPC), TREE_THREADS, smem, h->stream>>>(
-            td.s_bottom.bin_off, td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->us, h->root_G, h->g,
-            adj, h->S, h->ygrad, xgrad_out);
+        launch_pdl(h, fn, dim3(td.s_bottom.nbins, KP / KPC), TREE_THREADS, smem, h->stream, td.s_bottom.bin_off,
+                   td.s_bottom.bin_lvl_ptr, td.s_bottom.lvl_off, td.s_bottom.recs, h->ys, h->us, h->root_G, h->g, adj, h->S,
+                   h->ygrad, xgrad_out);
     }
     if (td.s_top.nbins > 0) {
         const size_t smem = (size_t)td.s_top.max_bin_nodes * (sizeof(SNode) + 24) + 4 * (td.s_top.max_bin_levels + 2);
         auto fn = k3s_tree_bwd<KP, 1, S_TOP_THREADS, 1, WITH_LADJ>;
         allow_max_smem(fn);
-        fn<<<dim3(td.s_top.nbins, KP), S_TOP_THREADS, smem, h->stream>>>(
-            td.s_top.bin_off, td.s_top.bin_lvl_ptr, td.s_top.lvl_off, td.s_top.recs, h->ys, h->us, h->root_G, h->g, adj,
-            h->S, h->ygrad, xgrad_out);
+        launch_pdl(h, fn, dim3(td.s_top.nbins, KP), S_TOP_THREADS, smem, h->stream, td.s_top.bin_off, td.s_top.bin_lvl_ptr,
+                   td.s_top.lvl_off, td.s_top.recs, h->ys, h->us, h->root_G, h->g, adj, h->S, h->ygrad, xgrad_out);
     }
     return POLEE_OK;
 }
@@ -1159,9 +1175,9 @@ int launch_tree_fwd(polee_handle *h, int KP, int clamp_x, int want_S, int want_l
         case TreeRoute::DfsRun: {
             const size_t smem = dfs_fwd_smem(td, KP);
             if (smem > 40 * 1024) DISPATCH_KP(KP, allow_max_smem(k3d_tree_fwd<KPC>));
-            DISPATCH_KP(KP, (k3d_tree_fwd<KPC><<<td.dfs_ctas, DFS_RUNS_PER_CTA * KPC, smem, h->stream>>>(
-                                td.N, td.dnodes, td.drun_anc_ptr, td.drun_anc, td.dcta_k0, h->ys, h->us, h->x, clamp_x,
-                                want_ladj, ladj_tree, td.max_depth + 2, (std::max(td.dfs_max_nk, 1) + 1) & ~1)));
+            DISPATCH_KP(KP, launch_pdl(h, k3d_tree_fwd<KPC>, td.dfs_ctas, DFS_RUNS_PER_CTA * KPC, smem, h->stream, td.N,
+                                       td.dnodes, td.drun_anc_ptr, td.drun_anc, td.dcta_k0, h->ys, h->us, h->x, clamp_x,
+                                       want_ladj, ladj_tree, td.max_depth + 2, (std::max(td.dfs_max_nk, 1) + 1) & ~1));
             h->S_deferred = want_S != 0;  // launch_mid adds S = sum_j x_j / efflen_j (k3_leaf_S) beside the likelihood pass
             break;
         }
