@@ -239,6 +239,19 @@ int polee_approx_log_prob_with_plan(const polee_hsb_plan *plan, int64_t B, int64
 int polee_approx_log_prob_device(const polee_hsb_plan *plan, int64_t B, int64_t param_batch, const float *d_x,
                                  const float *d_mu, const float *d_omega, const float *d_alpha, double *d_lp,
                                  float *d_x_grad, void *stream);
+/* HSBGrad, the gradient of HSB that the reference's op file leaves as a TODO (hsb_ops.cpp:123-125; DESIGN.md K4):
+ * x_grad [B][n] = dL/dx, y_logit [B][n-1] as HSB took it, y_logit_grad [B][n-1] = dL/dy_logit.  With y_k =
+ * 1 / (1 + exp(-y_logit_k)) and u_j (u_root = 1, u_left = y u_j, u_right = (1 - y) u_j) exactly as HSB makes them, in
+ * Float64 without contraction: G = x_grad at a leaf, G_j = y G_l + (1 - y) G_r at internal node j (index k), and
+ * y_logit_grad_k = Float32(((y (1 - y)) u_j) (G_l - G_r)).  The Float32 rounding of x is treated as the identity.  Every
+ * value depends only on a node's parent or children, so the result does not depend on the schedule; no atomics.
+ * Non-finite inputs propagate; n == 1 gives an empty output. */
+int polee_hsb_grad(int32_t device, int64_t B, int64_t n, const float *x_grad, const float *y_logit, const int32_t *left,
+                   const int32_t *right, const int32_t *leaf, int64_t idx_batch, float *y_logit_grad);
+int polee_hsb_grad_with_plan(const polee_hsb_plan *plan, int64_t B, const float *x_grad, const float *y_logit,
+                             float *y_logit_grad);
+int polee_hsb_grad_device(const polee_hsb_plan *plan, int64_t B, const float *d_x_grad, const float *d_y_logit,
+                          float *d_y_logit_grad, void *stream);
 const char *polee_hsb_last_error(void);
 /* make_inverse_ptt_params(node_parent_idxs, node_js)  src/ptt.jl:293-309 (host helper, exact ints) */
 int polee_make_inverse_ptt_params(int64_t num_nodes, const int32_t *node_parent_idxs, const int32_t *node_js,

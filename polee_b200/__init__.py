@@ -24,8 +24,11 @@ from .api import (  # noqa: F401
     exact_factorization,
     hclust,
     hsb,
+    hsb_grad,
+    hsb_torch,
     inv_hsb,
     inv_hsb_grad,
+    inv_hsb_torch,
     log_likelihood,
     make_inverse_ptt_params,
     optimize_likelihood,

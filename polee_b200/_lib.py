@@ -39,7 +39,8 @@ EXPORTS = [
     "polee_ptt_transform_gradients", "polee_ptt_inverse_transform", "polee_lsn_draws", "polee_hsb", "polee_inv_hsb",
     "polee_inv_hsb_grad", "polee_hsb_device", "polee_inv_hsb_device", "polee_inv_hsb_grad_device", "polee_hsb_plan_create", "polee_hsb_plan_destroy", "polee_hsb_with_plan",
     "polee_inv_hsb_with_plan", "polee_inv_hsb_grad_with_plan", "polee_approx_log_prob_with_plan",
-    "polee_approx_log_prob_device", "polee_hsb_last_error",
+    "polee_approx_log_prob_device", "polee_hsb_grad", "polee_hsb_grad_with_plan", "polee_hsb_grad_device",
+    "polee_hsb_last_error",
     "polee_make_inverse_ptt_params", "polee_exact_factorization", "polee_hclust", "polee_partition_rows", "polee_comm_unique_id", "polee_comm_init", "polee_comm_peer_export", "polee_comm_peer_import",
 ]
 

@@ -667,6 +667,20 @@ def inv_hsb_grad(y_grad, ladj_grad, y, ladj, left_index, right_index, leaf_index
     return bp
 
 
+def hsb_grad(x_grad, y_logit, left_index, right_index, leaf_index, device=0):
+    """hsb_grad(x_grad, y_logit, left, right, leaf) -> y_logit_grad [B][n-1] float32: the gradient of hsb(y_logit) that
+    the reference leaves as a TODO (hsb_ops.cpp:123-125); definition: include/polee_b200.h, DESIGN.md K4."""
+    y_logit = _c(y_logit, np.float32)
+    B, nm1 = y_logit.shape
+    n = nm1 + 1
+    x_grad = _c(x_grad, np.float32).reshape(B, n)
+    (l, r, f), ib = _hsb_idx(left_index, right_index, leaf_index, B, n)
+    out = np.zeros((B, nm1), np.float32)
+    _hsb_check(L.load_library().polee_hsb_grad(C.c_int32(device), C.c_int64(B), C.c_int64(n), _p(x_grad), _p(y_logit),
+                                               _p(l), _p(r), _p(f), C.c_int64(ib), _p(out)))
+    return out
+
+
 class HsbPlan:
     """The validated, level-scheduled tree(s) of the three HSB ops resident on the device (polee_hsb_plan_*), with the
     device-resident entry points (polee_*_device): every tensor argument is a DEVICE pointer (int), the work is
@@ -703,6 +717,10 @@ class HsbPlan:
     def inv_hsb_grad_device(self, B, d_y_grad, d_ladj_grad, d_y, d_backprops, stream=0):
         _hsb_check(self.lib.polee_inv_hsb_grad_device(self.p, C.c_int64(B), C.c_void_p(d_y_grad), C.c_void_p(d_ladj_grad),
                                                       C.c_void_p(d_y), C.c_void_p(d_backprops), C.c_void_p(stream)))
+
+    def hsb_grad_device(self, B, d_x_grad, d_y_logit, d_y_logit_grad, stream=0):
+        _hsb_check(self.lib.polee_hsb_grad_device(self.p, C.c_int64(B), C.c_void_p(d_x_grad), C.c_void_p(d_y_logit),
+                                                  C.c_void_p(d_y_logit_grad), C.c_void_p(stream)))
 
     def approx_log_prob(self, x, mu, omega, alpha, want_grad=True):
         """log q(x) of the LogitSkewNormalPTT approximation on this plan's tree(s) (polee_approx_log_prob_with_plan;
@@ -775,3 +793,79 @@ def approx_log_prob_torch(plan, x, mu, omega, alpha):
 
         _approx_log_prob_fn = ApproxLogProb
     return _approx_log_prob_fn.apply(plan, x, mu, omega, alpha)
+
+
+_hsb_fn = None
+_inv_hsb_fn = None
+
+
+def _stream_of(t):
+    import torch
+    return torch.cuda.current_stream(t.device).cuda_stream
+
+
+def hsb_torch(plan, y_logit):
+    """Differentiable HSB for a torch model: x [B][n] (float32) = hsb(y_logit [B][n-1]) on the plan's tree(s), computed
+    by polee_hsb_device on torch's current stream; the backward is HSBGrad (polee_hsb_grad_device)."""
+    global _hsb_fn
+    if _hsb_fn is None:
+        import torch
+
+        class Hsb(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, plan, y_logit):
+                y_logit = y_logit.detach().to(torch.float32).contiguous()
+                B = y_logit.shape[0]
+                x = torch.empty((B, plan.n), dtype=torch.float32, device=y_logit.device)
+                plan.hsb_device(B, y_logit.data_ptr(), x.data_ptr(), _stream_of(y_logit))
+                ctx.plan = plan
+                ctx.save_for_backward(y_logit)
+                return x
+
+            @staticmethod
+            def backward(ctx, grad_x):
+                (y_logit,) = ctx.saved_tensors
+                grad_x = grad_x.to(torch.float32).contiguous()
+                out = torch.empty_like(y_logit)
+                ctx.plan.hsb_grad_device(y_logit.shape[0], grad_x.data_ptr(), y_logit.data_ptr(), out.data_ptr(),
+                                         _stream_of(y_logit))
+                return None, out
+
+        _hsb_fn = Hsb
+    return _hsb_fn.apply(plan, y_logit)
+
+
+def inv_hsb_torch(plan, x):
+    """Differentiable InvHSB for a torch model: (y [B][n-1] float64, ladj [B][1] float32) = inv_hsb(x [B][n]) on the
+    plan's tree(s), computed by polee_inv_hsb_device on torch's current stream; the backward is InvHSBGrad
+    (polee_inv_hsb_grad_device), with a missing upstream gradient taken as zeros."""
+    global _inv_hsb_fn
+    if _inv_hsb_fn is None:
+        import torch
+
+        class InvHsb(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, plan, x):
+                x = x.detach().to(torch.float32).contiguous()
+                B = x.shape[0]
+                y = torch.empty((B, plan.n - 1), dtype=torch.float64, device=x.device)
+                ladj = torch.empty((B, 1), dtype=torch.float32, device=x.device)
+                plan.inv_hsb_device(B, x.data_ptr(), y.data_ptr(), ladj.data_ptr(), _stream_of(x))
+                ctx.plan = plan
+                ctx.save_for_backward(y)
+                return y, ladj
+
+            @staticmethod
+            def backward(ctx, grad_y, grad_ladj):
+                (y,) = ctx.saved_tensors
+                B = y.shape[0]
+                grad_y = torch.zeros_like(y) if grad_y is None else grad_y.to(torch.float64).contiguous()
+                grad_ladj = (torch.zeros((B,), dtype=torch.float32, device=y.device) if grad_ladj is None
+                             else grad_ladj.to(torch.float32).reshape(B).contiguous())
+                out = torch.empty((B, ctx.plan.n), dtype=torch.float32, device=y.device)
+                ctx.plan.inv_hsb_grad_device(B, grad_y.data_ptr(), grad_ladj.data_ptr(), y.data_ptr(), out.data_ptr(),
+                                             _stream_of(y))
+                return None, out
+
+        _inv_hsb_fn = InvHsb
+    return _inv_hsb_fn.apply(plan, x)

@@ -24,6 +24,8 @@ struct polee_hsb_plan {
     int32_t *bin_tree[2] = {nullptr, nullptr};
     int nbins[2] = {0, 0};
     int32_t *desc_order = nullptr;  // [ntrees][n-1] internal node ids in descending node order (ladj emulation)
+    int32_t *bin_pos = nullptr;     // [ntrees][N] a bottom-bin node's position in its bin's schedule; -1: top node (HSBGrad)
+    int max_bin_nodes = 0;          // most nodes of a bottom bin (HSBGrad's shared memory)
     std::string err;
     // scratch of the device-resident entry points (u, v / log u per row; y, y_grad and row partials of the density),
     // grown on demand and kept with the plan so a training step allocates nothing; calls on one plan are serialised by `mu`
@@ -227,6 +229,96 @@ __global__ void __launch_bounds__(HSB_THREADS)
     }
 }
 
+// HSBGrad (the reference's op file leaves it as a TODO, hsb_ops.cpp:123-125; definition: DESIGN.md K4).  With y and u
+// exactly as k4_hsb_fwd makes them, G = x_grad at a leaf and G_j = y G_l + (1 - y) G_r at an internal node (so
+// G_j = sum over the leaves under j of x_grad u_leaf / u_j), and y_logit_grad_k = y (1 - y) u_j (G_l - G_r).  Every
+// value depends only on a node's parent (u) or children (G), so any schedule gives the same bits.
+__device__ __forceinline__ double hsb_y(float y_logit) { return __ddiv_rn(1.0, __dadd_rn(1.0, exp((double)(-y_logit)))); }
+
+__device__ __forceinline__ double hsb_grad_node(double y, double uj, double gl, double gr, float *out) {
+    *out = (float)__dmul_rn(__dmul_rn(__dmul_rn(y, __dsub_rn(1.0, y)), uj), __dsub_rn(gl, gr));
+    return __dadd_rn(__dmul_rn(y, gl), __dmul_rn(__dsub_rn(1.0, y), gr));
+}
+
+// top bins (after k4_hsb_fwd wrote u and k4_hsb_grad_bin the G of the bottom-bin roots): bottom-up with u and G in global
+// memory ([B][N] plan scratch, indexed by node)
+__global__ void __launch_bounds__(HSB_THREADS)
+    k4_hsb_grad_top(Sched s, int shared_tree, const TreeNode *__restrict__ nodes_all, int64_t n, int64_t N,
+                    const float *__restrict__ y_logit, const double *__restrict__ us, double *__restrict__ gs,
+                    float *__restrict__ y_logit_grad) {
+    int tree;
+    int64_t row;
+    bin_row(s, shared_tree, tree, row);
+    const TreeNode *nodes = nodes_all + (size_t)tree * N;
+    const double *u = us + (size_t)row * N;
+    double *g = gs + (size_t)row * N;
+    const int l0 = s.bin_lvl_ptr[blockIdx.x], l1 = s.bin_lvl_ptr[blockIdx.x + 1] - 1;
+    for (int l = l1 - 1; l >= l0; --l) {
+        for (int q = s.lvl_off[l] + threadIdx.x; q < s.lvl_off[l + 1]; q += HSB_THREADS) {
+            const int node = s.sch_node[q];
+            const TreeNode nd = nodes[node];  // top nodes are internal: their subtrees exceed a bin
+            const size_t i = (size_t)row * (n - 1) + nd.k;
+            g[node] = hsb_grad_node(hsb_y(y_logit[i]), node == 0 ? 1.0 : u[node], g[nd.left], g[nd.right], &y_logit_grad[i]);
+        }
+        __syncthreads();
+    }
+}
+
+// bottom bins: one CTA per (bin, row) runs the bin's forward and then its backward with u and G in shared memory, so no
+// per-node value goes through global memory; in: u of the bin's roots (k4_hsb_fwd over the top bins), out: their G.
+// Shared memory: u[nb] and, per internal node, y from the forward until the backward replaces it with G.
+constexpr int HSB_GRAD_THREADS = 256;
+__global__ void __launch_bounds__(HSB_GRAD_THREADS)
+    k4_hsb_grad_bin(Sched s, int shared_tree, const TreeNode *__restrict__ nodes_all, const int32_t *__restrict__ bin_pos_all,
+                    int64_t n, int64_t N, const float *__restrict__ x_grad, const float *__restrict__ y_logit,
+                    const double *__restrict__ us, double *__restrict__ gs, float *__restrict__ y_logit_grad) {
+    extern __shared__ double hsb_smem[];
+    int tree;
+    int64_t row;
+    bin_row(s, shared_tree, tree, row);
+    const TreeNode *nodes = nodes_all + (size_t)tree * N;
+    const int32_t *pos = bin_pos_all + (size_t)tree * N;
+    const int l0 = s.bin_lvl_ptr[blockIdx.x], l1 = s.bin_lvl_ptr[blockIdx.x + 1] - 1;
+    const int q0 = s.lvl_off[l0];
+    double *su = hsb_smem, *sg = hsb_smem + (s.lvl_off[l1] - q0);
+    for (int l = l0; l < l1; ++l) {
+        for (int q = s.lvl_off[l] + threadIdx.x; q < s.lvl_off[l + 1]; q += HSB_GRAD_THREADS) {
+            const int node = s.sch_node[q];
+            const TreeNode nd = nodes[node];
+            double ui;
+            if (l == l0) {
+                ui = node == 0 ? 1.0 : us[(size_t)row * N + node];
+                su[q - q0] = ui;
+            } else {
+                ui = su[q - q0];
+            }
+            if (nd.leaf < 0) {
+                const double y = hsb_y(y_logit[(size_t)row * (n - 1) + nd.k]);
+                sg[q - q0] = y;
+                su[pos[nd.left]] = __dmul_rn(y, ui);
+                su[pos[nd.right]] = __dmul_rn(__dsub_rn(1.0, y), ui);
+            }
+        }
+        __syncthreads();
+    }
+    for (int l = l1 - 1; l >= l0; --l) {
+        for (int q = s.lvl_off[l] + threadIdx.x; q < s.lvl_off[l + 1]; q += HSB_GRAD_THREADS) {
+            const int node = s.sch_node[q];
+            const TreeNode nd = nodes[node];
+            double gj;
+            if (nd.leaf >= 0) {
+                gj = (double)x_grad[(size_t)row * n + nd.leaf];
+            } else {
+                const size_t i = (size_t)row * (n - 1) + nd.k;
+                gj = hsb_grad_node(sg[q - q0], su[q - q0], sg[pos[nd.left]], sg[pos[nd.right]], &y_logit_grad[i]);
+            }
+            sg[q - q0] = gj;
+            if (l == l0) gs[(size_t)row * N + node] = gj;
+        }
+        __syncthreads();
+    }
+}
+
 // K5: log q(x) of the LogitSkewNormalPTT approximation (definition: DESIGN.md K5) from the y and log u that k4_inv_hsb
 // wrote.  One thread per (internal node k, row); a row's terms are summed in Float64 in a fixed order (warp shuffles,
 // then the block's warps, then k5_row_sum over the blocks), so results are run-to-run identical without atomics.
@@ -334,6 +426,7 @@ int polee_hsb_plan_destroy(polee_hsb_plan *p) {
     cudaSetDevice(p->device);
     polee::dfree(p->nodes);
     polee::dfree(p->desc_order);
+    polee::dfree(p->bin_pos);
     polee::dfree(p->scr[0]); polee::dfree(p->scr[1]); polee::dfree(p->scr[2]);
     for (int s = 0; s < 2; ++s) {
         polee::dfree(p->bin_lvl_ptr[s]); polee::dfree(p->lvl_off[s]); polee::dfree(p->sch_node[s]); polee::dfree(p->bin_tree[s]);
@@ -353,11 +446,18 @@ int polee_hsb_plan_create(polee_hsb_plan **out, int32_t device, int64_t n, int64
     const int64_t N = 2 * n - 1;
     std::vector<TreeNode> nodes((size_t)idx_batch * N);
     std::vector<int32_t> blp[2] = {{0}, {0}}, lo[2], sn[2], bt[2];
+    std::vector<int32_t> bin_pos((size_t)idx_batch * N, -1);
+    int max_bin_nodes = 0;
     for (int64_t t = 0; t < idx_batch; ++t) {
         TreeHost th;
         std::string e = th.build_from_lrf(n, left + t * N, right + t * N, leaf + t * N, HSB_BIN_NODES);
         if (!e.empty()) return hsb_fail(POLEE_EBADTREE, "tree " + std::to_string(t) + ": " + e);
         std::copy(th.nodes.begin(), th.nodes.end(), nodes.begin() + (size_t)t * N);
+        for (int b = 0; b < th.bottom.nbins(); ++b) {
+            const int32_t q0 = th.bottom.lvl_off[th.bottom.bin_lvl_ptr[b]], q1 = th.bottom.lvl_off[th.bottom.bin_lvl_ptr[b + 1] - 1];
+            for (int32_t q = q0; q < q1; ++q) bin_pos[(size_t)t * N + th.bottom.sch_node[q]] = q - q0;
+            max_bin_nodes = std::max(max_bin_nodes, (int)(q1 - q0));
+        }
         const TreeSchedHost *hs[2] = {&th.top, &th.bottom};
         for (int s = 0; s < 2; ++s) {
             const int32_t node_base = (int32_t)sn[s].size(), lvl_base = (int32_t)lo[s].size();
@@ -370,8 +470,9 @@ int polee_hsb_plan_create(polee_hsb_plan **out, int32_t device, int64_t n, int64
         }
     }
     polee_hsb_plan *p = new polee_hsb_plan();
-    p->device = device; p->n = n; p->N = N; p->ntrees = idx_batch;
+    p->device = device; p->n = n; p->N = N; p->ntrees = idx_batch; p->max_bin_nodes = max_bin_nodes;
     cudaError_t e = up_vec(nodes, &p->nodes);
+    if (e == cudaSuccess) e = up_vec(bin_pos, &p->bin_pos);
     for (int s = 0; s < 2 && e == cudaSuccess; ++s) {
         p->nbins[s] = (int)bt[s].size();
         e = up_vec(blp[s], &p->bin_lvl_ptr[s]);
@@ -479,6 +580,34 @@ int polee_inv_hsb_grad_device(const polee_hsb_plan *p, int64_t B, const double *
     return POLEE_OK;
 }
 
+// HSBGrad: k4_hsb_fwd over the top bins (u of the top nodes and of the bottom-bin roots) -> k4_hsb_grad_bin over the
+// bottom bins (forward and backward in shared memory; G of the bin roots) -> k4_hsb_grad_top over the top bins.
+int polee_hsb_grad_device(const polee_hsb_plan *p, int64_t B, const float *d_x_grad, const float *d_y_logit,
+                          float *d_y_logit_grad, void *stream) {
+    int rc = check_plan(p, B);
+    if (rc) return rc;
+    if (!d_x_grad || !d_y_logit || !d_y_logit_grad) return hsb_fail(POLEE_EINVAL, "hsb_grad: null pointer");
+    if (p->n == 1) return POLEE_OK;  // no internal node: the output is empty
+    std::lock_guard<std::mutex> lk(p->mu);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int shared = p->ntrees == 1;
+    const unsigned rows = shared ? (unsigned)B : 1u;
+    double *d_us, *d_gs;
+    if ((rc = plan_scratch(p, 0, (size_t)B * p->N, &d_us))) return rc;
+    if ((rc = plan_scratch(p, 1, (size_t)B * p->N, &d_gs))) return rc;
+    if (p->nbins[0] > 0)  // top bins hold internal nodes only: x is not written
+        k4_hsb_fwd<<<dim3(p->nbins[0], rows), HSB_THREADS, 0, st>>>(sched_of(p, 0), shared, p->nodes, p->n, p->N, d_y_logit, d_us,
+                                                                   nullptr);
+    HCK(allow_max_smem(k4_hsb_grad_bin));
+    k4_hsb_grad_bin<<<dim3(p->nbins[1], rows), HSB_GRAD_THREADS, (size_t)p->max_bin_nodes * 2 * sizeof(double), st>>>(
+        sched_of(p, 1), shared, p->nodes, p->bin_pos, p->n, p->N, d_x_grad, d_y_logit, d_us, d_gs, d_y_logit_grad);
+    if (p->nbins[0] > 0)
+        k4_hsb_grad_top<<<dim3(p->nbins[0], rows), HSB_THREADS, 0, st>>>(sched_of(p, 0), shared, p->nodes, p->n, p->N, d_y_logit,
+                                                                        d_us, d_gs, d_y_logit_grad);
+    HCK(cudaGetLastError());
+    return POLEE_OK;
+}
+
 // k4_inv_hsb -> k5_lsn_log_density -> k5_row_sum [-> k4_inv_hsb_grad with ladj_grad = 1].  The Float32 ladj replay
 // (k4_ladj_chain) is not needed: the density sums -log u_j in Float64 with the other terms.
 int polee_approx_log_prob_device(const polee_hsb_plan *p, int64_t B, int64_t param_batch, const float *d_x,
@@ -565,6 +694,22 @@ int polee_inv_hsb_grad_with_plan(const polee_hsb_plan *p, int64_t B, const doubl
     return POLEE_OK;
 }
 
+int polee_hsb_grad_with_plan(const polee_hsb_plan *p, int64_t B, const float *x_grad, const float *y_logit, float *y_logit_grad) {
+    int rc = check_plan(p, B);
+    if (rc) return rc;
+    if (!x_grad || !y_logit || !y_logit_grad) return hsb_fail(POLEE_EINVAL, "hsb_grad: null pointer");
+    const int64_t nm1 = p->n - 1;
+    if (nm1 == 0) return POLEE_OK;
+    DevBuf db;
+    float *d_xg, *d_yl, *d_ylg;
+    HCK(db.upload(&d_xg, x_grad, (size_t)B * p->n));
+    HCK(db.upload(&d_yl, y_logit, (size_t)B * nm1));
+    HCK(db.alloc(&d_ylg, (size_t)B * nm1));
+    if ((rc = polee_hsb_grad_device(p, B, d_xg, d_yl, d_ylg, nullptr))) return rc;
+    HCK(cudaMemcpy(y_logit_grad, d_ylg, sizeof(float) * (size_t)B * nm1, cudaMemcpyDeviceToHost));
+    return POLEE_OK;
+}
+
 int polee_approx_log_prob_with_plan(const polee_hsb_plan *p, int64_t B, int64_t param_batch, const float *x,
                                     const float *mu, const float *omega, const float *alpha, double *lp, float *x_grad) {
     int rc = check_plan(p, B);
@@ -594,6 +739,16 @@ int polee_hsb(int32_t device, int64_t B, int64_t n, const float *y_logit, const 
     polee_hsb_plan *p = nullptr;
     int rc = polee_hsb_plan_create(&p, device, n, idx_batch, left, right, leaf);
     if (!rc) rc = polee_hsb_with_plan(p, B, y_logit, x);
+    polee_hsb_plan_destroy(p);
+    return rc;
+}
+
+int polee_hsb_grad(int32_t device, int64_t B, int64_t n, const float *x_grad, const float *y_logit, const int32_t *left,
+                   const int32_t *right, const int32_t *leaf, int64_t idx_batch, float *y_logit_grad) {
+    if (idx_batch != 1 && idx_batch != B) return hsb_fail(POLEE_EINVAL, "hsb_grad: idx_batch must be 1 or B");
+    polee_hsb_plan *p = nullptr;
+    int rc = polee_hsb_plan_create(&p, device, n, idx_batch, left, right, leaf);
+    if (!rc) rc = polee_hsb_grad_with_plan(p, B, x_grad, y_logit, y_logit_grad);
     polee_hsb_plan_destroy(p);
     return rc;
 }

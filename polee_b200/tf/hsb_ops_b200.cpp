@@ -1,7 +1,8 @@
 // hsb_ops_b200.cpp -- drop-in replacement for the reference's src/tensorflow_ext/hsb_ops.cpp: the same three
 // ops (names, inputs, outputs, dtypes, shape functions: hsb_ops.cpp:17-38, 128-150, 252-278) whose Compute()
 // forwards to libpolee_b200.so.  Python keeps doing `tf.load_op_library(...)` and calling `hsb`, `inv_hsb`,
-// `inv_hsb_grad` (src/polee_approx_likelihood.py:13-28, 50, 408) unchanged.
+// `inv_hsb_grad` (src/polee_approx_likelihood.py:13-28, 50, 408) unchanged.  A fourth op, HSBGrad, is the gradient
+// of HSB that the reference leaves as a TODO (hsb_ops.cpp:123-125); INTEGRATION.md §3 registers it for `hsb`.
 //
 // Build (mirrors src/tensorflow_ext/mkfile and PoleeModel.jl:53-64):
 //   g++ -std=c++14 -shared -fPIC -O2 hsb_ops_b200.cpp -o hsb_ops.so $TF_CFLAGS $TF_LFLAGS
@@ -235,3 +236,48 @@ class InvHSBGradOpB200 : public OpKernel {
 REGISTER_KERNEL_BUILDER(Name("InvHSBGrad").Device(DEVICE_CPU), InvHSBGradOpB200<false>);
 REGISTER_KERNEL_BUILDER(Name("InvHSBGrad").Device(DEVICE_GPU).HostMemory("left_index").HostMemory("right_index").HostMemory("leaf_index"),
                         InvHSBGradOpB200<true>);
+
+REGISTER_OP("HSBGrad")
+    .Input("x_grad: float32")
+    .Input("y_logit: float32")
+    .Input("left_index: int32")
+    .Input("right_index: int32")
+    .Input("leaf_index: int32")
+    .Output("y_logit_grad: float32")
+    .SetShapeFn([](shape_inference::InferenceContext* c) {
+        shape_inference::ShapeHandle y_logit, unused;
+        TF_RETURN_IF_ERROR(c->WithRank(c->input(0), 2, &unused));
+        TF_RETURN_IF_ERROR(c->WithRank(c->input(1), 2, &y_logit));
+        TF_RETURN_IF_ERROR(c->WithRank(c->input(2), 2, &unused));
+        TF_RETURN_IF_ERROR(c->WithRank(c->input(3), 2, &unused));
+        TF_RETURN_IF_ERROR(c->WithRank(c->input(4), 2, &unused));
+        c->set_output(0, y_logit);
+        return Status::OK();
+    });
+
+template <bool ON_DEVICE>
+class HSBGradOpB200 : public OpKernel {
+   public:
+    explicit HSBGradOpB200(OpKernelConstruction* context) : OpKernel(context) {}
+    void Compute(OpKernelContext* context) override {
+        const Tensor& x_grad = context->input(0);
+        const Tensor& y_logit = context->input(1);
+        const int64 B = y_logit.dim_size(0), n = y_logit.dim_size(1) + 1;
+        Tensor* out = nullptr;
+        OP_REQUIRES_OK(context, context->allocate_output(0, TensorShape({B, n - 1}), &out));
+        std::string err;
+        polee_hsb_plan* p = plan_for(B, n, &context->input(2).flat_inner_dims<int32>()(0, 0),
+                                     &context->input(3).flat_inner_dims<int32>()(0, 0),
+                                     &context->input(4).flat_inner_dims<int32>()(0, 0), &err);
+        if (!p) OP_REQUIRES_OK(context, fail(err));
+        const float* xg = &x_grad.flat_inner_dims<float>()(0, 0);
+        const float* yl = &y_logit.flat_inner_dims<float>()(0, 0);
+        float* o = &out->flat_inner_dims<float>()(0, 0);
+        const int rc = ON_DEVICE ? polee_hsb_grad_device(p, B, xg, yl, o, polee_tf_stream(context))
+                                 : polee_hsb_grad_with_plan(p, B, xg, yl, o);
+        if (rc != POLEE_OK) OP_REQUIRES_OK(context, fail(polee_hsb_last_error()));
+    }
+};
+REGISTER_KERNEL_BUILDER(Name("HSBGrad").Device(DEVICE_CPU), HSBGradOpB200<false>);
+REGISTER_KERNEL_BUILDER(Name("HSBGrad").Device(DEVICE_GPU).HostMemory("left_index").HostMemory("right_index").HostMemory("leaf_index"),
+                        HSBGradOpB200<true>);
