@@ -999,7 +999,11 @@ extern "C" int polee_lsn_draws(polee_handle *h, const float *zs0, int32_t K, flo
     rc = launch_elem(h, KP, K, false, false, true, d_noise, 1, !h->o.gradonly, nullptr);
     if (!rc) rc = launch_step_sequence(h, false, false, h->grad_out, d_xg, d_noise, 1);
     h->reparam_ready = false;
-    cudaError_t e = cudaStreamSynchronize(h->stream);
+    // a launch refused for its configuration shows only here: the outputs would be stale (the step counters are
+    // restored below on this path too)
+    cudaError_t e = cudaGetLastError();
+    if (!rc && e != cudaSuccess) rc = h->fail(POLEE_ECUDA, std::string("lsn_draws: ") + cudaGetErrorString(e));
+    e = cudaStreamSynchronize(h->stream);
     if (!rc && e != cudaSuccess) rc = h->fail(POLEE_ECUDA, std::string("lsn_draws: ") + cudaGetErrorString(e));
     if (!rc && xs) rc = download_kmajor<float, float>(h, h->x, K, KP, n, xs);
     if (!rc && ys) rc = download_kmajor<double, double>(h, h->ys, K, KP, nm1, ys);

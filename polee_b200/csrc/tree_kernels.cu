@@ -1090,6 +1090,11 @@ static size_t dfs_fwd_smem(const TreeDev &td, int KP) {
            (size_t)DFS_RUNS_PER_CTA * (DFS_RUN + 2) * sizeof(DNode);
 }
 
+// dynamic shared memory of k3p_tree_fwd: y and 1 - y of the group's ancestors by draw, the common prefix, the suffixes
+static size_t path_fwd_smem(const TreeDev &td, int KP) {
+    return (size_t)td.max_ganc * (16 * KP + 2) + 16 + 2 * (size_t)td.max_gsuf;
+}
+
 // The kernels that serve a tree at KP draws: the first route whose condition holds.
 //
 //   route         condition                                       forward        backward       inverse
@@ -1097,7 +1102,8 @@ static size_t dfs_fwd_smem(const TreeDev &td, int KP) {
 //   DfsRun        bins fit, DFS-run inputs built (pre-order,      k3d_tree_fwd   k3s_tree_bwd   k3_tree_inv
 //                 depth <= DFS_MAX_DEPTH), KP <= 16,
 //                 dfs_fwd_smem <= 200 KB
-//   PathProduct   bins fit, root-path tables built                k3p_tree_fwd   k3s_tree_bwd   k3_tree_inv
+//   PathProduct   bins fit, root-path tables built,               k3p_tree_fwd   k3s_tree_bwd   k3_tree_inv
+//                 path_fwd_smem <= 200 KB
 //   SmemLevels    bins fit                                        k3s_tree_fwd   k3s_tree_bwd   k3_tree_inv
 //   GlobalLevels  everything else                                 k3_tree_fwd    k3_tree_bwd    k3_tree_inv
 //
@@ -1114,7 +1120,7 @@ TreeRoute tree_route(const TreeDev &td, int KP) {
         (size_t)td.s_top.max_bin_nodes * (sizeof(SNode) + 24) + 4 * (td.s_top.max_bin_levels + 2) <= limit;
     if (!bins_fit) return TreeRoute::GlobalLevels;
     if (td.dnodes && KP <= 16 && dfs_fwd_smem(td, KP) <= limit) return TreeRoute::DfsRun;
-    if (td.ganc_ptr) return TreeRoute::PathProduct;
+    if (td.ganc_ptr && path_fwd_smem(td, KP) <= limit) return TreeRoute::PathProduct;
     return TreeRoute::SmemLevels;
 }
 
@@ -1182,7 +1188,7 @@ int launch_tree_fwd(polee_handle *h, int KP, int clamp_x, int want_S, int want_l
             break;
         }
         case TreeRoute::PathProduct: {
-            const size_t smem = (size_t)td.max_ganc * (16 * KP + 2) + 16 + 2 * (size_t)td.max_gsuf;
+            const size_t smem = path_fwd_smem(td, KP);
             if (smem > 40 * 1024) DISPATCH_KP(KP, allow_max_smem(k3p_tree_fwd<KPC>));
             DISPATCH_KP(KP, (k3p_tree_fwd<KPC><<<td.n_groups, PATH_SLOTS * KPC, smem, h->stream>>>(
                                 td.N, td.nodes, td.ganc_ptr, td.ganc, td.gcp, td.nsuf_ptr, td.nsuf, h->ys, h->us, h->x, clamp_x,
